@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- self-play env-steps/s including the E-MCTS search (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload c2|c1|c3]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload c2|c1|c3] [--dump-outputs DIR]
 
 One "step" = one self-play move for a whole batch of envs: root network forward -> E-MCTS search
 (num_simulations x select/expand/backward with env step, hash probe and network per simulation) ->
@@ -331,6 +331,7 @@ def run_b200(args, kind, kw, B, n, gamma, desc):
     side = torch.cuda.Stream(device=dev) if world > 1 else None
     gather_done = [None, None]
     tick = [0]
+    record = [None]  # the trajectory record of the latest step (a view into the scan buffer)
 
     def one_step(st):
         i = tick[0]
@@ -338,7 +339,7 @@ def run_b200(args, kind, kw, B, n, gamma, desc):
         if world > 1 and row == 0 and gather_done[buf] is not None:
             torch.cuda.current_stream().wait_event(gather_done[buf])  # the gather that last read this scan buffer has finished
         st, out = runner.step(st)
-        runner.trajectory(st, out, scan[buf][row])
+        record[0] = runner.trajectory(st, out, scan[buf][row])
         if world > 1 and row == T - 1:
             ready = torch.cuda.Event()
             ready.record()
@@ -395,6 +396,11 @@ def run_b200(args, kind, kw, B, n, gamma, desc):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms_total = float(t.item())
     value = world * B * args.steps / (ms_total * 1e-3)
+    if args.dump_outputs:  # before the e2e leg below steps the same state and output buffers again
+        arrays = {f"state_{k}": states[k] for k in ops.state_fields(env)}
+        arrays.update((k, v) for k, v in vars(out).items() if k != "state")
+        arrays["trajectory"] = record[0]
+        dump_outputs(args.dump_outputs, arrays, prefix="" if world == 1 else f"rank{rank}_")
 
     # ---- e2e: host buffers in, host results out, copies inside the timed region (rank-local, max over ranks).
     # A graph runner keeps its state fields in one device arena and the search outputs in another (ops.alloc_arena), so a host caller
@@ -577,6 +583,28 @@ def run_b200(args, kind, kw, B, n, gamma, desc):
         dist.destroy_process_group()
 
 
+DUMP_LIMIT_BYTES = 64 * 10**6
+
+
+def dump_outputs(out_dir, arrays, prefix=""):
+    """Write each [B, ...] tensor of `arrays` to out_dir/<prefix><name>.npy, so that the results of two builds can be compared
+    array for array.  Integers of up to 16 bits and floats of up to 32 go out as float32, wider ones as float64: both exact.  Above
+    DUMP_LIMIT_BYTES in all, every array keeps the same fixed, seeded sample of rows (envs)."""
+    host = {}
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        host[name] = a.astype(np.float32 if a.itemsize <= (4 if a.dtype.kind == "f" else 2) else np.float64)
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_LIMIT_BYTES:
+        B = len(next(iter(host.values())))
+        rows = np.sort(np.random.default_rng(0).choice(B, B * DUMP_LIMIT_BYTES // total, replace=False))
+        host = {name: a[rows] for name, a in host.items()}
+        print(f"bench.py: --dump-outputs keeps {len(rows)} of {B} rows (seed 0) of every array", file=sys.stderr)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(out_dir, f"{prefix}{name}.npy"), np.ascontiguousarray(a))
+
+
 _REAL_STDOUT = None
 
 
@@ -613,7 +641,14 @@ def main():
                     help="rebuild the parameter-derived tables every N steps (the reference runs selfplay_steps=8 DeepSea steps per model, config.py:105)")
     ap.add_argument("--no-fused-root", action="store_true", help="evaluate the root network with a separate eaz_mlp_forward_states call")
     ap.add_argument("--no-graph", action="store_true", help="launch kernels eagerly instead of replaying a CUDA graph of the step")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned (states, search outputs, trajectory record) "
+                         "to DIR/<name>.npy as float32 / float64")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the b200 implementation")
     kind, kw, B, n, gamma, desc = WORKLOADS[args.workload]
     if args.envs_per_gpu or args.sims:  # exploration knobs (not the BASELINE configs): the description says so
         B, n = args.envs_per_gpu or B, args.sims or n
