@@ -8,7 +8,7 @@ from __future__ import annotations
 
 import ctypes as C
 
-ABI_VERSION = 2
+ABI_VERSION = 3
 
 EAZ_OK = 0
 EAZ_ERR_INVALID_ARG = -1
@@ -38,6 +38,11 @@ def flag_streams(k: int) -> int:
 
 
 SEARCH_DEFAULT_FLAGS = FLAG_BETA_INTERIOR | FLAG_BETA_RAW | FLAG_BETA_FINAL
+
+PRIORITY_BAD_PRIORITY = 1 << 0
+PRIORITY_BAD_INDEX = 1 << 1
+PRIORITY_EMPTY = 1 << 2
+PRIORITY_BAD_ADD = 1 << 3
 
 MLP_EXACT = 0
 MLP_TENSOR = 1

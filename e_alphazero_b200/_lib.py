@@ -27,6 +27,7 @@ EXPORTS = [
     "eaz_search_workspace_bytes", "eaz_search_gumbel", "eaz_search_gumbel_profiled", "eaz_search_num_launches", "eaz_search_numeric_status",
     "eaz_reanalyze_targets",
     "eaz_convnet_workspace_bytes", "eaz_convnet_forward", "eaz_convnet_numeric_status",
+    "eaz_priority_tree_bytes", "eaz_priority_init", "eaz_priority_add_step", "eaz_priority_set", "eaz_priority_sample", "eaz_priority_status",
 ]
 
 
@@ -56,6 +57,7 @@ def load():
     lib.eaz_last_error.restype = C.c_char_p
     lib.eaz_search_workspace_bytes.restype = C.c_size_t
     lib.eaz_convnet_workspace_bytes.restype = C.c_size_t
+    lib.eaz_priority_tree_bytes.restype = C.c_size_t
     if lib.eaz_abi_version() != _abi.ABI_VERSION:
         raise EazError(f"ABI version mismatch: library {lib.eaz_abi_version()} vs bindings {_abi.ABI_VERSION}")
     _lib = lib

@@ -233,6 +233,54 @@ def trajectory_pack(env: EnvSpec, st: dict, action, out=None):
     return out
 
 
+# --------------------------------------------------------------------------- prioritised replay (csrc/replay.cu)
+def priority_tree_bytes(T: int, B: int) -> int:
+    n = load().eaz_priority_tree_bytes(int(T), int(B))
+    if n == 0:
+        check(-1, "eaz_priority_tree_bytes")
+    return int(n)
+
+
+def priority_init(tree, T: int, B: int, priority_exponent: float, seed: int = 0) -> None:
+    """eaz_priority_init on a uint8 device buffer of priority_tree_bytes(T, B)."""
+    check(load().eaz_priority_init(_ptr(tree), C.c_size_t(tree.numel()), int(T), int(B), C.c_float(priority_exponent), C.c_uint32(seed),
+                                   _stream()), "eaz_priority_init")
+
+
+def priority_add_step(tree, T: int, B: int, slot: int) -> None:
+    check(load().eaz_priority_add_step(_ptr(tree), C.c_size_t(tree.numel()), int(T), int(B), int(slot), _stream()), "eaz_priority_add_step")
+
+
+def priority_set(tree, T: int, B: int, indices, priorities) -> None:
+    """eaz_priority_set: indices int32 [K], priorities float32 [K], both contiguous device tensors."""
+    import torch
+
+    if indices.numel() != priorities.numel():
+        raise EazError("set_priorities: indices and priorities differ in length")
+    check(load().eaz_priority_set(_ptr(tree), C.c_size_t(tree.numel()), int(T), int(B), _ptr(indices, torch.int32), _ptr(priorities, torch.float32),
+                                  int(indices.numel()), _stream()), "eaz_priority_set")
+
+
+def priority_sample(tree, T: int, B: int, indices, probabilities, states=None, rewards=None, first=None, first_rewards=None, second=None,
+                    second_rewards=None) -> None:
+    """eaz_priority_sample: K = indices.numel() draws into the given buffers; with `states` ([T,B,S] uint8) the compact records
+    (and with `rewards` [T,B] the rewards) of both slots of every drawn pair are gathered into first / second [K,S]."""
+    import torch
+
+    S = 0 if states is None else states.shape[-1]
+    check(load().eaz_priority_sample(_ptr(tree), C.c_size_t(tree.numel()), int(T), int(B), int(indices.numel()), _ptr(states, torch.uint8),
+                                     _ptr(rewards, torch.float32), S, _ptr(indices, torch.int32), _ptr(probabilities, torch.float32),
+                                     _ptr(first, torch.uint8), _ptr(first_rewards, torch.float32), _ptr(second, torch.uint8),
+                                     _ptr(second_rewards, torch.float32), _stream()), "eaz_priority_sample")
+
+
+def priority_status(tree) -> int:
+    """eaz_priority_status: synchronises; raises EazError if a sticky EAZ_PRIORITY_* bit is set, else returns 0."""
+    flags = C.c_int32(0)
+    check(load().eaz_priority_status(_ptr(tree), C.c_size_t(tree.numel()), _stream(), C.byref(flags)), "eaz_priority_status")
+    return int(flags.value)
+
+
 def subleq_test_cases(task: int, ws: int):
     import numpy as np
 

@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define EAZ_ABI_VERSION 2
+#define EAZ_ABI_VERSION 3
 
 enum {
   EAZ_OK = 0,
@@ -417,6 +417,47 @@ int eaz_reanalyze_targets(const eaz_reanalyze_config* cfg, int32_t B, int32_t A,
                           const float* value_epistemic_std, const float* next_state_value, const float* next_rewards,
                           const uint8_t* next_terminated, const uint8_t* terminated, const uint8_t* invalid_actions,
                           float* value_target, float* ube_target, float* exploration_policy_target, void* stream);
+
+/* ------------------------------------------------------------------------ */
+/* Prioritised replay sampling (SURVEY 8f-3): the sum tree of the reference's  */
+/* flashbax prioritised flat buffer (main.py:217-225 priority_exponent,        */
+/* main.py:413-414 sample + batch.indices, main.py:454 set_priorities) over a  */
+/* compact replay ring of T time slots x B envs.  Item i = t * B + b is the    */
+/* pair (slot t, slot (t+1) % T) of env b; its weight is priority^exponent.    */
+/* The tree, its header (cursor, length, max priority, draw counter, sticky    */
+/* status) and the descent / node-sum / stratification order are specified in  */
+/* csrc/replay.cu; every call below is asynchronous on `stream`, allocates     */
+/* nothing and does not synchronise (except eaz_priority_status).              */
+
+enum {
+  EAZ_PRIORITY_BAD_PRIORITY = 1 << 0, /* a negative or non-finite priority was stored as 0 */
+  EAZ_PRIORITY_BAD_INDEX = 1 << 1,    /* an index outside [0, T*B) was skipped */
+  EAZ_PRIORITY_EMPTY = 1 << 2,        /* sampled a tree whose total weight was 0 (outputs: index 0, probability 0) */
+  EAZ_PRIORITY_BAD_ADD = 1 << 3       /* add_step for a slot that is neither the cursor nor the newest slot (ignored) */
+};
+
+/* Bytes of the caller-owned tree buffer for T >= 2 slots x B >= 1 envs (T * B < 2^31); 0 (and a message) otherwise.
+ * The buffer must be 128-byte aligned. */
+size_t eaz_priority_tree_bytes(int32_t T, int32_t B);
+/* Zero the tree and write the header: exponent (0 <= alpha <= 1), seed, max priority 1, draw counter 0, cursor 0, length 0. */
+int eaz_priority_init(void* tree, size_t tree_bytes, int32_t T, int32_t B, float priority_exponent, uint32_t seed, void* stream);
+/* Slot `slot` of the ring has just been written (the ring's add): the items starting at slot-1 get max_priority^alpha, the
+ * items starting at `slot` get 0; cursor / length advance (or stay, when the newest slot was rewritten). */
+int eaz_priority_add_step(void* tree, size_t tree_bytes, int32_t T, int32_t B, int32_t slot, void* stream);
+/* flashbax set_priorities: leaves indices[k] = priorities[k]^alpha for the K device entries (the last occurrence of a duplicated
+ * index wins; invalid items keep weight 0), max_priority = max(max_priority, priorities), ancestors recomputed. */
+int eaz_priority_set(void* tree, size_t tree_bytes, int32_t T, int32_t B, const int32_t* indices, const float* priorities, int32_t K,
+                     void* stream);
+/* flashbax sample: K stratified draws (1 <= K <= 2^24) -> indices [K] and probabilities [K] = weight / total.  If `states`
+ * (the ring's compact records [T,B,S]) is non-NULL the same kernel gathers both slots of every drawn pair into first / second
+ * [K,S] (and `rewards` [T,B], if non-NULL, into first_rewards / second_rewards [K]) for eaz_env_uncompact.  Advances the draw
+ * counter. */
+int eaz_priority_sample(void* tree, size_t tree_bytes, int32_t T, int32_t B, int32_t K, const uint8_t* states, const float* rewards, int32_t S,
+                        int32_t* indices, float* probabilities, uint8_t* first, float* first_rewards, uint8_t* second,
+                        float* second_rewards, void* stream);
+/* SYNCHRONISES `stream` and reads the sticky EAZ_PRIORITY_* bits into *flags_out; returns EAZ_ERR_UNSUPPORTED with a message if
+ * any is set, 0 otherwise. */
+int eaz_priority_status(const void* tree, size_t tree_bytes, void* stream, int32_t* flags_out);
 
 #ifdef __cplusplus
 }
