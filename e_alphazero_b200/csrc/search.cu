@@ -73,6 +73,7 @@ struct Tree {
   int32_t* cell;  // DeepSea: observation cell of the pending leaf (saves the network kernel a dependent load)
   int32_t* table;
   uint8_t* ds_seen;
+  float4* ds_out;  // DeepSea, persistent search: per-cell network outputs (psearch.cuh: ds_output_table_kernel)
   uint8_t* wimg;  // tensor-path weight images (mlp_mode TENSOR)
   int2* path;     // [max_depth][B] (node, action) per level of the current descent
   int32_t* path_len;
@@ -88,7 +89,8 @@ struct Layout {
 
 static size_t align_up(size_t x) { return (x + 255) & ~(size_t)255; }
 
-static void make_layout(int B, int N, int A, int S, int table_len, int obs_dim, size_t wimg_bytes, int max_depth, Layout* L) {
+static void make_layout(int B, int N, int A, int S, int table_len, int obs_dim, size_t wimg_bytes, size_t out_table_bytes, int max_depth,
+                        Layout* L) {
   const size_t nb = (size_t)N * B, nba = nb * A;
   size_t o = 0;
   int i = 0;
@@ -100,7 +102,8 @@ static void make_layout(int B, int N, int A, int S, int table_len, int obs_dim, 
   L->zero_end = o;
   L->ones_begin = L->ones_end = o;
   put((size_t)B * 4);                   // 3 cell
-  for (int k = 4; k < 14; ++k) put(0);  // (slots kept so that the scratch offsets below stay stable)
+  put(out_table_bytes);                 // 4 ds_out
+  for (int k = 5; k < 14; ++k) put(0);  // (slots kept so that the scratch offsets below stay stable)
   put((size_t)B * A * 4);  // 14 gumbel
   put((size_t)B * A * 4);  // 15 net_logits
   put((size_t)B * 4);      // 16 net_value
@@ -137,6 +140,7 @@ static Tree make_tree(void* ws, const Layout& L, int B, int N, int A, int S) {
   t.leaf = (int32_t*)(p + L.off[21]);
   t.table = (int32_t*)(p + L.off[22]);
   t.ds_seen = p + L.off[23];
+  t.ds_out = (float4*)(p + L.off[4]);
   t.wimg = p + L.off[24];
   t.path = (int2*)(p + L.off[25]);
   t.path_len = (int32_t*)(p + L.off[26]);
@@ -494,7 +498,7 @@ __global__ void __launch_bounds__(128) root_init_kernel(Tree t, SearchParams sp,
 #include "psearch.cuh"
 namespace eaz {
 
-// ------------------------------------------------------------------ persistent tile-resident search (psearch.cuh): eligibility + launch
+// ------------------------------------------------------------------ persistent search (psearch.cuh): eligibility, output table, launch
 static unsigned long long* g_ps_trace = nullptr;  // eaz_debug_set_ps_trace
 static bool persistent_eligible(int B, int N, int A, int flags, const EnvDesc& env, int mlp_mode, int* ncap_out) {
   static const bool disabled = getenv("EAZ_NO_PERSISTENT") != nullptr;  // measurement knob: the per-simulation launch chain instead
@@ -504,48 +508,44 @@ static bool persistent_eligible(int B, int N, int A, int flags, const EnvDesc& e
   if (flags & EAZ_FLAG_PUCT) return false;  // PUCT selection has no staged form: DIRECT chain
   if (N > 16383) return false;              // 16-bit cached selections
   const int ncap = (N + 1) & ~1;
-  int dev = 0, max_optin = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&max_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) != cudaSuccess) return false;
-  if (ps::smem_bytes(ncap, env.size) > (size_t)max_optin) return false;  // trees too large for the shared-memory caches
-  // At most two waves of clusters: a tile's chain (network -> tree -> network ...) is latency-bound, so every further wave adds a whole
-  // search time, while the per-simulation launch chain fills the machine with every kernel.  Measured at DeepSea-100 x 8192 trees x 128
-  // simulations (C4: 64 tiles on 37 co-resident clusters, two waves): 3.99 ms persistent vs 4.6 - 4.9 ms chain (before the kernel's
-  // spills were removed: 5.2 vs 4.5); at 4096 trees = 32 tiles: 0.83 vs 1.29 ms.  Larger batches stay on the chain (unmeasured beyond).
-  static int max_clusters[32] = {0};  // per device, queried once (idempotent; a race only repeats the query)
-  if (dev >= 0 && dev < 32 && max_clusters[dev] == 0) {
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3(ps::kCtas * 64);
-    cfg.blockDim = dim3(ps::kThreads);
-    cfg.dynamicSmemBytes = (size_t)max_optin;  // (any eligible shape: one CTA per SM either way)
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = ps::kCtas;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    int nc = 0;
-    if (cudaFuncSetAttribute(ps::ds_search_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cfg.dynamicSmemBytes) != cudaSuccess ||
-        cudaOccupancyMaxActiveClusters(&nc, ps::ds_search_kernel, &cfg) != cudaSuccess || nc < 1) {
+  int dev = 0, max_optin = 0, sms = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 32 ||
+      cudaDeviceGetAttribute(&max_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) != cudaSuccess ||
+      cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess)
+    return false;
+  const size_t smem = ps::smem_bytes(ncap, env.size);
+  if (smem > (size_t)max_optin) return false;  // trees too large for the shared-memory caches
+  // At most two waves of CTAs: a CTA's chain of simulations is latency-bound, so every further wave adds a whole search time, while the
+  // per-simulation launch chain fills the machine with every kernel.  Measured at DeepSea-100 x 8192 trees x 128 simulations (C4), with
+  // the network still evaluated inside the kernel: two waves 3.99 ms persistent vs 4.6 - 4.9 ms chain.  Larger batches stay on the chain
+  // (unmeasured beyond).
+  static bool attr_set[32] = {false};  // per device (idempotent; a race only repeats the call)
+  if (!attr_set[dev]) {
+    if (cudaFuncSetAttribute(ps::ds_search_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, max_optin) != cudaSuccess) {
       cudaGetLastError();
-      nc = -1;
+      return false;
     }
-    max_clusters[dev] = nc;
+    attr_set[dev] = true;
   }
-  static const bool any_waves = getenv("EAZ_PERSISTENT_WAVES") != nullptr;  // measurement knob: allow more tiles than co-resident clusters
-  if (!any_waves && (dev < 0 || dev >= 32 || ceil_div(B, ps::kTile) > 2 * max_clusters[dev])) return false;
+  int per_sm = 0;  // co-resident CTAs per SM at this shape's shared memory
+  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ps::ds_search_kernel, ps::kThreads, smem) != cudaSuccess || per_sm < 1) {
+    cudaGetLastError();
+    return false;
+  }
+  static const bool any_waves = getenv("EAZ_PERSISTENT_WAVES") != nullptr;  // measurement knob: allow more CTAs than two waves
+  if (!any_waves && ceil_div(B, ps::kSlots) > 2 * per_sm * sms) return false;
   if (ncap_out) *ncap_out = ncap;
   return true;
 }
 
-static int launch_persistent(const Tree& t, const SearchParams& sp, const EnvDesc& env, const NetDesc& net, const TensorWeights& tw,
-                             const eaz_search_inputs* in, int lhead, int ncap, cudaStream_t st) {
-  ps::Args a{};
-  a.t = t;
-  a.sp = sp;
-  a.env = env;
-  a.beta = in->beta;
-  a.invalid = in->invalid_actions;
+// bytes of the per-cell output table the persistent search reads (DeepSea, tensor mode)
+static size_t ds_out_bytes(int mlp_mode, const EnvDesc& env) {
+  return (mlp_mode == EAZ_MLP_TENSOR && env.kind == EAZ_ENV_DEEPSEA) ? (size_t)env.obs_dim * sizeof(float4) : 0;
+}
+
+// per-model table of the three head outputs of every DeepSea cell (after launch_deepsea_seen_table and prepare_tensor_weights)
+static int launch_output_table(const Tree& t, const EnvDesc& env, const NetDesc& net, const TensorWeights& tw, int lhead, cudaStream_t st) {
+  ps::TableArgs a{};
   const int heads[ps::kHeads] = {EAZ_HEAD_VALUE, EAZ_HEAD_UBE, lhead};
   for (int r = 0; r < ps::kHeads; ++r) {
     const int h = heads[r];
@@ -561,24 +561,33 @@ static int launch_persistent(const Tree& t, const SearchParams& sp, const EnvDes
   a.ds_seen = t.ds_seen;
   a.max_u = net.max_u;
   a.novelty_scale = net.novelty_scale;
+  a.cells = env.obs_dim;
+  a.out = t.ds_out;
+  static bool attr_set = false;  // idempotent; a race only repeats the call
+  if (!attr_set) {
+    if (cudaError_t e = cudaFuncSetAttribute(ps::ds_output_table_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ps::kTableSmem);
+        e != cudaSuccess)
+      return cuda_fail(e, "cudaFuncSetAttribute(ds_output_table_kernel)");
+    attr_set = true;
+  }
+  ps::ds_output_table_kernel<<<dim3(ceil_div(env.obs_dim, ps::kRows), ps::kHeads), ps::kTableThreads, ps::kTableSmem, st>>>(a);
+  EAZ_CHECK_LAUNCH("ds_output_table_kernel");
+  return 0;
+}
+
+static int launch_persistent(const Tree& t, const SearchParams& sp, const EnvDesc& env, const eaz_search_inputs* in, int ncap, cudaStream_t st) {
+  ps::Args a{};
+  a.t = t;
+  a.sp = sp;
+  a.env = env;
+  a.beta = in->beta;
+  a.invalid = in->invalid_actions;
+  a.ds_out = t.ds_out;
   a.ncap = ncap;
   a.trace = g_ps_trace;
-  const size_t smem = ps::smem_bytes(ncap, env.size);
   // (cudaFuncAttributeMaxDynamicSharedMemorySize was raised to the largest eligible size by persistent_eligible)
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(ceil_div(t.B, ps::kTile) * ps::kCtas);
-  cfg.blockDim = dim3(ps::kThreads);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = ps::kCtas;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  cudaError_t le = cudaLaunchKernelEx(&cfg, ps::ds_search_kernel, a);
-  if (le != cudaSuccess) return cuda_fail(le, "ds_search_kernel launch");
+  ps::ds_search_kernel<<<ceil_div(t.B, ps::kSlots), ps::kThreads, ps::smem_bytes(ncap, env.size), st>>>(a);
+  EAZ_CHECK_LAUNCH("ds_search_kernel");
   return 0;
 }
 
@@ -950,7 +959,7 @@ static int run_search(const Tree& t, const SearchParams& sp, const EnvDesc& env,
     if (!flags && tw && tw->w2_ck16[0] && persistent_eligible(t.B, t.N, t.A, sp.flags, env, mlp_mode, &ncap)) {  // ONE launch runs all sp.n simulations
       {
         ProfScope ps_scope(CLS_SELECT, st);
-        if (int rc = launch_persistent(t, sp, env, net, *tw, in, lhead, ncap, st)) return rc;
+        if (int rc = launch_persistent(t, sp, env, in, ncap, st)) return rc;
       }
       ProfScope pf(CLS_FINAL, st);
       finalize_kernel<G, J><<<grid, 128, 0, st>>>(t, sp, in->beta, in->invalid_actions, so, (int)(in->gumbel == nullptr));
@@ -1106,7 +1115,7 @@ int eaz_mlp_forward_states(const eaz_fc_params* net, const eaz_env* env, const e
 static size_t layout_bytes(const eaz_search_config* cfg, const EnvDesc& d, int batch) {
   Layout L;
   make_layout(batch, cfg->num_simulations + 1, d.num_actions, d.compact_bytes, (cfg->max_num_considered_actions + 1) * cfg->num_simulations,
-              d.obs_dim, wimg_bytes_for(cfg->mlp_mode, d), cfg->max_depth > 0 ? cfg->max_depth : cfg->num_simulations, &L);
+              d.obs_dim, wimg_bytes_for(cfg->mlp_mode, d), ds_out_bytes(cfg->mlp_mode, d), cfg->max_depth > 0 ? cfg->max_depth : cfg->num_simulations, &L);
   return L.total;
 }
 // EAZ_FLAG_STREAMS(k): the batch is cut into up to k sub-batches of whole 128-tree tiles; returns their sizes (count in *parts)
@@ -1146,7 +1155,7 @@ int32_t eaz_search_num_launches(const eaz_search_config* cfg, const eaz_env* env
   int sizes[8], parts = 1;
   if (cfg->batch >= 1) sub_batches(cfg, sizes, &parts);  // EAZ_FLAG_STREAMS: every sub-batch launches its own sequence
   if (cfg->batch >= 1 && persistent_eligible(cfg->batch, cfg->num_simulations + 1, d.num_actions, cfg->flags, d, cfg->mlp_mode, nullptr))
-    return 1 + 2 + (build_tables ? prep : 0) + 1 + 1;  // memset + pack + root init + [tables] + ONE persistent kernel + finalize (+1 with a fused root)
+    return 1 + 2 + (build_tables ? prep + 1 : 0) + 1 + 1;  // memset + pack + root init + [tables + output table] + ONE persistent kernel + finalize (+1 with a fused root)
   return parts * (1 + 2 + (build_tables ? prep : 0) + per_sim * cfg->num_simulations + 1 + 1);
 }
 
@@ -1158,7 +1167,7 @@ static int search_one(const eaz_search_config* cfg, const eaz_search_inputs* in,
   if (int rc = check_search(cfg, in, out, &env, &net)) return rc;
   const int B = cfg->batch, n = cfg->num_simulations, N = n + 1, A = env.num_actions, S = env.compact_bytes;
   Layout L;
-  make_layout(B, N, A, S, (cfg->max_num_considered_actions + 1) * n, env.obs_dim, wimg_bytes_for(cfg->mlp_mode, env),
+  make_layout(B, N, A, S, (cfg->max_num_considered_actions + 1) * n, env.obs_dim, wimg_bytes_for(cfg->mlp_mode, env), ds_out_bytes(cfg->mlp_mode, env),
               cfg->max_depth > 0 ? cfg->max_depth : n, &L);
   if (!workspace || workspace_bytes < L.total || ((uintptr_t)workspace & 255)) {
     set_error("search workspace must be >= %zu bytes and 256-byte aligned (got %zu)", L.total, workspace_bytes);
@@ -1185,6 +1194,8 @@ static int search_one(const eaz_search_config* cfg, const eaz_search_inputs* in,
   if (cfg->mlp_mode == EAZ_MLP_TENSOR) {
     const int lhead = cfg->exploration ? EAZ_HEAD_EXPLORE : EAZ_HEAD_EXPLOIT;
     if (int rc = prepare_tensor_weights(net, env, (1 << EAZ_HEAD_VALUE) | (1 << EAZ_HEAD_UBE) | (1 << lhead), t.wimg, &tw, st, build_tables)) return rc;
+    if (build_tables && persistent_eligible(B, N, A, cfg->flags, env, cfg->mlp_mode, nullptr))
+      if (int rc = launch_output_table(t, env, net, tw, lhead, st)) return rc;
   }
   }
 
@@ -1278,7 +1289,7 @@ int eaz_search_gumbel(const eaz_search_config* cfg, const eaz_search_inputs* in,
     if (cfg->batch >= 1 && in->env && make_env_desc(in->env, &d) == 0)
       persistent = persistent_eligible(cfg->batch, cfg->num_simulations + 1, d.num_actions, cfg->flags, d, cfg->mlp_mode, nullptr);
   }
-  if (parts <= 1 || tl_prof != nullptr || persistent) {  // (the persistent kernel's clusters are independent chains already: nothing to split)
+  if (parts <= 1 || tl_prof != nullptr || persistent) {  // (the persistent kernel's CTAs are independent chains already: nothing to split)
     eaz_search_config c = *cfg;
     c.flags = (c.flags & ~(kFlagManyTrees | kFlagSqFused)) | (cfg->batch >= kManyTrees ? kFlagManyTrees : 0) | (subleq_fused_for(cfg->batch) ? kFlagSqFused : 0);
     return search_one(&c, in, out, workspace, workspace_bytes, stream);
@@ -1395,7 +1406,7 @@ int eaz_search_numeric_status(const eaz_search_config* cfg, const eaz_env* env_i
   for (int p = 0; p < parts; ++p) {
     Layout L;
     make_layout(sizes[p], cfg->num_simulations + 1, env.num_actions, env.compact_bytes, (cfg->max_num_considered_actions + 1) * cfg->num_simulations,
-                env.obs_dim, wbytes, cfg->max_depth > 0 ? cfg->max_depth : cfg->num_simulations, &L);
+                env.obs_dim, wbytes, ds_out_bytes(cfg->mlp_mode, env), cfg->max_depth > 0 ? cfg->max_depth : cfg->num_simulations, &L);
     if (ws_off + L.total > workspace_bytes) break;
     const uint8_t* ns = (const uint8_t*)workspace + ws_off + L.off[24] + wbytes - 256;
     uint32_t f = 0;
@@ -1459,8 +1470,8 @@ int eaz_search_gumbel_profiled(const eaz_search_config* cfg, const eaz_search_in
   return rc;
 }
 
-// Debug hook (not in the public header): device buffer of num_simulations * 8 u64 receiving the per-simulation milestones of cluster 0
-// of the persistent search kernel (psearch.cuh: Trace).
+// Debug hook (not in the public header): device buffer of num_simulations * 128 u64 receiving the per-simulation milestones of the
+// tree warps of CTA 0 of the persistent search kernel (psearch.cuh: Trace).
 void eaz_debug_set_ps_trace(unsigned long long* device_buffer) { eaz::g_ps_trace = device_buffer; }
 
 // Debug hook (not in the public header): device buffer of (n+1)*B*8 int64 receiving per-tree section stamps of tree_step_kernel.

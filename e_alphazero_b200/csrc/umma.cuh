@@ -78,49 +78,6 @@ __device__ __forceinline__ void mbar_wait_warp(uint64_t* bar, uint32_t parity) {
     if (__any_sync(0xffffffffu, ok != 0)) break;
   }
 }
-// The same waits for roles that are IDLE for microseconds (a network role during the tree phase, a tree warp during the network
-// phase): between polls the warp sleeps, so that it does not take issue slots from the warps of the other phase that share its
-// scheduler (psearch.cuh: about a third of the kernel's 400 M warp instructions were polls).
-#ifndef EAZ_WAIT_HINT_NS
-#define EAZ_WAIT_HINT_NS 0
-#endif
-// try_wait with a suspend-time hint: the hardware parks the thread until the phase completes or the hint expires, so a waiting role
-// neither issues polls nor wakes up late (measurement option EAZ_WAIT_HINT_NS: replaces the sleep between polls below).
-__device__ __forceinline__ bool mbar_try_wait_hint(uint64_t* bar, uint32_t parity, uint32_t hint_ns) {
-  uint32_t ok;
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n"
-      "selp.u32 %0, 1, 0, p;\n"
-      "}\n"
-      : "=r"(ok)
-      : "r"(smem_u32(bar)), "r"(parity), "r"(hint_ns)
-      : "memory");
-  return ok != 0;
-}
-__device__ __forceinline__ void mbar_wait_warp_idle(uint64_t* bar, uint32_t parity, unsigned ns) {
-  const bool poller = (threadIdx.x & 31) == 0;
-  while (true) {
-    uint32_t ok = 0;
-#if EAZ_WAIT_HINT_NS
-    if (poller) ok = mbar_try_wait_hint(bar, parity, EAZ_WAIT_HINT_NS) ? 1u : 0u;
-    if (__any_sync(0xffffffffu, ok != 0)) break;
-#else
-    if (poller) ok = mbar_try_wait(bar, parity) ? 1u : 0u;
-    if (__any_sync(0xffffffffu, ok != 0)) break;
-    __nanosleep(ns);
-#endif
-  }
-}
-__device__ __forceinline__ void mbar_wait_idle(uint64_t* bar, uint32_t parity, unsigned ns) {
-#if EAZ_WAIT_HINT_NS
-  while (!mbar_try_wait_hint(bar, parity, EAZ_WAIT_HINT_NS)) {
-  }
-#else
-  while (!mbar_try_wait(bar, parity)) __nanosleep(ns);
-#endif
-}
 // One lane of the (converged) warp.  tcgen05.mma issued under `if (elect_one())` from warp-uniform values takes its descriptors from
 // uniform registers; inside an `if (lane == 0)` region the compiler wraps every tcgen05.mma in an ELECT / R2UR.BROADCAST loop
 // (~100 cycles per instruction).

@@ -1,4 +1,5 @@
-"""Per-simulation timeline of cluster 0 of the persistent search kernel (psearch.cuh: Trace; globaltimer ns) -- a measurement aid.
+"""Per-simulation timeline of the 16 tree warps of CTA 0 of the persistent search kernel (psearch.cuh: Trace; globaltimer ns) -- a
+measurement aid.
 Usage (on a B200): python profiles/trace_psearch.py [c2|c4] [num_simulations]"""
 import ctypes as C
 import os
@@ -24,7 +25,7 @@ states = ops.env_init(env, B)
 for _ in range(4):
     states, _ = runner.step(states)
 torch.cuda.synchronize()
-buf = torch.zeros(n * 200 + 256, dtype=torch.int64, device="cuda")
+buf = torch.zeros(n * 128 + 256, dtype=torch.int64, device="cuda")
 lib = _lib.load()
 lib.eaz_debug_set_ps_trace(C.c_void_p(buf.data_ptr()))
 e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -33,45 +34,34 @@ states, _ = runner.step(states)
 e1.record()
 torch.cuda.synchronize()
 lib.eaz_debug_set_ps_trace(None)
-raw = buf.cpu().numpy().astype(np.int64)
-t = raw[: n * 8].reshape(n, 8)
-names = ["cells_full", "A stored", "acc done", "outs sent", "out_full", "backward", "refresh", "published"]
-print(f"{desc}: step {e0.elapsed_time(e1):.3f} ms; cluster 0 per simulation, ns since the simulation's cells_full")
-print("  it " + " ".join(f"{nm:>10s}" for nm in names) + "   period")
-for it in range(n):
-    row = t[it] - t[it, 0]
-    period = (t[it + 1, 0] - t[it, 0]) if it + 1 < n else 0
-    if it < 6 or it % 8 == 0 or it >= n - 2:
-        print(f"{it:4d} " + " ".join(f"{int(v):10d}" for v in row) + f" {int(period):8d}")
-d = np.diff(t[:, 0])
-print(f"mean period {d.mean():.0f} ns (min {d.min()}, max {d.max()}); means since cells_full: " +
-      ", ".join(f"{nm} {np.mean(t[:-1, k] - t[:-1, 0]):.0f}" for k, nm in enumerate(names)))
-
-pub = raw[n * 8: n * 72].reshape(n, 64)
-Ls = raw[n * 72: n * 136].reshape(n, 64) & 0xFFFFFFFF
-print("per simulation: out_full -> publish of every tree warp of cluster 0 (ns): median / p90 / max, path length of the slowest warp, max path length")
-for it in range(0, n - 1, 4):
-    d = pub[it] - t[it, 4]
-    k = int(np.argmax(d))
-    print(f"{it:4d}  median {int(np.median(d)):6d}  p90 {int(np.percentile(d, 90)):6d}  max {int(d.max()):6d} (warp {k}, L {int(Ls[it, k])})  Lmax {int(Ls[it].max())}  "
-          f"next cells_full - last publish {int(t[it + 1, 0] - pub[it].max()):6d}")
-ch = raw[n * 136: n * 136 + 32].reshape(16, 2)
-print("simulation 8, head CTA 0, MMA warp: per chunk A ready / B ready (ns since cells_full)")
-print("  " + "  ".join(f"{c}:{int(ch[c, 0] - t[8, 0])}/{int(ch[c, 1] - t[8, 0])}" for c in range(16)))
-for it in (8, 12, 24):
-    d = (pub[it] - t[it, 4]) // 100
-    print(f"simulation {it}: out_full -> publish per tree warp (x100 ns), rows = CTAs 0..3; then path lengths")
-    for r in range(4):
-        print("   " + " ".join(f"{int(v):4d}" for v in d[16 * r:16 * r + 16]) + "   | " + " ".join(f"{int(v):2d}" for v in Ls[it, 16 * r:16 * r + 16]))
-
-seen = raw[n * 136 + 64: n * 200 + 64].reshape(n, 64)
-for it in (8, 12, 24):
-    print(f"simulation {it}: per tree warp, out_full seen (x100 ns after CTA 0 warp 0 saw it) / own tree phase = publish - seen (x100 ns)")
-    for r in range(4):
-        print("   " + " ".join(f"{int(a):3d}/{int(b):3d}" for a, b in zip((seen[it, 16 * r:16 * r + 16] - t[it, 4]) // 100, (pub[it, 16 * r:16 * r + 16] - seen[it, 16 * r:16 * r + 16]) // 100)))
-
-ga = raw[n * 200 + 64: n * 200 + 128].reshape(16, 4)
-print("simulation 8, head CTA 0, gather groups: per chunk loads issued / stage free / stored / fenced (ns since cells_full)")
-for c in range(16):
-    print(f"  chunk {c:2d} (group {c % 4}): " + " ".join(f"{int(v - t[8, 0]):6d}" for v in ga[c]) + f"   MMA warp saw A at {int(ch[c, 0] - t[8, 0])}")
-
+raw = buf.cpu().numpy().astype(np.int64)[: n * 128].reshape(n, 16, 8)
+L = raw[:, :, 5] & 0xFFFFFFFF
+direct = (raw[:, :, 5] >> 32) != 0
+# phases of simulation `it` of one warp: table wait + expand = expand done - staging done of it - 1; then backward, refresh, descent
+# (the next leaf's table load is issued at its end) and staging; period = descent done of it - descent done of it - 1
+ok = ~direct[1:] & ~direct[:-1] & (raw[1:, :, 3] > 0) & (raw[:-1, :, 4] > 0)
+cur, prev = raw[1:], raw[:-1]
+phases = {
+    "expand": cur[:, :, 0] - prev[:, :, 4],
+    "backward": cur[:, :, 1] - cur[:, :, 0],
+    "refresh": cur[:, :, 2] - cur[:, :, 1],
+    "descent": cur[:, :, 3] - cur[:, :, 2],
+    "stage": cur[:, :, 4] - cur[:, :, 3],
+}
+period = cur[:, :, 3] - prev[:, :, 3]
+print(f"{desc}: step {e0.elapsed_time(e1):.3f} ms; CTA 0, 16 tree warps x {n} simulations ({int(direct.sum())} warp-steps DIRECT)")
+print("per-simulation period and phases of a warp, ns (staged simulations whose predecessor was staged as well): mean / median / p90")
+for name, v in [("period", period)] + list(phases.items()):
+    x = v[ok]
+    print(f"  {name:9s} {x.mean():8.0f} {np.median(x):8.0f} {np.percentile(x, 90):8.0f}")
+print("  it  period (mean over warps)  " + " ".join(f"{k:>8s}" for k in phases) + "   Lmax")
+for it in range(1, n - 1):
+    if it < 6 or it % 8 == 0 or it >= n - 3:
+        m = ok[it - 1]
+        if not m.any():
+            continue
+        print(f"{it:4d} {period[it - 1][m].mean():10.0f}              " + " ".join(f"{v[it - 1][m].mean():8.0f}" for v in phases.values()) +
+              f"   {int(L[it].max()):4d}")
+dd = np.where(raw[:, :, 3] > 0, raw[:, :, 3], np.nan)  # (0: a DIRECT step)
+span = np.nanmax(dd, axis=1) - np.nanmin(dd, axis=1)
+print(f"spread of 'descent done' across the 16 warps of a simulation: mean {np.nanmean(span[1:-1]):.0f} ns (warps are not synchronised)")
