@@ -28,6 +28,7 @@ EXPORTS = [
     "eaz_reanalyze_targets",
     "eaz_convnet_workspace_bytes", "eaz_convnet_forward", "eaz_convnet_numeric_status",
     "eaz_priority_tree_bytes", "eaz_priority_init", "eaz_priority_add_step", "eaz_priority_set", "eaz_priority_sample", "eaz_priority_status",
+    "eaz_replay_add", "eaz_priority_sample_keyed", "eaz_priority_status_async",
 ]
 
 

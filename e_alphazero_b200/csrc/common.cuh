@@ -149,6 +149,27 @@ __host__ __device__ inline uint32_t ds_pack(int step, int col, int term, int tru
 #define EAZ_SQ_FLAG_TRUNC 2
 #define EAZ_SQ_FLAG_SOLVED 4
 
+// pgx.State leaves of env b -> its compact record at `out` (eaz_env_compact; the replay ring's add writes the same records)
+__device__ __forceinline__ void pack_state(const EnvDesc& env, const StateSoA& s, int b, uint8_t* out) {
+  const int term = s.terminated[b] != 0, trunc = s.truncated ? (s.truncated[b] != 0) : 0;
+  if (env.kind == EAZ_ENV_DEEPSEA) {
+    reinterpret_cast<uint32_t*>(out)[b] = ds_pack(s.step_count[b], s.col[b], term, trunc);
+    return;
+  }
+  const int S = env.compact_bytes, ws = env.ws;
+  uint8_t* o = out + (size_t)b * S;
+  uint16_t* h = reinterpret_cast<uint16_t*>(o);
+  for (int i = 0; i < 8; ++i) {
+    h[i] = (uint16_t)s.input_after[(size_t)b * 8 + i];
+    h[8 + i] = (uint16_t)s.output_after[(size_t)b * 8 + i];
+  }
+  h[16] = (uint16_t)s.step_count[b];
+  o[34] = (uint8_t)s.task[b];
+  o[35] = (uint8_t)((term ? EAZ_SQ_FLAG_TERM : 0) | (trunc ? EAZ_SQ_FLAG_TRUNC : 0) | (s.solved[b] ? EAZ_SQ_FLAG_SOLVED : 0));
+  o[36] = o[37] = o[38] = o[39] = 0;
+  for (int i = 0; i < S - EAZ_SQ_HDR; ++i) o[EAZ_SQ_HDR + i] = i < ws ? (uint8_t)s.memory[(size_t)b * ws + i] : 0;
+}
+
 // pgx.Env.step around DeepSea._step (deep_sea.py:59-81).  Returns the new
 // packed state; *reward receives rewards[0].
 __device__ __forceinline__ uint32_t deepsea_step(uint32_t s, int action, int N, const uint8_t* __restrict__ amap,

@@ -31,9 +31,14 @@
 //     index i, probability = eaz_div(w_i, total).  The draw counter advances once per call.  total == 0 (or not finite)
 //     sets EAZ_PRIORITY_EMPTY and every sample is index 0, probability 0.
 //
+// A keyed sample (eaz_priority_sample_keyed) is sample(K) with (seed, draw_ctr) := (key[0], key[1]) that writes nothing into
+// the buffer: no counter advance, no status bit.  eaz_replay_add's add_step is add_step(c) with c = the header's cursor.
+//
 // Kernels: add_step is one CTA (two rows of B leaves, then their ancestors level by level); set is a tag pass (atomicMax
 // of k per leaf: last occurrence wins), a leaf pass, and one launch per level above the leaves; sample is one warp per
-// sample (descent + gather of both slots' compact records and rewards) and a one-thread counter bump.  All latency-bound.
+// sample (descent + gather of both slots' compact records and rewards) and, unless keyed, a one-thread counter bump.
+// eaz_replay_add is a compaction kernel that writes ring row `cursor` (read from the header) followed by add_step with the
+// slot taken from the header, so the cursor never leaves the device.  All latency-bound.
 #include "common.cuh"
 
 #include <float.h>
@@ -129,13 +134,15 @@ __global__ void prio_init_kernel(PrioTree tr, float alpha, uint32_t seed) {
   *tr.hdr = h;
 }
 
+// c < 0: the slot is the header's cursor (eaz_replay_add: no host copy of the cursor exists)
 __global__ void __launch_bounds__(1024) prio_add_step_kernel(PrioTree tr, int c) {
-  __shared__ int s_ok;
+  __shared__ int s_ok, s_c;
   __shared__ float s_w;
   const int T = tr.T, B = tr.B;
-  const int rp = c == 0 ? T - 1 : c - 1;
   if (threadIdx.x == 0) {
     const PrioHeader h = *tr.hdr;
+    if (c < 0) c = h.cursor;
+    s_c = c;
     int ok = 1, cur = h.cursor, len = h.length;
     if (c == h.cursor) {
       cur = c + 1 == T ? 0 : c + 1;
@@ -150,6 +157,8 @@ __global__ void __launch_bounds__(1024) prio_add_step_kernel(PrioTree tr, int c)
   }
   __syncthreads();
   if (!s_ok) return;
+  c = s_c;
+  const int rp = c == 0 ? T - 1 : c - 1;
   const float w = s_w;
   for (int j = threadIdx.x; j < 2 * B; j += blockDim.x) {
     if (j < B) tr.lvl[0][(size_t)rp * B + j] = w;
@@ -213,11 +222,13 @@ __device__ __forceinline__ float prio_uniform(uint32_t seed, uint32_t ctr, uint3
   return __fmul_rn((float)(h >> 8), 5.9604644775390625e-08f);  // 24 random bits * 2^-24: exact
 }
 
-__global__ void __launch_bounds__(256) prio_sample_kernel(PrioTree tr, int K, const uint8_t* __restrict__ states,
-                                                          const float* __restrict__ rewards, int S, int32_t* __restrict__ out_idx,
-                                                          float* __restrict__ out_prob, uint8_t* __restrict__ first,
-                                                          float* __restrict__ first_r, uint8_t* __restrict__ second,
-                                                          float* __restrict__ second_r) {
+// key == nullptr: (seed, draw_ctr) from the header, an empty tree sets EAZ_PRIORITY_EMPTY (the caller bumps the counter).
+// key != nullptr (keyed sampling): (seed, draw_ctr) = (key[0], key[1]) and the tree is only read.
+__global__ void __launch_bounds__(256) prio_sample_kernel(PrioTree tr, int K, const uint32_t* __restrict__ key,
+                                                          const uint8_t* __restrict__ states, const float* __restrict__ rewards, int S,
+                                                          int32_t* __restrict__ out_idx, float* __restrict__ out_prob,
+                                                          uint8_t* __restrict__ first, float* __restrict__ first_r,
+                                                          uint8_t* __restrict__ second, float* __restrict__ second_r) {
   const int k = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (k >= K) return;
   const float* node = tr.root;
@@ -225,9 +236,10 @@ __global__ void __launch_bounds__(256) prio_sample_kernel(PrioTree tr, int K, co
   int i = 0;
   float prob = 0.0f;
   if (!(total > 0.0f && total <= FLT_MAX)) {
-    if (lane == 0) atomicOr(&tr.hdr->status, (uint32_t)EAZ_PRIORITY_EMPTY);
+    if (lane == 0 && key == nullptr) atomicOr(&tr.hdr->status, (uint32_t)EAZ_PRIORITY_EMPTY);
   } else {
-    float u = eaz_mul(eaz_div(eaz_add((float)k, prio_uniform(tr.hdr->seed, tr.hdr->draw_ctr, (uint32_t)k)), (float)K), total);
+    const uint32_t seed = key ? key[0] : tr.hdr->seed, ctr = key ? key[1] : tr.hdr->draw_ctr;
+    float u = eaz_mul(eaz_div(eaz_add((float)k, prio_uniform(seed, ctr, (uint32_t)k)), (float)K), total);
     int j = 0;
     float wc = 0.0f;
     for (int l = tr.L - 1; l >= 1; --l) {
@@ -264,6 +276,33 @@ __global__ void __launch_bounds__(256) prio_sample_kernel(PrioTree tr, int K, co
 }
 
 __global__ void prio_bump_kernel(PrioHeader* hdr) { hdr->draw_ctr += 1u; }
+
+// eaz_replay_add, first launch: the B states into ring row `cursor` (read on the device; prio_add_step_kernel advances it after)
+__global__ void replay_compact_kernel(EnvDesc env, StateSoA s, const PrioHeader* __restrict__ hdr, uint8_t* __restrict__ ring_states,
+                                      float* __restrict__ ring_rewards, int B) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  const size_t slot = (size_t)hdr->cursor;
+  pack_state(env, s, b, ring_states + slot * B * env.compact_bytes);
+  ring_rewards[slot * B + b] = s.rewards[b];
+}
+
+static int prio_sample_launch(void* tree, size_t tree_bytes, int32_t T, int32_t B, int32_t K, const uint32_t* key, const uint8_t* states,
+                              const float* rewards, int32_t S, int32_t* indices, float* probabilities, uint8_t* first, float* first_rewards,
+                              uint8_t* second, float* second_rewards, cudaStream_t s, const char* who) {
+  PrioTree tr;
+  if (int rc = prio_view(tree, tree_bytes, T, B, &tr, who)) return rc;
+  EAZ_CHECK_ARG(K >= 1 && K <= (1 << 24), "%s: K = %d outside [1, 2^24]", who, K);
+  EAZ_CHECK_ARG(indices && probabilities, "%s: NULL indices / probabilities", who);
+  if (states) {
+    EAZ_CHECK_ARG(S >= 1 && first && second, "%s: gathering needs S >= 1 and first / second buffers", who);
+    EAZ_CHECK_ARG(!rewards || (first_rewards && second_rewards), "%s: rewards given without first / second reward buffers", who);
+  }
+  prio_sample_kernel<<<ceil_div(K, 8), 256, 0, s>>>(tr, K, key, states, rewards, S, indices, probabilities, first, first_rewards, second,
+                                                    second_rewards);
+  EAZ_CHECK_LAUNCH("prio_sample_kernel");
+  return 0;
+}
 
 }  // namespace eaz
 
@@ -321,20 +360,48 @@ int eaz_priority_set(void* tree, size_t tree_bytes, int32_t T, int32_t B, const 
 int eaz_priority_sample(void* tree, size_t tree_bytes, int32_t T, int32_t B, int32_t K, const uint8_t* states, const float* rewards, int32_t S,
                         int32_t* indices, float* probabilities, uint8_t* first, float* first_rewards, uint8_t* second,
                         float* second_rewards, void* stream) {
-  PrioTree tr;
-  if (int rc = prio_view(tree, tree_bytes, T, B, &tr, "eaz_priority_sample")) return rc;
-  EAZ_CHECK_ARG(K >= 1 && K <= (1 << 24), "eaz_priority_sample: K = %d outside [1, 2^24]", K);
-  EAZ_CHECK_ARG(indices && probabilities, "eaz_priority_sample: NULL indices / probabilities");
-  if (states) {
-    EAZ_CHECK_ARG(S >= 1 && first && second, "eaz_priority_sample: gathering needs S >= 1 and first / second buffers");
-    EAZ_CHECK_ARG(!rewards || (first_rewards && second_rewards), "eaz_priority_sample: rewards given without first / second reward buffers");
-  }
   cudaStream_t s = (cudaStream_t)stream;
-  prio_sample_kernel<<<ceil_div(K, 8), 256, 0, s>>>(tr, K, states, rewards, S, indices, probabilities, first, first_rewards, second,
-                                                    second_rewards);
-  EAZ_CHECK_LAUNCH("prio_sample_kernel");
-  prio_bump_kernel<<<1, 1, 0, s>>>(tr.hdr);
+  if (int rc = prio_sample_launch(tree, tree_bytes, T, B, K, nullptr, states, rewards, S, indices, probabilities, first, first_rewards, second,
+                                  second_rewards, s, "eaz_priority_sample"))
+    return rc;
+  prio_bump_kernel<<<1, 1, 0, s>>>((PrioHeader*)tree);
   EAZ_CHECK_LAUNCH("prio_bump_kernel");
+  return 0;
+}
+
+int eaz_priority_sample_keyed(const void* tree, size_t tree_bytes, int32_t T, int32_t B, int32_t K, const uint32_t* key, const uint8_t* states,
+                              const float* rewards, int32_t S, int32_t* indices, float* probabilities, uint8_t* first, float* first_rewards,
+                              uint8_t* second, float* second_rewards, void* stream) {
+  EAZ_CHECK_ARG(key != nullptr, "eaz_priority_sample_keyed: NULL key (a device uint32[2])");
+  return prio_sample_launch(const_cast<void*>(tree), tree_bytes, T, B, K, key, states, rewards, S, indices, probabilities, first, first_rewards,
+                            second, second_rewards, (cudaStream_t)stream, "eaz_priority_sample_keyed");
+}
+
+int eaz_replay_add(const eaz_env* env, const eaz_state* state, uint8_t* ring_states, float* ring_rewards, void* tree, size_t tree_bytes,
+                   int32_t T, int32_t B, void* stream) {
+  EnvDesc d;
+  if (int rc = make_env_desc(env, &d)) return rc;
+  PrioTree tr;
+  if (int rc = prio_view(tree, tree_bytes, T, B, &tr, "eaz_replay_add")) return rc;
+  EAZ_CHECK_ARG(state && state->step_count && state->rewards && state->terminated, "eaz_replay_add: NULL state / step_count / rewards / terminated");
+  if (d.kind == EAZ_ENV_DEEPSEA) EAZ_CHECK_ARG(state->col != nullptr, "eaz_replay_add: col is NULL");
+  else EAZ_CHECK_ARG(state->memory && state->task && state->solved && state->input_after && state->output_after, "eaz_replay_add: NULL Subleq leaf");
+  EAZ_CHECK_ARG(ring_states && ring_rewards, "eaz_replay_add: NULL ring_states / ring_rewards");
+  cudaStream_t s = (cudaStream_t)stream;
+  replay_compact_kernel<<<ceil_div(B, 128), 128, 0, s>>>(d, soa_of(state), tr.hdr, ring_states, ring_rewards, B);
+  EAZ_CHECK_LAUNCH("replay_compact_kernel");
+  prio_add_step_kernel<<<1, 1024, 0, s>>>(tr, -1);
+  EAZ_CHECK_LAUNCH("prio_add_step_kernel");
+  return 0;
+}
+
+int eaz_priority_status_async(const void* tree, size_t tree_bytes, int32_t* flags_dev, void* stream) {
+  EAZ_CHECK_ARG(tree && tree_bytes >= sizeof(PrioHeader), "eaz_priority_status_async: NULL / short tree buffer");
+  EAZ_CHECK_ARG(flags_dev != nullptr, "eaz_priority_status_async: NULL flags");
+  if (cudaError_t e = cudaMemcpyAsync(flags_dev, (const uint8_t*)tree + offsetof(PrioHeader, status), sizeof(int32_t), cudaMemcpyDeviceToDevice,
+                                      (cudaStream_t)stream);
+      e != cudaSuccess)
+    return cuda_fail(e, "eaz_priority_status_async copy");
   return 0;
 }
 

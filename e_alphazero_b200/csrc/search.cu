@@ -175,23 +175,7 @@ struct SearchParams {
 __global__ void pack_states_kernel(EnvDesc env, StateSoA s, uint8_t* __restrict__ out, int B) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
-  const int term = s.terminated[b] != 0, trunc = s.truncated ? (s.truncated[b] != 0) : 0;
-  if (env.kind == EAZ_ENV_DEEPSEA) {
-    reinterpret_cast<uint32_t*>(out)[b] = ds_pack(s.step_count[b], s.col[b], term, trunc);
-    return;
-  }
-  const int S = env.compact_bytes, ws = env.ws;
-  uint8_t* o = out + (size_t)b * S;
-  uint16_t* h = reinterpret_cast<uint16_t*>(o);
-  for (int i = 0; i < 8; ++i) {
-    h[i] = (uint16_t)s.input_after[(size_t)b * 8 + i];
-    h[8 + i] = (uint16_t)s.output_after[(size_t)b * 8 + i];
-  }
-  h[16] = (uint16_t)s.step_count[b];
-  o[34] = (uint8_t)s.task[b];
-  o[35] = (uint8_t)((term ? EAZ_SQ_FLAG_TERM : 0) | (trunc ? EAZ_SQ_FLAG_TRUNC : 0) | (s.solved[b] ? EAZ_SQ_FLAG_SOLVED : 0));
-  o[36] = o[37] = o[38] = o[39] = 0;
-  for (int i = 0; i < S - EAZ_SQ_HDR; ++i) o[EAZ_SQ_HDR + i] = i < ws ? (uint8_t)s.memory[(size_t)b * ws + i] : 0;
+  pack_state(env, s, b, out);
 }
 
 // inverse of pack_states_kernel: compact records -> pgx.State leaves (replay-buffer decode, SURVEY 8f-3)

@@ -10,6 +10,9 @@
 //   eaz_mlp_forward_states   forward.apply(params, state, states.observation)            selfplay.py:89, reanalyze.py:67,90
 //   eaz_reanalyze_targets    the target arithmetic after the search                      reanalyze.py:86-129
 //   eaz_hash_update     BaseHash.update on the observations of a training batch           network/hashes.py:45-50, train.py:22
+//   eaz_replay_init / _add / _sample / _set_priorities / _status
+//                       flashbax make_prioritised_flat_buffer on the compact ring         main.py:217-225, 383-385, 413-414, 454
+//                       (csrc/replay.cu: the write cursor lives in the tree header, sampling is keyed and reads nothing it writes)
 //
 // XLA owns every buffer (results and the workspace are XLA-allocated), the stream comes from PlatformStream, errors travel as
 // ffi::Error carrying eaz_last_error().  The handlers hold no state.
@@ -30,6 +33,7 @@
 //     (module order fc_az_net/linear, linear_1 .. linear_11, fully_connected.py:49-81), then the hash state `binary_set` U8.
 #include <cuda_runtime_api.h>
 
+#include <algorithm>
 #include <cstdint>
 #include <string>
 
@@ -363,6 +367,179 @@ ffi::Error HashUpdateImpl(cudaStream_t stream, ffi::Buffer<ffi::F32> x, ffi::Buf
   return EazError(eaz_hash_update(x.typed_data(), (int32_t)dims[0], (int32_t)dims[1], bits, binary_set->typed_data(), stream), "eaz_hash_update");
 }
 
+// ------------------------------------------------------------------------------------------------ prioritised replay ring
+// flashbax's prioritised flat buffer (main.py:217-225, 383-385, 413-414, 454) as three arrays the program threads through its
+// calls: ring_states U8[T,B,S] (eaz_env_compact records), ring_rewards F32[T,B] and the sum tree U8[eaz_priority_tree_bytes(T, B)],
+// whose header holds the write cursor, so no call needs a host value.  Every check below runs before anything touches a device.
+
+// T >= 2, B >= 1, T * B < 2^31, and a 128-byte aligned tree buffer of at least eaz_priority_tree_bytes(T, B)
+template <typename Buf>
+ffi::Error CheckTree(const Buf& tree, int64_t T, int64_t B, size_t* bytes) {
+  if (T < 2 || B < 1 || T > INT32_MAX || B > INT32_MAX || T * B >= ((int64_t)1 << 31))
+    return Bad("replay: need T >= 2 time slots, B >= 1 envs and T * B < 2^31 (got T=" + std::to_string(T) + ", B=" + std::to_string(B) + ")");
+  const size_t need = eaz_priority_tree_bytes((int32_t)T, (int32_t)B);
+  if (need == 0) return EazError(EAZ_ERR_INVALID_ARG, "eaz_priority_tree_bytes");
+  if (tree.size_bytes() < need)
+    return Bad("replay: tree buffer of " + std::to_string(tree.size_bytes()) + " bytes, eaz_priority_tree_bytes = " + std::to_string(need));
+  if (reinterpret_cast<uintptr_t>(tree.untyped_data()) % 128 != 0) return Bad("replay: the tree buffer must be 128-byte aligned");
+  *bytes = tree.size_bytes();
+  return ffi::Error::Success();
+}
+
+// ring_states [T,B,S] and ring_rewards [T,B] -> T, B, S
+template <typename BufS, typename BufR>
+ffi::Error RingDims(const BufS& states, const BufR& rewards, int64_t* T, int64_t* B, int64_t* S) {
+  const auto ds = states.dimensions();
+  const auto dr = rewards.dimensions();
+  if (ds.size() != 3 || dr.size() != 2 || dr[0] != ds[0] || dr[1] != ds[1]) return Bad("replay: ring_states must be [T, B, S] and ring_rewards [T, B]");
+  *T = ds[0], *B = ds[1], *S = ds[2];
+  return ffi::Error::Success();
+}
+
+// S must be the env's compact record size
+ffi::Error CheckRecord(const eaz_env& env, int64_t S) {
+  const int32_t cb = eaz_env_compact_bytes(&env);
+  if (cb <= 0) return EazError(EAZ_ERR_INVALID_ARG, "eaz_env_compact_bytes");
+  if (S != cb) return Bad("replay: ring_states must be [T, B, eaz_env_compact_bytes = " + std::to_string(cb) + "]");
+  return ffi::Error::Success();
+}
+
+// the state leaves starting at src[first] hold exactly n envs each
+int64_t LeafElems(const eaz_env& env, size_t k) {  // elements per env of leaf k (eaz_state order)
+  if (k < kCommonLeaves || env.kind == EAZ_ENV_DEEPSEA) return 1;
+  return k == kCommonLeaves ? env.word_size : k >= kCommonLeaves + 3 ? EAZ_SUBLEQ_IO_LEN : 1;
+}
+ffi::Error CheckLeafRows(ffi::RemainingArgs& args, size_t first, const eaz_env& env, int64_t n) {
+  for (size_t k = 0; k < NumLeaves(env); ++k) {
+    auto b = args.get<ffi::AnyBuffer>(first + k);
+    if (!b.has_value()) return b.error();
+    if ((int64_t)b->element_count() != n * LeafElems(env, k)) return Bad("replay: state leaf " + std::to_string(k) + " does not hold " + std::to_string(n) + " envs");
+  }
+  return ffi::Error::Success();
+}
+ffi::Error CheckLeafRows(ffi::RemainingRets& rets, size_t first, const eaz_env& env, int64_t n) {
+  for (size_t k = 0; k < NumLeaves(env); ++k) {
+    auto b = rets.get<ffi::AnyBuffer>(first + k);
+    if (!b.has_value()) return b.error();
+    if ((int64_t)(*b)->element_count() != n * LeafElems(env, k)) return Bad("replay: result leaf " + std::to_string(k) + " does not hold " + std::to_string(n) + " envs");
+  }
+  return ffi::Error::Success();
+}
+
+// the functional form of an aliased update: without input_output_aliases the result starts as a copy of the input
+ffi::Error CopyUnlessAliased(void* dst, const void* src, size_t bytes, cudaStream_t stream) {
+  if (dst == src || bytes == 0) return ffi::Error::Success();
+  const cudaError_t e = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, stream);
+  if (e != cudaSuccess) return ffi::Error(ffi::ErrorCode::kInternal, std::string("replay copy: ") + cudaGetErrorString(e));
+  return ffi::Error::Success();
+}
+
+// rets : ring_states U8[T,B,S], ring_rewards F32[T,B] (both zeroed), tree U8[eaz_priority_tree_bytes(T, B)]
+ffi::Error ReplayInitImpl(cudaStream_t stream, ffi::ResultBuffer<ffi::U8> ring_states, ffi::ResultBuffer<ffi::F32> ring_rewards,
+                          ffi::ResultBuffer<ffi::U8> tree, int32_t T, int32_t B, float priority_exponent, int32_t seed) {
+  size_t tree_bytes = 0;
+  EAZ_FFI_TRY(CheckTree(*tree, T, B, &tree_bytes));
+  int64_t t, b, S;
+  EAZ_FFI_TRY(RingDims(*ring_states, *ring_rewards, &t, &b, &S));
+  if (t != T || b != B) return Bad("EazReplayInit: ring_states must be [T, B, S] and ring_rewards [T, B]");
+  if (!(priority_exponent >= 0.0f && priority_exponent <= 1.0f)) return Bad("EazReplayInit: priority_exponent must lie in [0, 1]");
+  cudaError_t e = cudaMemsetAsync(ring_states->untyped_data(), 0, ring_states->size_bytes(), stream);
+  if (e == cudaSuccess) e = cudaMemsetAsync(ring_rewards->untyped_data(), 0, ring_rewards->size_bytes(), stream);
+  if (e != cudaSuccess) return ffi::Error(ffi::ErrorCode::kInternal, std::string("ring memset: ") + cudaGetErrorString(e));
+  return EazError(eaz_priority_init(tree->untyped_data(), tree_bytes, T, B, priority_exponent, (uint32_t)seed, stream), "eaz_priority_init");
+}
+
+// args : action_map, ring_states_in U8[T,B,S], ring_rewards_in F32[T,B], tree_in U8, then the state leaves of the B envs
+// rets : ring_states, ring_rewards, tree (alias each to its input; otherwise the inputs are copied first)
+ffi::Error ReplayAddImpl(cudaStream_t stream, ffi::AnyBuffer action_map, ffi::Buffer<ffi::U8> states_in, ffi::Buffer<ffi::F32> rewards_in,
+                         ffi::Buffer<ffi::U8> tree_in, ffi::RemainingArgs leaves, ffi::ResultBuffer<ffi::U8> ring_states,
+                         ffi::ResultBuffer<ffi::F32> ring_rewards, ffi::ResultBuffer<ffi::U8> tree, int32_t env_kind, int32_t size,
+                         int32_t word_size, int32_t binary_encoding, int32_t reward_fn) {
+  const eaz_env env = MakeEnv(env_kind, size, word_size, binary_encoding, reward_fn, action_map.untyped_data());
+  int64_t T, B, S;
+  EAZ_FFI_TRY(RingDims(states_in, rewards_in, &T, &B, &S));
+  size_t in_bytes = 0, tree_bytes = 0;
+  EAZ_FFI_TRY(CheckTree(tree_in, T, B, &in_bytes));
+  EAZ_FFI_TRY(CheckTree(*tree, T, B, &tree_bytes));
+  EAZ_FFI_TRY(CheckRecord(env, S));
+  if (ring_states->size_bytes() != states_in.size_bytes() || ring_rewards->size_bytes() != rewards_in.size_bytes() || tree_bytes != in_bytes)
+    return Bad("EazReplayAdd: each result must have the shape of its input");
+  if (leaves.size() != NumLeaves(env)) return Bad("EazReplayAdd: wrong number of state leaves");
+  EAZ_FFI_TRY(CheckLeafRows(leaves, 0, env, B));
+  size_t i = 0;
+  eaz_state st;
+  EAZ_FFI_TRY(ReadStateArgs(leaves, &i, env, B, &st));
+  EAZ_FFI_TRY(CopyUnlessAliased(ring_states->untyped_data(), states_in.untyped_data(), states_in.size_bytes(), stream));
+  EAZ_FFI_TRY(CopyUnlessAliased(ring_rewards->untyped_data(), rewards_in.untyped_data(), rewards_in.size_bytes(), stream));
+  EAZ_FFI_TRY(CopyUnlessAliased(tree->untyped_data(), tree_in.untyped_data(), in_bytes, stream));
+  return EazError(eaz_replay_add(&env, &st, ring_states->typed_data(), ring_rewards->typed_data(), tree->untyped_data(), tree_bytes, (int32_t)T,
+                                 (int32_t)B, stream),
+                  "eaz_replay_add");
+}
+
+// args : action_map, ring_states U8[T,B,S], ring_rewards F32[T,B], tree U8, key U32[2] = (seed, draw counter); none is aliased or written
+// rets : indices S32[K], probabilities F32[K], the decoded `first` state leaves (K envs), the `second` state leaves,
+//        scratch U8[2 K (S + 4) + 16] (the gathered compact records and rewards)
+ffi::Error ReplaySampleImpl(cudaStream_t stream, ffi::AnyBuffer action_map, ffi::Buffer<ffi::U8> ring_states, ffi::Buffer<ffi::F32> ring_rewards,
+                            ffi::Buffer<ffi::U8> tree, ffi::Buffer<ffi::U32> key, ffi::ResultBuffer<ffi::S32> indices,
+                            ffi::ResultBuffer<ffi::F32> probabilities, ffi::RemainingRets out, int32_t env_kind, int32_t size, int32_t word_size,
+                            int32_t binary_encoding, int32_t reward_fn, int32_t K) {
+  const eaz_env env = MakeEnv(env_kind, size, word_size, binary_encoding, reward_fn, action_map.untyped_data());
+  int64_t T, B, S;
+  EAZ_FFI_TRY(RingDims(ring_states, ring_rewards, &T, &B, &S));
+  size_t tree_bytes = 0;
+  EAZ_FFI_TRY(CheckTree(tree, T, B, &tree_bytes));
+  EAZ_FFI_TRY(CheckRecord(env, S));
+  if (K < 1 || K > (1 << 24)) return Bad("EazReplaySample: K = " + std::to_string(K) + " outside [1, 2^24]");
+  if (key.element_count() != 2) return Bad("EazReplaySample: key must be U32[2]");
+  if ((int64_t)indices->element_count() != K || (int64_t)probabilities->element_count() != K) return Bad("EazReplaySample: indices / probabilities must be [K]");
+  const size_t nl = NumLeaves(env);
+  if (out.size() != 2 * nl + 1) return Bad("EazReplaySample: wrong number of results (first leaves, second leaves, scratch)");
+  EAZ_FFI_TRY(CheckLeafRows(out, 0, env, K));
+  EAZ_FFI_TRY(CheckLeafRows(out, nl, env, K));
+  size_t j = 0;
+  eaz_state first, second;
+  EAZ_FFI_TRY(ReadStateRets(out, &j, env, K, &first));
+  EAZ_FFI_TRY(ReadStateRets(out, &j, env, K, &second));
+  auto scratch = out.get<ffi::AnyBuffer>(j);
+  if (!scratch.has_value()) return scratch.error();
+  void* ws = AlignUp((*scratch)->untyped_data(), 16);
+  const size_t ws_bytes = (*scratch)->size_bytes() - std::min((*scratch)->size_bytes(), (size_t)((uint8_t*)ws - (uint8_t*)(*scratch)->untyped_data()));
+  if (ws_bytes < (size_t)2 * K * (S + 4)) return Bad("EazReplaySample: scratch must hold 2 K (S + 4) + 16 bytes");
+  float* first_r = static_cast<float*>(ws);
+  float* second_r = first_r + K;
+  uint8_t* first_c = reinterpret_cast<uint8_t*>(second_r + K);
+  uint8_t* second_c = first_c + (size_t)K * S;
+  EAZ_FFI_TRY(EazError(eaz_priority_sample_keyed(tree.untyped_data(), tree_bytes, (int32_t)T, (int32_t)B, K, key.typed_data(),
+                                                 ring_states.typed_data(), ring_rewards.typed_data(), (int32_t)S, indices->typed_data(),
+                                                 probabilities->typed_data(), first_c, first_r, second_c, second_r, stream),
+                       "eaz_priority_sample_keyed"));
+  EAZ_FFI_TRY(EazError(eaz_env_uncompact(&env, first_c, first_r, &first, K, stream), "eaz_env_uncompact"));
+  return EazError(eaz_env_uncompact(&env, second_c, second_r, &second, K, stream), "eaz_env_uncompact");
+}
+
+// args : indices S32[K], priorities F32[K], tree_in U8;  rets : tree (alias it to tree_in)
+ffi::Error ReplaySetPrioritiesImpl(cudaStream_t stream, ffi::Buffer<ffi::S32> indices, ffi::Buffer<ffi::F32> priorities, ffi::Buffer<ffi::U8> tree_in,
+                                   ffi::ResultBuffer<ffi::U8> tree, int32_t T, int32_t B) {
+  size_t in_bytes = 0, tree_bytes = 0;
+  EAZ_FFI_TRY(CheckTree(tree_in, T, B, &in_bytes));
+  EAZ_FFI_TRY(CheckTree(*tree, T, B, &tree_bytes));
+  if (tree_bytes != in_bytes) return Bad("EazReplaySetPriorities: the tree result must have the shape of tree_in");
+  const size_t K = indices.element_count();
+  if (priorities.element_count() != K) return Bad("EazReplaySetPriorities: indices and priorities differ in length");
+  if (K > (size_t)INT32_MAX) return Bad("EazReplaySetPriorities: more than 2^31 - 1 entries");
+  EAZ_FFI_TRY(CopyUnlessAliased(tree->untyped_data(), tree_in.untyped_data(), in_bytes, stream));
+  return EazError(eaz_priority_set(tree->untyped_data(), tree_bytes, T, B, indices.typed_data(), priorities.typed_data(), (int32_t)K, stream),
+                  "eaz_priority_set");
+}
+
+// args : tree U8;  rets : flags S32[1], the sticky EAZ_PRIORITY_* bits (copied on the stream, no synchronisation)
+ffi::Error ReplayStatusImpl(cudaStream_t stream, ffi::Buffer<ffi::U8> tree, ffi::ResultBuffer<ffi::S32> flags) {
+  if (reinterpret_cast<uintptr_t>(tree.untyped_data()) % 128 != 0) return Bad("replay: the tree buffer must be 128-byte aligned");
+  if (flags->element_count() != 1) return Bad("EazReplayStatus: flags must be S32[1]");
+  return EazError(eaz_priority_status_async(tree.untyped_data(), tree.size_bytes(), flags->typed_data(), stream), "eaz_priority_status_async");
+}
+
 }  // namespace
 
 #define EAZ_ENV_ATTRS() \
@@ -481,3 +658,57 @@ XLA_FFI_DEFINE_HANDLER_SYMBOL(EazHashUpdate, HashUpdateImpl,
                                   .Arg<ffi::Buffer<ffi::U8>>()   // binary_set_in
                                   .Ret<ffi::Buffer<ffi::U8>>()   // binary_set
                                   .Attr<int32_t>("bits"));
+
+XLA_FFI_DEFINE_HANDLER_SYMBOL(EazReplayInit, ReplayInitImpl,
+                              ffi::Ffi::Bind()
+                                  .Ctx<ffi::PlatformStream<cudaStream_t>>()
+                                  .Ret<ffi::Buffer<ffi::U8>>()   // ring_states
+                                  .Ret<ffi::Buffer<ffi::F32>>()  // ring_rewards
+                                  .Ret<ffi::Buffer<ffi::U8>>()   // tree
+                                  .Attr<int32_t>("T")
+                                  .Attr<int32_t>("B")
+                                  .Attr<float>("priority_exponent")
+                                  .Attr<int32_t>("seed"));
+
+XLA_FFI_DEFINE_HANDLER_SYMBOL(EazReplayAdd, ReplayAddImpl,
+                              ffi::Ffi::Bind()
+                                  .Ctx<ffi::PlatformStream<cudaStream_t>>()
+                                  .Arg<ffi::AnyBuffer>()         // action_map
+                                  .Arg<ffi::Buffer<ffi::U8>>()   // ring_states_in
+                                  .Arg<ffi::Buffer<ffi::F32>>()  // ring_rewards_in
+                                  .Arg<ffi::Buffer<ffi::U8>>()   // tree_in
+                                  .RemainingArgs()               // state leaves
+                                  .Ret<ffi::Buffer<ffi::U8>>()   // ring_states
+                                  .Ret<ffi::Buffer<ffi::F32>>()  // ring_rewards
+                                  .Ret<ffi::Buffer<ffi::U8>>()   // tree
+                                  EAZ_ENV_ATTRS());
+
+XLA_FFI_DEFINE_HANDLER_SYMBOL(EazReplaySample, ReplaySampleImpl,
+                              ffi::Ffi::Bind()
+                                  .Ctx<ffi::PlatformStream<cudaStream_t>>()
+                                  .Arg<ffi::AnyBuffer>()         // action_map
+                                  .Arg<ffi::Buffer<ffi::U8>>()   // ring_states
+                                  .Arg<ffi::Buffer<ffi::F32>>()  // ring_rewards
+                                  .Arg<ffi::Buffer<ffi::U8>>()   // tree
+                                  .Arg<ffi::Buffer<ffi::U32>>()  // key
+                                  .Ret<ffi::Buffer<ffi::S32>>()  // indices
+                                  .Ret<ffi::Buffer<ffi::F32>>()  // probabilities
+                                  .RemainingRets()               // first leaves, second leaves, scratch
+                                  EAZ_ENV_ATTRS()
+                                  .Attr<int32_t>("K"));
+
+XLA_FFI_DEFINE_HANDLER_SYMBOL(EazReplaySetPriorities, ReplaySetPrioritiesImpl,
+                              ffi::Ffi::Bind()
+                                  .Ctx<ffi::PlatformStream<cudaStream_t>>()
+                                  .Arg<ffi::Buffer<ffi::S32>>()  // indices
+                                  .Arg<ffi::Buffer<ffi::F32>>()  // priorities
+                                  .Arg<ffi::Buffer<ffi::U8>>()   // tree_in
+                                  .Ret<ffi::Buffer<ffi::U8>>()   // tree
+                                  .Attr<int32_t>("T")
+                                  .Attr<int32_t>("B"));
+
+XLA_FFI_DEFINE_HANDLER_SYMBOL(EazReplayStatus, ReplayStatusImpl,
+                              ffi::Ffi::Bind()
+                                  .Ctx<ffi::PlatformStream<cudaStream_t>>()
+                                  .Arg<ffi::Buffer<ffi::U8>>()   // tree
+                                  .Ret<ffi::Buffer<ffi::S32>>());  // flags

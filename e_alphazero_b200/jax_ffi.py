@@ -12,6 +12,7 @@ Call shapes mirror the reference (file:line under /root/reference/src):
     forward_states(...)                  selfplay.py:89, reanalyze.py:67,90
     reanalyze_targets(...)               reanalyze.py:86-129
     hash_update(...)                     train.py:22 (network/hashes.py:45-50)
+    make_prioritised_flat_buffer(...)    main.py:217-225 (init / add / sample / set_priorities: main.py:383-385, 413-414, 454)
 """
 from __future__ import annotations
 
@@ -32,7 +33,9 @@ _eaz = ctypes.CDLL(os.path.join(_HERE, "libeaz_b200.so"), mode=ctypes.RTLD_GLOBA
 _shim = ctypes.CDLL(os.path.join(_HERE, "libeaz_xla_ffi.so"))
 for _name, _sym in (("eaz_search", "EazSearch"), ("eaz_env_step", "EazEnvStep"), ("eaz_env_init", "EazEnvInit"),
                     ("eaz_mlp_forward_states", "EazMlpForwardStates"), ("eaz_reanalyze_targets", "EazReanalyzeTargets"),
-                    ("eaz_hash_update", "EazHashUpdate")):
+                    ("eaz_hash_update", "EazHashUpdate"),
+                    ("eaz_replay_init", "EazReplayInit"), ("eaz_replay_add", "EazReplayAdd"), ("eaz_replay_sample", "EazReplaySample"),
+                    ("eaz_replay_set_priorities", "EazReplaySetPriorities"), ("eaz_replay_status", "EazReplayStatus")):
     jax.ffi.register_ffi_target(_name, jax.ffi.pycapsule(getattr(_shim, _sym)), platform="CUDA")
 
 i32, f32 = np.int32, np.float32
@@ -198,3 +201,108 @@ def hash_update(binary_set, x, bits=24):
     """BaseHash.update (hashes.py:45-50): sets the bits of the rows of x (float32 [B, D]) in `binary_set` (donated)."""
     return jax.ffi.ffi_call("eaz_hash_update", jax.ShapeDtypeStruct(binary_set.shape, binary_set.dtype), input_output_aliases={1: 0})(
         x.astype(jnp.float32), binary_set, bits=i32(bits))
+
+
+# ------------------------------------------------------------------------------------------------ prioritised replay
+_LEAF_NAMES = {ENV_DEEPSEA: ["_step_count", "rewards", "terminated", "truncated", "_horizontal_position"],
+               ENV_SUBLEQ: ["_step_count", "rewards", "terminated", "truncated", "_memory_state", "_task", "_solved", "_example_input_after",
+                            "_example_output_after"]}
+
+
+def _leaf_types(env: EnvSpec, n):
+    """ShapeDtypeStructs of the state leaves of n envs, in eaz_state order"""
+    s = lambda *shape, dt=jnp.int32: jax.ShapeDtypeStruct((n,) + shape, dt)
+    common = [s(), s(1, dt=jnp.float32), s(dt=jnp.bool_), s(dt=jnp.bool_)]
+    if env.kind == ENV_DEEPSEA:
+        return common + [s()]
+    return common + [s(env.word_size), s(), s(dt=jnp.bool_), s(8), s(8)]
+
+
+class ReplayState(NamedTuple):
+    """The buffer state a jitted program threads through its steps: compact records [T,B,S], rewards [T,B] and the sum tree, whose
+    header holds the write cursor and length (csrc/replay.cu)."""
+    states: jax.Array
+    rewards: jax.Array
+    tree: jax.Array
+
+
+class PrioritisedSample(NamedTuple):
+    """flashbax's PrioritisedTrajectoryBufferSample: experience = (first, second), each a dict of pgx.State leaves for K envs
+    (`template_state.replace(**first)` makes it a pgx.State), indices int32 [K] (handles for set_priorities), probabilities [K]."""
+    experience: tuple
+    indices: jax.Array
+    probabilities: jax.Array
+
+
+class PrioritisedFlatBuffer(NamedTuple):
+    init: object
+    add: object
+    sample: object
+    set_priorities: object
+    can_sample: object
+    status: object
+
+
+def make_prioritised_flat_buffer(env: EnvSpec, max_length_time_axis, add_batch_size, sample_batch_size, priority_exponent=0.6):
+    """flashbax.make_prioritised_flat_buffer (main.py:217-225) on the compact ring, as pure functions of jax arrays:
+
+        init(template_state, seed) -> ReplayState          (seed: a Python int, it becomes an attribute)
+        add(rs, states) -> ReplayState                     one time step of the add_batch_size envs, at the device cursor
+        sample(rs, key) -> PrioritisedSample               sample_batch_size pairs drawn from key; rs is only read
+        set_priorities(rs, indices, priorities) -> ReplayState
+        can_sample(rs) -> bool[]                           at least two time steps stored
+        status(rs) -> int32[]                              the sticky EAZ_PRIORITY_* bits (0: nothing went wrong)
+
+    add and set_priorities alias their inputs to their results; donate `rs` at the jit boundary (donate_argnums) so that XLA
+    updates the three arrays in place instead of copying them."""
+    T, B, K = int(max_length_time_axis), int(add_batch_size), int(sample_batch_size)
+    from . import _abi  # ctypes mirrors of the POD structs (no torch)
+
+    e = _abi.EazEnv(env.kind, env.size, None, env.word_size, env.binary_encoding, env.reward_fn)
+    _eaz.eaz_priority_tree_bytes.restype = ctypes.c_size_t
+    S = int(_eaz.eaz_env_compact_bytes(ctypes.byref(e)))
+    tree_bytes = int(_eaz.eaz_priority_tree_bytes(T, B))
+    if S <= 0 or tree_bytes == 0:
+        raise ValueError(_eaz_error())
+    ring_types = [jax.ShapeDtypeStruct((T, B, S), jnp.uint8), jax.ShapeDtypeStruct((T, B), jnp.float32),
+                  jax.ShapeDtypeStruct((tree_bytes,), jnp.uint8)]
+    names = _LEAF_NAMES[env.kind]
+
+    def init(template_state=None, seed=0):
+        del template_state  # the ring stores compact records; its shapes come from env, T and B
+        out = jax.ffi.ffi_call("eaz_replay_init", ring_types)(T=i32(T), B=i32(B), priority_exponent=f32(priority_exponent),
+                                                              seed=i32(np.uint32(seed).view(np.int32)))
+        return ReplayState(*out)
+
+    def add(rs: ReplayState, states):
+        out = jax.ffi.ffi_call("eaz_replay_add", ring_types, input_output_aliases={1: 0, 2: 1, 3: 2})(
+            env.amap(), rs.states, rs.rewards, rs.tree, *state_leaves(env, states), **env.attrs())
+        return ReplayState(*out)
+
+    def sample(rs: ReplayState, key):
+        words = jax.random.bits(key, (2,), jnp.uint32)  # (seed, draw counter) of the contract's stratified draws
+        out_types = ([jax.ShapeDtypeStruct((K,), jnp.int32), jax.ShapeDtypeStruct((K,), jnp.float32)] + _leaf_types(env, K) +
+                     _leaf_types(env, K) + [jax.ShapeDtypeStruct((2 * K * (S + 4) + 16,), jnp.uint8)])
+        out = jax.ffi.ffi_call("eaz_replay_sample", out_types)(env.amap(), rs.states, rs.rewards, rs.tree, words, **env.attrs(), K=i32(K))
+        n = len(names)
+        first, second = dict(zip(names, out[2:2 + n])), dict(zip(names, out[2 + n:2 + 2 * n]))
+        return PrioritisedSample((first, second), out[0], out[1])
+
+    def set_priorities(rs: ReplayState, indices, priorities):
+        tree = jax.ffi.ffi_call("eaz_replay_set_priorities", ring_types[2], input_output_aliases={2: 0})(
+            indices.astype(jnp.int32).reshape(-1), priorities.astype(jnp.float32).reshape(-1), rs.tree, T=i32(T), B=i32(B))
+        return rs._replace(tree=tree)
+
+    def can_sample(rs: ReplayState):
+        length = jax.lax.bitcast_convert_type(rs.tree[20:24], jnp.int32)  # PrioHeader.length (bytes 20..23 of the header)
+        return length >= 2
+
+    def status(rs: ReplayState):
+        return jax.ffi.ffi_call("eaz_replay_status", jax.ShapeDtypeStruct((1,), jnp.int32))(rs.tree)[0]
+
+    return PrioritisedFlatBuffer(init, add, sample, set_priorities, can_sample, status)
+
+
+def _eaz_error():
+    _eaz.eaz_last_error.restype = ctypes.c_char_p
+    return _eaz.eaz_last_error().decode("utf-8", "replace")

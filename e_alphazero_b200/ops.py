@@ -281,6 +281,42 @@ def priority_status(tree) -> int:
     return int(flags.value)
 
 
+def replay_add(env: EnvSpec, st: dict, ring_states, ring_rewards, tree) -> None:
+    """eaz_replay_add: one time step of `st` into ring row `cursor` of ring_states [T,B,S] / ring_rewards [T,B], with the cursor read
+    and advanced on the device (no host copy of it exists, so a captured call appends at the current cursor on every replay)."""
+    import torch
+
+    T, B = ring_states.shape[0], ring_states.shape[1]
+    if _batch(st) != B or tuple(ring_rewards.shape) != (T, B) or ring_states.shape[2] != env.compact_bytes:
+        raise EazError("replay_add: ring_states must be [T, B, compact_bytes] and ring_rewards [T, B] for the B envs of the state")
+    e, s = env.struct(), state_struct(env, st)
+    check(load().eaz_replay_add(C.byref(e), C.byref(s), _ptr(ring_states, torch.uint8), _ptr(ring_rewards, torch.float32), _ptr(tree),
+                                C.c_size_t(tree.numel()), int(T), int(B), _stream()), "eaz_replay_add")
+
+
+def priority_sample_keyed(tree, T: int, B: int, key, indices, probabilities, states=None, rewards=None, first=None, first_rewards=None,
+                          second=None, second_rewards=None) -> None:
+    """eaz_priority_sample_keyed: as priority_sample with (seed, draw counter) = key, a uint32-valued int32 [2] device tensor; the
+    tree is only read."""
+    import torch
+
+    if key.numel() != 2:
+        raise EazError("priority_sample_keyed: key must hold two 32-bit words")
+    S = 0 if states is None else states.shape[-1]
+    check(load().eaz_priority_sample_keyed(_ptr(tree), C.c_size_t(tree.numel()), int(T), int(B), int(indices.numel()), _ptr(key, torch.int32),
+                                           _ptr(states, torch.uint8), _ptr(rewards, torch.float32), S, _ptr(indices, torch.int32),
+                                           _ptr(probabilities, torch.float32), _ptr(first, torch.uint8), _ptr(first_rewards, torch.float32),
+                                           _ptr(second, torch.uint8), _ptr(second_rewards, torch.float32), _stream()),
+          "eaz_priority_sample_keyed")
+
+
+def priority_status_async(tree, flags) -> None:
+    """eaz_priority_status_async: the sticky EAZ_PRIORITY_* word into the int32 [1] device tensor `flags`, without synchronising."""
+    import torch
+
+    check(load().eaz_priority_status_async(_ptr(tree), C.c_size_t(tree.numel()), _ptr(flags, torch.int32), _stream()), "eaz_priority_status_async")
+
+
 def subleq_test_cases(task: int, ws: int):
     import numpy as np
 

@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define EAZ_ABI_VERSION 3
+#define EAZ_ABI_VERSION 4
 
 enum {
   EAZ_OK = 0,
@@ -458,6 +458,23 @@ int eaz_priority_sample(void* tree, size_t tree_bytes, int32_t T, int32_t B, int
 /* SYNCHRONISES `stream` and reads the sticky EAZ_PRIORITY_* bits into *flags_out; returns EAZ_ERR_UNSUPPORTED with a message if
  * any is set, 0 otherwise. */
 int eaz_priority_status(const void* tree, size_t tree_bytes, void* stream, int32_t* flags_out);
+
+/* ABI 4 (appended): the replay ring with its cursor on the device, for callers that cannot keep it on the host (a jitted JAX
+ * program, a CUDA graph replayed many times). */
+
+/* The ring's add at the DEVICE cursor (slot = the header's cursor, never read by the host): `state`'s B envs go into
+ * ring_states[slot] [B,S] in the eaz_env_compact encoding and rewards[:,0] into ring_rewards[slot] [B], then add_step(slot).  The
+ * result equals eaz_env_compact + the row copies + eaz_priority_add_step(tree, ..., cursor) bit for bit.  Two launches. */
+int eaz_replay_add(const eaz_env* env, const eaz_state* state, uint8_t* ring_states, float* ring_rewards, void* tree, size_t tree_bytes,
+                   int32_t T, int32_t B, void* stream);
+/* eaz_priority_sample with (seed, draw counter) taken from `key` (device uint32[2]) instead of the header.  Writes nothing into
+ * the tree (no counter advance, no status bit): a pure function of the tree, the ring and the key.  An empty tree gives index 0,
+ * probability 0. */
+int eaz_priority_sample_keyed(const void* tree, size_t tree_bytes, int32_t T, int32_t B, int32_t K, const uint32_t* key, const uint8_t* states,
+                              const float* rewards, int32_t S, int32_t* indices, float* probabilities, uint8_t* first, float* first_rewards,
+                              uint8_t* second, float* second_rewards, void* stream);
+/* Copies the sticky EAZ_PRIORITY_* word into the device int32 *flags_dev on `stream`; does not synchronise. */
+int eaz_priority_status_async(const void* tree, size_t tree_bytes, int32_t* flags_dev, void* stream);
 
 #ifdef __cplusplus
 }
