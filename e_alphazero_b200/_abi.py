@@ -8,7 +8,7 @@ from __future__ import annotations
 
 import ctypes as C
 
-ABI_VERSION = 4
+ABI_VERSION = 5
 
 EAZ_OK = 0
 EAZ_ERR_INVALID_ARG = -1
@@ -46,6 +46,10 @@ PRIORITY_BAD_ADD = 1 << 3
 
 MLP_EXACT = 0
 MLP_TENSOR = 1
+
+# eaz_search_config.root_prior / action_sampling (selfplay.py:92-98, 125-134)
+ROOT_PRIOR_GIVEN, ROOT_PRIOR_UNIFORM = 0, 1
+ACTION_SEARCH, ACTION_VISITS, ACTION_IMPROVED = 0, 1, 2
 
 _p = C.c_void_p
 
@@ -114,6 +118,8 @@ class EazSearchConfig(C.Structure):
         ("pb_c_base", C.c_float),
         ("temperature", C.c_float),
         ("noise_seed", C.c_uint32),
+        ("root_prior", C.c_int32),
+        ("action_sampling", C.c_int32),
     ]
 
 
@@ -260,6 +266,7 @@ class EazSearchInputs(C.Structure):
         ("gumbel", _p),
         ("env", C.POINTER(EazEnv)),
         ("net", C.POINTER(EazFcParams)),
+        ("sample_gumbel", _p),
     ]
 
 
@@ -324,6 +331,8 @@ def default_search_config(**kw) -> EazSearchConfig:
         pb_c_base=19652.0,
         temperature=1.0,
         noise_seed=0,
+        root_prior=ROOT_PRIOR_GIVEN,
+        action_sampling=ACTION_SEARCH,
     )
     for k, v in kw.items():
         if not hasattr(cfg, k):

@@ -17,6 +17,10 @@
 // Per simulation: select (+ fused DeepSea step | Subleq step kernel) -> network
 // -> expand + backward.  Everything is enqueued on the caller's stream with no
 // host synchronisation, so a whole search is CUDA-graph capturable.
+//
+// The optional parts of the self-play step (cfg.root_prior / action_sampling,
+// selfplay.py:92-98,125-134) live in root_init_kernel and finalize_kernel, which
+// every search path (persistent, launch chain, stream sub-batch) runs.
 #include "mlp.cuh"
 
 #include <cstdlib>
@@ -78,7 +82,8 @@ struct Tree {
   int2* path;     // [max_depth][B] (node, action) per level of the current descent
   int32_t* path_len;
   int32_t* tile_ctr;  // [2][tiles] completion counters of the tile-flag protocol (common.cuh)
-  uint32_t* draw_ctr;  // [1] number of searches that drew their own root noise on this workspace (counter-based generator)
+  uint32_t* draw_ctr;  // [0] number of searches that drew their own noise on this workspace (counter-based generator), [1] its value
+                       // at this search's root_init (read by finalize_kernel while it advances [0])
 };
 
 struct Layout {
@@ -118,7 +123,7 @@ static void make_layout(int B, int N, int A, int S, int table_len, int obs_dim, 
   put((size_t)max_depth * B * 8);  // 25 path
   put((size_t)B * 4);              // 26 path_len
   put((size_t)2 * ceil_div(B, kTileRows) * 4);  // 27 tile counters: [tiles] tree done, [tiles] network done
-  put(16);                                      // 28 draw counter of the in-kernel root noise
+  put(16);                                      // 28 draw counter of the in-kernel noise, [1] its value for the action draw
   L->total = o;
 }
 
@@ -429,18 +434,35 @@ __device__ __forceinline__ int puct_select(const SearchParams& sp, const Edge<G,
   bool valid[J];                                                           \
   _Pragma("unroll") for (int j = 0; j < J; ++j) valid[j] = (gl + G * j) < t.A;
 
+// In-kernel standard Gumbel noise: a counter-based stream keyed by (noise_seed, draw counter of the workspace, tree, action), with one
+// more round by kSampleSalt for the noise of the action draw (EAZ_ACTION_*): u in (0, 1) with 24 bits, g = -log(-log(u))
+constexpr uint32_t kSampleSalt = 0x53414D50u;
+__device__ __forceinline__ float stream_gumbel(uint32_t seed, uint32_t ctr, uint32_t tree, uint32_t a, bool sample) {
+  uint32_t h = seed + EAZ_XX_P1;
+  h = xx_round(h, ctr);
+  h = xx_round(h, tree);
+  h = xx_round(h, a);
+  if (sample) h = xx_round(h, kSampleSalt);
+  h ^= h >> 15; h *= EAZ_XX_P2; h ^= h >> 13; h *= EAZ_XX_P3; h ^= h >> 16;
+  const float u = __fmul_rn(__fadd_rn((float)(h >> 8), 0.5f), 5.9604644775390625e-08f);
+  return -eaz_log(-eaz_log(u));
+}
+
 // ------------------------------------------------------------------ root initialisation (A.1 steps 1-2, A.2)
+// prior_logits == NULL: the uniform root prior (EAZ_ROOT_PRIOR_UNIFORM), every logit 0 before the masking.  keep_draw_ctr: copy the
+// draw counter to draw_ctr[1], where finalize_kernel reads it for the noise of the action draw while it advances draw_ctr[0].
 template <int G, int J>
 __global__ void __launch_bounds__(128) root_init_kernel(Tree t, SearchParams sp, const float* __restrict__ prior_logits,
                                                          const float* __restrict__ value, const float* __restrict__ var,
                                                          const float* __restrict__ gumbel, const uint8_t* __restrict__ invalid,
-                                                         float* __restrict__ out_value, float* __restrict__ out_ube, int batch_offset) {
+                                                         float* __restrict__ out_value, float* __restrict__ out_ube, int batch_offset,
+                                                         int keep_draw_ctr) {
   EAZ_GROUP_PROLOGUE();
   float lg[J];
   float m = -INFINITY;
 #pragma unroll
   for (int j = 0; j < J; ++j) {
-    lg[j] = (in_range && valid[j]) ? prior_logits[(size_t)b * t.A + gl + G * j] : 0.0f;
+    lg[j] = (in_range && valid[j] && prior_logits) ? prior_logits[(size_t)b * t.A + gl + G * j] : 0.0f;
     if (valid[j]) m = fmaxf(m, lg[j]);
   }
   m = group_max<G>(m);
@@ -451,20 +473,8 @@ __global__ void __launch_bounds__(128) root_init_kernel(Tree t, SearchParams sp,
     const int a = gl + G * j;
     const bool inv = invalid && invalid[(size_t)b * t.A + a];
     t.edges[(size_t)b * t.A + a].pl = inv ? EAZ_F32_MIN : __fsub_rn(lg[j], m);  // _mask_invalid_actions (reanalyze.py:16-29)
-    // jax.random.gumbel(gumbel_rng) of mctx policies.py: pre-drawn by the caller, or (gumbel == NULL) drawn here from a counter-based
-    // stream keyed by (noise_seed, draw counter of this workspace, tree, action): u in (0, 1) with 24 bits, g = -log(-log(u))
-    float g;
-    if (gumbel) {
-      g = gumbel[(size_t)b * t.A + a];
-    } else {
-      uint32_t h = sp.noise_seed + EAZ_XX_P1;
-      h = xx_round(h, t.draw_ctr[0]);
-      h = xx_round(h, (uint32_t)(batch_offset + b));
-      h = xx_round(h, (uint32_t)a);
-      h ^= h >> 15; h *= EAZ_XX_P2; h ^= h >> 13; h *= EAZ_XX_P3; h ^= h >> 16;
-      const float u = __fmul_rn(__fadd_rn((float)(h >> 8), 0.5f), 5.9604644775390625e-08f);
-      g = -eaz_log(-eaz_log(u));
-    }
+    // jax.random.gumbel(gumbel_rng) of mctx policies.py: pre-drawn by the caller, or (gumbel == NULL) drawn here
+    const float g = gumbel ? gumbel[(size_t)b * t.A + a] : stream_gumbel(sp.noise_seed, t.draw_ctr[0], (uint32_t)(batch_offset + b), (uint32_t)a, false);
     t.gumbel[(size_t)b * t.A + a] = __fmul_rn(sp.gumbel_scale, g);
   }
   if (gl == 0) {
@@ -474,6 +484,7 @@ __global__ void __launch_bounds__(128) root_init_kernel(Tree t, SearchParams sp,
     t.nodes[b] = r;
     if (out_value) out_value[b] = r.val;  // selfplay.py:139-140 value_prediction / ube_prediction
     if (out_ube) out_ube[b] = r.var;
+    if (keep_draw_ctr && b == 0) t.draw_ctr[1] = t.draw_ctr[0];
   }
 }
 
@@ -706,15 +717,44 @@ __global__ void __launch_bounds__(3 * kSq16Epb) subleq16_tree_step_kernel(Tree t
   t.reward[b] = reward;
 }
 
+// categorical draw as Gumbel-max (mctx policies.py: _get_logits_from_probs + _apply_temperature + categorical): the argmax over valid,
+// not excluded actions of (x - max x) / max(tiny, temperature) + g with x = log(max(w, tiny)); ties go to the lowest index, and a row
+// with every action excluded gets the lowest valid one
+template <int G, int J>
+__device__ __forceinline__ int gumbel_max_draw(const float (&w)[J], const bool (&valid)[J], const bool (&excluded)[J], const float (&g)[J],
+                                               float temperature, int gl) {
+  float x[J];
+  float m = -INFINITY;
+#pragma unroll
+  for (int j = 0; j < J; ++j) {
+    x[j] = eaz_log(eaz_max(w[j], EAZ_F32_TINY));
+    if (valid[j]) m = fmaxf(m, x[j]);
+  }
+  m = group_max<G>(m);
+  const float tdiv = eaz_max(EAZ_F32_TINY, temperature);
+  float best = -INFINITY;
+  int besti = 1 << 30;
+#pragma unroll
+  for (int j = 0; j < J; ++j) {
+    const float s = (valid[j] && !excluded[j]) ? __fadd_rn(__fdiv_rn(__fsub_rn(x[j], m), tdiv), g[j]) : -INFINITY;
+    const int ia = valid[j] ? gl + G * j : (1 << 30);
+    if (s > best || (s == best && ia < besti)) { best = s; besti = ia; }
+  }
+  return group_argmax<G>(best, besti);
+}
+
 // ------------------------------------------------------------------ policy output (A.1 step 4) + epistemic_summary (A.7)
 struct SummaryOut {
   int32_t* action;
   float *action_weights, *value, *value_std, *visit_counts, *visit_probs, *qvalues, *qvalues_var;
 };
 
+// sampling (EAZ_ACTION_*): the played action is drawn from the visit probabilities or action_weights with the noise sample_gumbel, or
+// (sample_gumbel == NULL) with the in-kernel stream at the draw counter root_init_kernel kept in draw_ctr[1]
 template <int G, int J>
 __global__ void __launch_bounds__(128) finalize_kernel(Tree t, SearchParams sp, const float* __restrict__ beta_in,
-                                                        const uint8_t* __restrict__ invalid, SummaryOut out, int bump_draw_ctr) {
+                                                        const uint8_t* __restrict__ invalid, SummaryOut out, int bump_draw_ctr,
+                                                        int sampling, const float* __restrict__ sample_gumbel, int batch_offset) {
   EAZ_GROUP_PROLOGUE();
   const float beta = (in_range && beta_in) ? beta_in[b] : 0.0f;
   float gum[J];
@@ -736,24 +776,13 @@ __global__ void __launch_bounds__(128) finalize_kernel(Tree t, SearchParams sp, 
   float x[J], p[J];
   if (sp.flags & EAZ_FLAG_PUCT) {
     // mctx policies.muzero_policy: action_weights = visit_probs; action ~ categorical(log(visit_probs) / temperature) = Gumbel-max
-    float m = -INFINITY;
+    bool none[J];
 #pragma unroll
     for (int j = 0; j < J; ++j) {
       p[j] = sumN > 0 ? __fdiv_rn((float)e.vis[j], eaz_max((float)sumN, 1.0f)) : __fdiv_rn(1.0f, (float)t.A);
-      x[j] = eaz_log(eaz_max(p[j], EAZ_F32_TINY));
-      if (valid[j]) m = fmaxf(m, x[j]);
+      none[j] = false;
     }
-    m = group_max<G>(m);
-    const float tdiv = eaz_max(EAZ_F32_TINY, sp.temperature);
-    float best = -INFINITY;
-    int besti = 1 << 30;
-#pragma unroll
-    for (int j = 0; j < J; ++j) {
-      const float s = valid[j] ? __fadd_rn(__fdiv_rn(__fsub_rn(x[j], m), tdiv), gum[j]) : -INFINITY;
-      const int ia = valid[j] ? gl + G * j : (1 << 30);
-      if (s > best || (s == best && ia < besti)) { best = s; besti = ia; }
-    }
-    act = group_argmax<G>(best, besti);
+    act = gumbel_max_draw<G, J>(p, valid, none, gum, sp.temperature, gl);
   } else {
     act = root_argmax<G, J>(e, valid, gum, inval, cq, maxN, gl);  // considered_visit = max visit count
     // action_weights = softmax(mask_invalid(root_logits + completed_q))
@@ -767,6 +796,19 @@ __global__ void __launch_bounds__(128) finalize_kernel(Tree t, SearchParams sp, 
 #pragma unroll
     for (int j = 0; j < J; ++j) x[j] = inval[j] ? EAZ_F32_MIN : __fsub_rn(x[j], m);
     group_softmax<G, J>(x, valid, p);
+    if (sampling) {  // selfplay.py:125-134: the played action ~ visit counts / improved policy instead of the policy's action
+      float w[J], sg[J];
+#pragma unroll
+      for (int j = 0; j < J; ++j) {
+        const int a = gl + G * j;
+        w[j] = sampling == EAZ_ACTION_IMPROVED ? p[j]
+                                               : (sumN > 0 ? __fdiv_rn((float)e.vis[j], eaz_max((float)sumN, 1.0f)) : __fdiv_rn(1.0f, (float)t.A));
+        sg[j] = !(in_range && valid[j]) ? 0.0f
+                : sample_gumbel        ? sample_gumbel[(size_t)b * t.A + a]
+                                       : stream_gumbel(sp.noise_seed, t.draw_ctr[1], (uint32_t)(batch_offset + b), (uint32_t)a, true);
+      }
+      act = gumbel_max_draw<G, J>(w, valid, inval, sg, sp.temperature, gl);
+    }
   }
   if (blockIdx.x == 0 && threadIdx.x == 0 && bump_draw_ctr) t.draw_ctr[0] += 1u;  // (root_init of this search has long finished)
   if (!in_range) return;
@@ -897,7 +939,7 @@ __global__ void export_tree_kernel(Tree t, TreeOut o) {
 template <int G, int J>
 static int run_search(const Tree& t, const SearchParams& sp, const EnvDesc& env, const NetDesc& net, const eaz_search_inputs* in,
                       const SummaryOut& so, int mlp_mode, int exploration, const TensorWeights* tw, float* root_out_value, float* root_out_ube,
-                      int batch_offset, cudaStream_t st) {
+                      int batch_offset, int root_prior, int sampling, cudaStream_t st) {
   const int envs_per_block = 4 * (32 / G);
   const int grid = ceil_div(t.B, envs_per_block);
   const int lhead = exploration ? EAZ_HEAD_EXPLORE : EAZ_HEAD_EXPLOIT;  // context.py:132
@@ -932,10 +974,13 @@ static int run_search(const Tree& t, const SearchParams& sp, const EnvDesc& env,
     root_value = t.net_value;
     root_var = t.net_ube;
   }
+  // the draw counter advances once per search that draws noise itself: root noise (gumbel == NULL) and / or the noise of the action draw
+  const bool draw_sample = sampling != EAZ_ACTION_SEARCH && !in->sample_gumbel;
+  const int bump_draw_ctr = (int)(in->gumbel == nullptr || draw_sample);
   {
     ProfScope ps(CLS_INIT, st);
-    root_init_kernel<G, J><<<grid, 128, 0, st>>>(t, sp, root_logits, root_value, root_var, in->gumbel, in->invalid_actions, root_out_value, root_out_ube,
-                                                  batch_offset);
+    root_init_kernel<G, J><<<grid, 128, 0, st>>>(t, sp, root_prior == EAZ_ROOT_PRIOR_UNIFORM ? nullptr : root_logits, root_value, root_var, in->gumbel,
+                                                  in->invalid_actions, root_out_value, root_out_ube, batch_offset, (int)draw_sample);
   }
   EAZ_CHECK_LAUNCH("root_init_kernel");
   if constexpr (G == ps::kG && J == 1) {
@@ -946,7 +991,7 @@ static int run_search(const Tree& t, const SearchParams& sp, const EnvDesc& env,
         if (int rc = launch_persistent(t, sp, env, in, ncap, st)) return rc;
       }
       ProfScope pf(CLS_FINAL, st);
-      finalize_kernel<G, J><<<grid, 128, 0, st>>>(t, sp, in->beta, in->invalid_actions, so, (int)(in->gumbel == nullptr));
+      finalize_kernel<G, J><<<grid, 128, 0, st>>>(t, sp, in->beta, in->invalid_actions, so, bump_draw_ctr, sampling, in->sample_gumbel, batch_offset);
       EAZ_CHECK_LAUNCH("finalize_kernel");
       return 0;
     }
@@ -1007,7 +1052,7 @@ static int run_search(const Tree& t, const SearchParams& sp, const EnvDesc& env,
   }
   {
     ProfScope ps(CLS_FINAL, st);
-    finalize_kernel<G, J><<<grid, 128, 0, st>>>(t, sp, in->beta, in->invalid_actions, so, (int)(in->gumbel == nullptr));
+    finalize_kernel<G, J><<<grid, 128, 0, st>>>(t, sp, in->beta, in->invalid_actions, so, bump_draw_ctr, sampling, in->sample_gumbel, batch_offset);
   }
   EAZ_CHECK_LAUNCH("finalize_kernel");
   return 0;
@@ -1035,6 +1080,14 @@ static int check_search(const eaz_search_config* cfg, const eaz_search_inputs* i
   EAZ_CHECK_ARG(fused_root || (in->prior_logits && in->value && in->value_epistemic_variance),
                 "search inputs: prior_logits / value / value_epistemic_variance must be all non-NULL, or all NULL (fused root)");
   EAZ_CHECK_ARG(out->action != nullptr, "search outputs: action must be non-NULL");
+  EAZ_CHECK_ARG(cfg->root_prior == EAZ_ROOT_PRIOR_GIVEN || cfg->root_prior == EAZ_ROOT_PRIOR_UNIFORM, "root_prior %d is not an EAZ_ROOT_PRIOR_*",
+                cfg->root_prior);
+  EAZ_CHECK_ARG(cfg->action_sampling >= EAZ_ACTION_SEARCH && cfg->action_sampling <= EAZ_ACTION_IMPROVED, "action_sampling %d is not an EAZ_ACTION_*",
+                cfg->action_sampling);
+  EAZ_CHECK_ARG(!(cfg->flags & EAZ_FLAG_PUCT) || (cfg->root_prior == EAZ_ROOT_PRIOR_GIVEN && cfg->action_sampling == EAZ_ACTION_SEARCH),
+                "root_prior / action_sampling are options of the Gumbel policy: not with EAZ_FLAG_PUCT");
+  EAZ_CHECK_ARG(cfg->action_sampling == EAZ_ACTION_SEARCH || (isfinite(cfg->temperature) && cfg->temperature > 0.0f),
+                "action_sampling needs a finite temperature > 0 (got %g)", (double)cfg->temperature);
   if ((size_t)(cfg->num_simulations + 1) * cfg->batch * env->num_actions >= ((size_t)1 << 31)) {
     set_error("tree of %d nodes x %d envs x %d actions exceeds 2^31 edges: shard the batch", cfg->num_simulations + 1, cfg->batch, env->num_actions);
     return EAZ_ERR_UNSUPPORTED;
@@ -1186,7 +1239,7 @@ static int search_one(const eaz_search_config* cfg, const eaz_search_inputs* in,
   SummaryOut so{out->action, out->action_weights, out->value, out->value_epistemic_std, out->visit_counts, out->visit_probs,
                 out->qvalues, out->qvalues_epistemic_variance};
   int rc;
-#define EAZ_RUN(G, J) rc = run_search<G, J>(t, sp, env, net, in, so, cfg->mlp_mode, cfg->exploration, cfg->mlp_mode == EAZ_MLP_TENSOR ? &tw : nullptr, out->root_value, out->root_ube, batch_offset, st)
+#define EAZ_RUN(G, J) rc = run_search<G, J>(t, sp, env, net, in, so, cfg->mlp_mode, cfg->exploration, cfg->mlp_mode == EAZ_MLP_TENSOR ? &tw : nullptr, out->root_value, out->root_ube, batch_offset, cfg->root_prior, cfg->action_sampling, st)
   if (A <= 2) EAZ_RUN(2, 1);
   else if (A <= 4) EAZ_RUN(4, 1);
   else if (A <= 8) EAZ_RUN(8, 1);
@@ -1331,6 +1384,7 @@ int eaz_search_gumbel(const eaz_search_config* cfg, const eaz_search_inputs* in,
     si.embedding = e0 ? &es : nullptr;
     si.invalid_actions = offu(in->invalid_actions, A);
     si.gumbel = offf(in->gumbel, A);
+    si.sample_gumbel = offf(in->sample_gumbel, A);
     eaz_search_outputs so = *out;
     so.action = (int32_t*)offi(out->action, 1);
     so.action_weights = (float*)offf(out->action_weights, A);

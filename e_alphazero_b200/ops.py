@@ -579,7 +579,8 @@ class SearchPlan:
     def run(self, root: dict, profile: bool = False, reuse_prepared: bool | None = False):
         """root: prior_logits [B,A], value [B], value_epistemic_variance [B], beta [B], embedding (state dict),
         gumbel [B,A] pre-drawn standard Gumbel noise (absent / None: drawn inside the search from cfg.noise_seed and the
-        workspace's draw counter), optional invalid_actions [B,A] (bool/uint8).
+        workspace's draw counter), optional invalid_actions [B,A] (bool/uint8), optional sample_gumbel [B,A]: the noise of the
+        action draw of cfg.action_sampling (absent / None: drawn inside the search like `gumbel`).
 
         The returned tensors are THIS PLAN'S buffers: the next run() overwrites them (clone what must survive).
         reuse_prepared: False = rebuild the parameter-derived tables, True = the caller promises env / net are unchanged,
@@ -592,7 +593,8 @@ class SearchPlan:
             inv = inv.to(u8)
         e, n, s = self.env.struct(), self.net.struct(), state_struct(self.env, root["embedding"])
         inp = _abi.EazSearchInputs(_ptr(root.get("prior_logits"), f32), _ptr(root.get("value"), f32), _ptr(root.get("value_epistemic_variance"), f32),
-                                   _ptr(root["beta"], f32), C.pointer(s), _ptr(inv), _ptr(root.get("gumbel"), f32), C.pointer(e), C.pointer(n))
+                                   _ptr(root["beta"], f32), C.pointer(s), _ptr(inv), _ptr(root.get("gumbel"), f32), C.pointer(e), C.pointer(n),
+                                   _ptr(root.get("sample_gumbel"), f32))
         o = _abi.EazSearchOutputs()
         for name, _, _ in _abi.SEARCH_OUTPUT_FIELDS:
             setattr(o, name, _ptr(self.out.get(name)))

@@ -30,18 +30,34 @@ class SelfplayRunner:
     `clone_outputs=True`, or use `trajectory()` (one packed int32 [B,4] record per step, written into a caller-owned [T,B,4] buffer).
 
     device_noise=True draws the root Gumbel noise inside the search (counter-based stream keyed by `seed`, the number of searches run
-    and the tree index) instead of five elementwise torch kernels per step; parity tests pass `gumbel=` explicitly."""
+    and the tree index) instead of five elementwise torch kernels per step; parity tests pass `gumbel=` explicitly.
+
+    The optional parts of the reference's step: uniform_prior=True searches from a uniform root prior instead of the network's root
+    logits (selfplay.py:92-98); action_sampling="visit_counts" / "improved_policy" plays an action drawn from the search's visit
+    counts / action_weights at `temperature` instead of its own action (selfplay.py:125-134).  Both run inside the search kernels.
+    The noise of that draw follows the rules of the root noise: `sample_gumbel=` if given, else drawn from the runner's generator
+    (inside the CUDA graph when captured), or by the search itself with device_noise=True.  `SelfplayOutput.action` and
+    `trajectory()` carry the played action."""
+
+    ACTION_SAMPLING = {"search": _abi.ACTION_SEARCH, "visit_counts": _abi.ACTION_VISITS, "improved_policy": _abi.ACTION_IMPROVED}
 
     def __init__(self, env_spec: ops.EnvSpec, net: ops.FcParams, batch: int, num_simulations: int, discount: float,
                  exploration_beta: float = 0.0, directed_exploration: bool = False, rescale_values: bool = True,
                  mlp_mode: int = _abi.MLP_EXACT, tasks=(1,), device="cuda", seed: int = 0, use_graph: bool = False, fused_root: bool = False,
-                 streams: int = 1, device_noise: bool = False, clone_outputs: bool = False):
+                 streams: int = 1, device_noise: bool = False, clone_outputs: bool = False, uniform_prior: bool = False,
+                 action_sampling: str = "search", temperature: float = 1.0):
         torch = require_cuda()
+        if action_sampling not in self.ACTION_SAMPLING:
+            raise ValueError(f"action_sampling must be one of {sorted(self.ACTION_SAMPLING)}, got {action_sampling!r}")
         self.env, self.net, self.B, self.device = env_spec, net, batch, device
         self.directed = directed_exploration
         self.cfg = _abi.default_search_config(batch=batch, num_simulations=num_simulations, discount=discount,
                                               exploration=int(directed_exploration), rescale_values=int(rescale_values), mlp_mode=mlp_mode)
         self.cfg.noise_seed = int(seed) & 0xFFFFFFFF
+        self.cfg.root_prior = _abi.ROOT_PRIOR_UNIFORM if uniform_prior else _abi.ROOT_PRIOR_GIVEN
+        self.cfg.action_sampling = self.ACTION_SAMPLING[action_sampling]
+        self.cfg.temperature = float(temperature)
+        self.sampling = self.cfg.action_sampling != _abi.ACTION_SEARCH
         self.device_noise, self.clone_outputs = bool(device_noise), bool(clone_outputs)
         if streams > 1:  # EAZ_FLAG_STREAMS: sub-batches searched concurrently (tree kernel of one overlaps the network kernel of another)
             self.cfg.flags |= _abi.flag_streams(streams)
@@ -78,15 +94,16 @@ class SelfplayRunner:
         idx = torch.randint(0, self.tasks.numel(), (self.B,), device=self.device, generator=self.gen)
         return self.tasks[idx].contiguous()
 
-    def step(self, states: dict, gumbel=None, task_ids=None):
-        """states: device state dict (updated in place).  Returns (states, SelfplayOutput)."""
+    def step(self, states: dict, gumbel=None, task_ids=None, sample_gumbel=None):
+        """states: device state dict (updated in place); sample_gumbel: the noise of the action draw (action_sampling only).
+        Returns (states, SelfplayOutput)."""
         if self.use_graph:
-            return self._step_graph(states, gumbel, task_ids)
+            return self._step_graph(states, gumbel, task_ids, sample_gumbel)
         reuse = not self._stale
         self._stale = False
-        return self._step_eager(states, gumbel, task_ids, reuse_prepared=reuse)
+        return self._step_eager(states, gumbel, task_ids, reuse_prepared=reuse, sample_gumbel=sample_gumbel)
 
-    def _step_graph(self, states, gumbel, task_ids):
+    def _step_graph(self, states, gumbel, task_ids, sample_gumbel=None):
         torch = require_cuda()
         subleq = self.env.kind == _abi.ENV_SUBLEQ
         if self._static is None:
@@ -96,15 +113,17 @@ class SelfplayRunner:
             for k, v in states.items():
                 st[k].copy_(v)
             sg = torch.zeros((self.B, self.A), dtype=torch.float32, device=self.device)
+            ss = torch.zeros((self.B, self.A), dtype=torch.float32, device=self.device)
             stt = torch.ones(self.B, dtype=torch.int32, device=self.device) if subleq else None
             self._step_eager({k: v.clone() for k, v in st.items()}, self.draw_gumbel(), self._draw_tasks() if subleq else None,
-                             reuse_prepared=False)  # warm-up: one-time attribute setup / allocations
+                             reuse_prepared=False, sample_gumbel=ss)  # warm-up: one-time attribute setup / allocations
             torch.cuda.synchronize()
-            self._static = (st, sg, stt)
-        st, sg, stt = self._static
-        draw = gumbel is None and (task_ids is None or not subleq)  # noise drawn inside the graph unless the caller supplies it
-        in_search = draw and self.device_noise                      # ... by the search itself (no torch kernels)
-        key = (not self._stale, draw, in_search)
+            self._static = (st, sg, stt, ss)
+        st, sg, stt, ss = self._static
+        draw = gumbel is None and sample_gumbel is None and (task_ids is None or not subleq)  # noise drawn inside the graph unless
+        in_search = draw and self.device_noise                                                # supplied ... by the search itself
+        host_sample = self.sampling and (sample_gumbel is not None or not self.device_noise)  # the action draw's noise in `ss`
+        key = (not self._stale, draw, in_search, host_sample)
         if key not in self._graphs:
             g = torch.cuda.CUDAGraph()
             g.register_generator_state(self.gen)
@@ -112,9 +131,11 @@ class SelfplayRunner:
                 if draw:
                     if not in_search:
                         sg.copy_(self.draw_gumbel())
+                    if host_sample:
+                        ss.copy_(self.draw_gumbel())
                     if subleq:
                         stt.copy_(self._draw_tasks())
-                _, out = self._step_eager(st, None if in_search else sg, stt, reuse_prepared=key[0])
+                _, out = self._step_eager(st, None if in_search else sg, stt, reuse_prepared=key[0], sample_gumbel=ss if host_sample else None)
             self._graphs[key] = (g, out)
         g, out = self._graphs[key]
         for k in st:
@@ -122,6 +143,8 @@ class SelfplayRunner:
                 st[k].copy_(states[k])
         if not draw:
             sg.copy_(gumbel if gumbel is not None else self.draw_gumbel())
+            if host_sample:
+                ss.copy_(sample_gumbel if sample_gumbel is not None else self.draw_gumbel())
             if subleq:
                 stt.copy_(task_ids if task_ids is not None else self._draw_tasks())
         g.replay()
@@ -145,10 +168,12 @@ class SelfplayRunner:
         of, ov = ops.alloc_arena(self.plan.out_specs, "cpu", pinned=True)
         return sf, sv, of, ov
 
-    def _step_eager(self, states: dict, gumbel=None, task_ids=None, reuse_prepared=None):
+    def _step_eager(self, states: dict, gumbel=None, task_ids=None, reuse_prepared=None, sample_gumbel=None):
         torch = require_cuda()
         if gumbel is None and not self.device_noise:
             gumbel = self.draw_gumbel()
+        if sample_gumbel is None and self.sampling and not self.device_noise:
+            sample_gumbel = self.draw_gumbel()
         if self.fused_root:  # selfplay.py:89 inside the search call (policy head = the recurrent_fn's: main.py:262)
             root = dict(beta=self.beta, embedding=states, gumbel=gumbel)
         else:
@@ -156,6 +181,8 @@ class SelfplayRunner:
             logits = ev["explore_logits"] if self.directed else ev["exploit_logits"]  # :93-95
             root = dict(prior_logits=logits, value=ev["value"], value_epistemic_variance=ev["ube"], beta=self.beta, embedding=states,
                         gumbel=gumbel)
+        if self.sampling:
+            root["sample_gumbel"] = sample_gumbel
         out = self.plan.run(root, reuse_prepared=reuse_prepared)  # :107-117 (invalid_actions = ~legal_action_mask = none)
         if self.fused_root:
             ev = dict(value=out["root_value"], ube=out["root_ube"])

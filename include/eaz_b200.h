@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define EAZ_ABI_VERSION 4
+#define EAZ_ABI_VERSION 5
 
 enum {
   EAZ_OK = 0,
@@ -236,9 +236,22 @@ typedef struct eaz_search_config {
   /* ABI 2 (appended): mctx muzero_policy parameters, read only with EAZ_FLAG_PUCT */
   float pb_c_init;          /* 1.25 */
   float pb_c_base;          /* 19652 */
-  float temperature;        /* 1.0 */
+  float temperature;        /* 1.0; also the temperature of the draw of action_sampling != EAZ_ACTION_SEARCH */
   uint32_t noise_seed;      /* tie-break noise stream */
+  /* ABI 5 (appended): the optional parts of the self-play step (selfplay.py:92-98, 125-134); 0 = off, not with EAZ_FLAG_PUCT */
+  int32_t root_prior;       /* EAZ_ROOT_PRIOR_* */
+  int32_t action_sampling;  /* EAZ_ACTION_* */
 } eaz_search_config;
+
+/* Root prior (selfplay.py:92-98).  UNIFORM: the root's prior logits are 0 for every action (then _mask_invalid_actions: invalid ones get
+ * EAZ_F32_MIN), whatever prior_logits holds and also with a fused root; the root value / UBE and every node below the root are
+ * unchanged. */
+enum { EAZ_ROOT_PRIOR_GIVEN = 0, EAZ_ROOT_PRIOR_UNIFORM = 1 };
+/* Played action (selfplay.py:125-134).  SEARCH: the Gumbel policy's action.  VISITS / IMPROVED: a categorical draw from the visit
+ * probabilities / from this search's action_weights, as the Gumbel-max argmax over valid, not invalid actions of
+ * (x_a - max_a x_a) / max(tiny, temperature) + g_a with x_a = log(max(w_a, tiny)) and g = sample_gumbel (ties: lowest index; a row
+ * whose actions are all invalid plays 0).  Only `action` changes; action_weights and the summary are those of the search. */
+enum { EAZ_ACTION_SEARCH = 0, EAZ_ACTION_VISITS = 1, EAZ_ACTION_IMPROVED = 2 };
 
 enum {
   EAZ_MLP_EXACT = 0, /* fp32 FMA chains in index order: bit-identical to the oracle */
@@ -263,6 +276,12 @@ typedef struct eaz_search_inputs {
                                             searches run on this workspace so far, tree, action) */
   const eaz_env* env;
   const eaz_fc_params* net;              /* params=model */
+  /* ABI 5 (appended) */
+  const float* sample_gumbel;            /* [B,A] pre-drawn standard Gumbel noise of the action draw (cfg.action_sampling != 0; not
+                                            scaled by gumbel_scale).  NULL = drawn inside the search from the stream of `gumbel`
+                                            with one more xx round by 0x53414D50 after the action: (noise_seed, the same draw
+                                            counter value, tree, action).  The workspace's draw counter advances once per search
+                                            that draws either noise itself */
 } eaz_search_inputs;
 
 typedef struct eaz_search_outputs {
