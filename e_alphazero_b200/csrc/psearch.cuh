@@ -17,7 +17,7 @@
 // simulations: 16 tree warps (two trees per warp, 16 lanes each -- the mapping of tree_step2_kernel) keep, per tree and for the whole
 // search, the cached selection and the compact env state of EVERY node in shared memory (the pointer-chase descent never leaves the
 // SM), plus a staging area with the node / edge records of the current path.  Per simulation a tree warp runs: expand (with the leaf's
-// table entry) + backward + action refresh (the STAGED arithmetic of tree_step.cuh, bit-identical) -> descent over the cached
+// table entry) + backward + action refresh (tree_step.cuh: staged2_*, the staged step of tree_step2_kernel) -> descent over the cached
 // selections -> DeepSea transition -> load of the new leaf's table entry -> stage the new path's records.  Trees that cannot be staged
 // (path longer than kNodes - 1, re-expanded leaf under a max_depth cut-off) take tree_step_direct for that simulation and
 // re-synchronise their shared-memory caches.
@@ -275,18 +275,17 @@ __global__ void __launch_bounds__(kTableThreads, 1) ds_output_table_kernel(const
 constexpr int kTWarps = 16;          // tree warps per CTA
 constexpr int kSlots = 2 * kTWarps;  // trees per CTA
 constexpr int kThreads = kTWarps * 32;
-// per-tree staging area (uint32 words); layout of tree_step.cuh Stage2<2>, sized for kNodes staged nodes (path + leaf)
-constexpr int kW = 16;                // lanes per tree
-constexpr int kG = 2;                 // lanes per node (A <= 2)
-constexpr int kPR = kW / kG;          // nodes refreshed per round
+// per-tree staging area (uint32 words), sized for kNodes staged nodes (path + leaf).  The edge and back words and the leaf priors
+// (misc [8..8+A)) have the layout of tree_step2_kernel's staging area, which the staged step of tree_step.cuh (staged2_*) reads; the
+// root words, the other misc words and the 16-bit next words are this kernel's own.
+constexpr int kG = 2;                          // lanes per node (A <= 2)
+constexpr int kPR = kStaged2Lanes / kG;        // nodes refreshed per round
 constexpr int kRounds = 3;
-constexpr int kNodes = kRounds * kPR; // 24
-constexpr int kLaneWords = 10;        // ci1, vis, pl, rew, val, vvar, dis, raw, rawvar, prior probability
-constexpr int kEdgeWords = kRounds * kLaneWords * kW;  // 480
-constexpr int kBackWords = 4 * 32;    // [node | action << 16, visits -> child value, value -> child variance, variance][level]
-constexpr int kRootWords = 4;         // [a] gumbel + (logit - max logit), [2 + a] invalid flag
-constexpr int kMiscWords = 12;        // [0] considered visit, [8..8+A) leaf priors
-constexpr int kTreeWords = kEdgeWords + kBackWords + kRootWords + kMiscWords;  // + ncap state words + ncap/2 next words
+constexpr int kNodes = kRounds * kPR;          // 24
+constexpr int kEdgeWords = kRounds * kStaged2LaneWords * kStaged2Lanes;  // 480
+constexpr int kRootWords = 4;                  // [a] gumbel + (logit - max logit), [2 + a] invalid flag
+constexpr int kMiscWords = 12;                 // [0] considered visit, [1] number of considered actions, [8..8+A) leaf priors
+constexpr int kTreeWords = kEdgeWords + kStaged2BackWords + kRootWords + kMiscWords;  // + ncap state words + ncap/2 next words
 
 __host__ __device__ inline int tree_words(int ncap) { return kTreeWords + ncap + ncap / 2; }  // ncap even
 constexpr int kAmapMax = 16384;  // the DeepSea action map (N x N bytes) is mirrored in shared memory when it fits (N <= 128)
@@ -302,9 +301,6 @@ __device__ __forceinline__ uint32_t lds_u16(uint32_t addr) {
   return v;
 }
 __device__ __forceinline__ void sts_u32(uint32_t addr, uint32_t v) { asm volatile("st.shared.u32 [%0], %1;" ::"r"(addr), "r"(v) : "memory"); }
-__device__ __forceinline__ uint32_t pack_next16(int packed) {  // NodeRec.pad0 (action | child + 1 << 8) -> 16 bits (action | child + 1 << 2)
-  return (uint32_t)(packed & 3) | ((uint32_t)(packed >> 8) << 2);
-}
 
 // Optional timeline of CTA 0 (eaz_debug_set_ps_trace): per simulation `it` and tree warp w, at [(it * kTWarps + w) * 8 + k], globaltimer
 // stamps of k = 0 expand done (the leaf's table entry has been used), 1 backward done, 2 refresh done, 3 descent done (the next leaf's
@@ -355,7 +351,7 @@ __global__ void __launch_bounds__(kThreads, 1) ds_search_kernel(const __grid_con
   __syncthreads();
 
   // ================================================================ tree warps: two trees each (16 lanes per tree)
-  const int hl = lane & (kW - 1), hbase = lane & kW, sub = lane >> 4;
+  const int hl = lane & (kStaged2Lanes - 1), hbase = lane & kStaged2Lanes, sub = lane >> 4;
   const int slot = 2 * tw + sub;
   const int b0 = blockIdx.x * kSlots + 2 * tw;  // the warp's first tree
   const int b = b0 + sub;
@@ -367,10 +363,11 @@ __global__ void __launch_bounds__(kThreads, 1) ds_search_kernel(const __grid_con
   uint32_t* const sw = tree_smem + (size_t)slot * tree_words(ncap);
   uint32_t* const s_edge = sw;
   uint32_t* const s_back = sw + kEdgeWords;
-  uint32_t* const s_root = s_back + kBackWords;
+  uint32_t* const s_root = s_back + kStaged2BackWords;
   uint32_t* const s_misc = s_root + kRootWords;
   uint32_t* const s_state = s_misc + kMiscWords;
   uint16_t* const s_next = reinterpret_cast<uint16_t*>(s_state + ncap);
+  const Staged2Lane w{lane, hl, hbase, gl, glev, valid1[0], in_batch, uB, uA, ub, s_edge, s_back, s_misc};
   const float beta = (in_batch && a.beta) ? a.beta[b] : 0.0f;
   const bool std_backup = (sp.flags & EAZ_FLAG_BACKUP_STD) != 0;
   uint32_t* const st_global = reinterpret_cast<uint32_t*>(t.states);
@@ -384,7 +381,7 @@ __global__ void __launch_bounds__(kThreads, 1) ds_search_kernel(const __grid_con
   // ---- reload everything the persistent state mirrors from the workspace (after a DIRECT step)
   auto resync = [&](int sim) {
     if (in_batch) {
-      for (int nd = hl; nd <= sim + 1 && nd < ncap; nd += kW) {
+      for (int nd = hl; nd <= sim + 1 && nd < ncap; nd += kStaged2Lanes) {
         s_next[nd] = (uint16_t)pack_next16(t.nodes[(unsigned)nd * uB + ub].pad0);
         s_state[nd] = st_global[(unsigned)nd * uB + ub];
       }
@@ -394,7 +391,7 @@ __global__ void __launch_bounds__(kThreads, 1) ds_search_kernel(const __grid_con
       const uint32_t ns = st_global[(unsigned)leaf * uB + ub];
       term = EAZ_DS_TERM(ns) != 0;
       net = __ldg(a.ds_out + deepsea_obs_index(ns, a.env.size));
-      for (int lev = hl; lev < L && lev < 32; lev += kW) {
+      for (int lev = hl; lev < L && lev < 32; lev += kStaged2Lanes) {
         const int2 pa = t.path[(unsigned)lev * uB + ub];
         s_back[lev] = (uint32_t)pa.x | ((uint32_t)pa.y << 16);
       }
@@ -410,7 +407,7 @@ __global__ void __launch_bounds__(kThreads, 1) ds_search_kernel(const __grid_con
     if (in_batch) {  // backward operands: this lane owns levels hl and hl + 16
 #pragma unroll
       for (int k = 0; k < 2; ++k) {
-        const int lev = hl + kW * k;
+        const int lev = hl + kStaged2Lanes * k;
         if (lev < L) {
           const uint4 nrec = reinterpret_cast<const uint4*>(t.nodes + ((s_back[lev] & 0xffffu) * uB + ub))[0];
           s_back[1 * 32 + lev] = nrec.x;
@@ -419,7 +416,7 @@ __global__ void __launch_bounds__(kThreads, 1) ds_search_kernel(const __grid_con
         }
       }
     }
-    const int Lw = max(L, __shfl_xor_sync(0xffffffffu, L, kW));
+    const int Lw = max(L, __shfl_xor_sync(0xffffffffu, L, kStaged2Lanes));
 #pragma unroll
     for (int r = 0; r < kRounds; ++r) {
       if (r * kPR <= Lw) {  // warp-uniform
@@ -436,13 +433,7 @@ __global__ void __launch_bounds__(kThreads, 1) ds_search_kernel(const __grid_con
         const float xl[1] = {__uint_as_float(h0.z)};
         float pr[1];
         group_softmax<kG, 1>(xl, valid1, pr);  // p = max(tiny, softmax(prior logits)) of _compute_mixed_value
-        if (on) {
-          uint32_t* se = s_edge + r * kLaneWords * kW + hl;
-          se[0 * kW] = h0.x; se[1 * kW] = h0.y; se[2 * kW] = h0.z; se[3 * kW] = h0.w;
-          se[4 * kW] = h1.x; se[5 * kW] = h1.y; se[6 * kW] = h1.z;
-          se[7 * kW] = n1.x; se[8 * kW] = n1.y;
-          se[9 * kW] = __float_as_uint(eaz_max(EAZ_F32_TINY, pr[0]));
-        }
+        if (on) staged2_store_lane(s_edge, r, hl, h0, h1, n1, pr[0]);
       }
     }
     // the root's seq-halving visit target for the refresh of step `sim_next` (s_root[0..1] hold gumbel + logit, [2..3] the invalid flags)
@@ -492,162 +483,13 @@ __global__ void __launch_bounds__(kThreads, 1) ds_search_kernel(const __grid_con
       continue;
     }
 
-    // ---- 1. expand
-    const unsigned lslot = (unsigned)leaf * uB + ub;
-    const float nv = in_batch ? net.x : 0.0f, nu = in_batch ? net.y : 0.0f;
-    const float m = __shfl_sync(0xffffffffu, group_max<kG>(lg), hbase);  // context.py:135: max over the A <= kG logit lanes (the rest hold -inf)
-    const float pl_leaf = __fsub_rn(lg, m);                              // legal_action_mask is all True (:137)
-    if (in_batch && hl < t.A) {
-      t.edges[(size_t)(lslot * uA + hl)].pl = pl_leaf;
-      s_misc[8 + hl] = __float_as_uint(pl_leaf);
-    }
-    const float value = term ? 0.0f : nv;  // :140
-    const float var = term ? 0.0f : nu;    // :141
-    float disc = sp.discount;
-    if (sp.two_players) disc = __fmul_rn(disc, -1.0f);  // :142-143
-    if (term) disc = 0.0f;                              // :144
-    if (in_batch && hl == 0) {
-      const uint32_t last = s_back[L - 1];
-      const int last_node = (int)(last & 0xffffu), last_act = (int)(last >> 16);
-      uint4* ln = reinterpret_cast<uint4*>(t.nodes + lslot);  // update_tree_node: a fresh leaf (staging condition)
-      ln[0] = make_uint4(1u, __float_as_uint(value), __float_as_uint(var), 0u);
-      ln[1] = make_uint4(__float_as_uint(value), __float_as_uint(var), (unsigned)(last_node + 1), (unsigned)(last_act + 1));
-      EdgeRec* pe0 = t.edges + (size_t)(((unsigned)last_node * uB + ub) * uA + (unsigned)last_act);
-      pe0->ci1 = leaf + 1;
-      pe0->rew = reward;  // :139
-      pe0->dis = disc;
-    }
+    // ---- 1. expand, 2. backward, 3. refresh (tree_step.cuh)
+    const Staged2Leaf f = staged2_expand<kG>(t, sp, w, L, leaf, reward, lg, in_batch ? net.x : 0.0f, in_batch ? net.y : 0.0f, term);
     if (lane == 0) trc.stamp(it, tw, 0);
-
-    // ---- 2. backward: rounds of 16 levels, deepest first; lane = level within the round
-    float lv = value, lvar = std_backup ? __fsqrt_rn(var) : var;
-    float below_val = value, below_var = var;
-    const int Lw = max(L, __shfl_xor_sync(0xffffffffu, L, kW));
-#pragma unroll 1
-    for (int k = Lw > kW ? 1 : 0; k >= 0; --k) {
-      const int lo = kW * k, cnt = min(max(L - lo, 0), kW);
-      const int lev = lo + hl;
-      const bool have = in_batch && hl < cnt;
-      int my_node = 0, my_act = 0, nvis = 0, cvis = 0;
-      float nval = 0.0f, nvar = 0.0f, rr = 0.0f, dd = 0.0f;
-      if (have) {
-        const uint32_t pa = s_back[lev];
-        my_node = (int)(pa & 0xffffu);
-        my_act = (int)(pa >> 16);
-        nvis = (int)s_back[32 + lev];
-        nval = __uint_as_float(s_back[64 + lev]);
-        nvar = __uint_as_float(s_back[96 + lev]);
-        const uint32_t* se = s_edge + (lev / kPR) * kLaneWords * kW + (lev % kPR) * kG + my_act;  // the traversed edge in the refresh staging
-        cvis = (int)se[1 * kW];
-        rr = __uint_as_float(se[3 * kW]);
-        dd = __uint_as_float(se[6 * kW]);
-        if (lev == L - 1) { rr = reward; dd = disc; }  // written by the expand step above
-      }
-      const int cmax = max(cnt, __shfl_xor_sync(0xffffffffu, cnt, kW));
-      float my_lv = 0.0f, my_lvar = 0.0f;
-      for (int i = cmax - 1; i >= 0; --i) {  // the recurrences, in the reference's op order
-        const float r = __shfl_sync(0xffffffffu, rr, hbase + i), d = __shfl_sync(0xffffffffu, dd, hbase + i);
-        if (i < cnt) {
-          lv = __fadd_rn(r, __fmul_rn(d, lv));
-          lvar = std_backup ? __fadd_rn(0.0f, __fmul_rn(fabsf(d), lvar)) : __fadd_rn(0.0f, __fmul_rn(__fmul_rn(d, d), lvar));
-          if (hl == i) { my_lv = lv; my_lvar = lvar; }
-        }
-      }
-      const float count = (float)nvis;
-      const float pv = __fdiv_rn(__fadd_rn(__fmul_rn(nval, count), my_lv), __fadd_rn(count, 1.0f));
-      float pvar;
-      if (std_backup) {
-        const float psd = __fdiv_rn(__fadd_rn(__fmul_rn(__fsqrt_rn(nvar), count), my_lvar), __fadd_rn(count, 1.0f));
-        pvar = __fmul_rn(psd, psd);
-      } else {
-        pvar = __fdiv_rn(__fadd_rn(__fmul_rn(nvar, count), my_lvar), __fadd_rn(count, 1.0f));
-      }
-      // children_values[parent, a] = the child's CURRENT (already updated) mean: one level deeper
-      float cval = __shfl_down_sync(0xffffffffu, pv, 1, kW), cvarr = __shfl_down_sync(0xffffffffu, pvar, 1, kW);
-      if (hl == cnt - 1) { cval = below_val; cvarr = below_var; }
-      if (have) {
-        const unsigned pslot = (unsigned)my_node * uB + ub;
-        EdgeRec* pe = t.edges + (size_t)(pslot * uA + (unsigned)my_act);
-        reinterpret_cast<uint4*>(t.nodes + pslot)[0] = make_uint4((unsigned)(nvis + 1), __float_as_uint(pv), __float_as_uint(pvar), 0u);
-        pe->vis = cvis + 1;
-        *reinterpret_cast<float2*>(&pe->val) = make_float2(cval, cvarr);
-        s_back[32 + lev] = __float_as_uint(cval);  // for the refresh below: the traversed edge's new child value / variance
-        s_back[64 + lev] = __float_as_uint(cvarr);
-      }
-      const float b0v = __shfl_sync(0xffffffffu, pv, hbase), b0r = __shfl_sync(0xffffffffu, pvar, hbase);
-      if (cnt > 0) { below_val = b0v; below_var = b0r; }
-    }
-    __syncwarp();
+    staged2_backward<kG>(t, w, f, std_backup);
     if (lane == 0) trc.stamp(it, tw, 1);
     if (!do_select) continue;  // the last step only completes the backward
-
-    // ---- 3. refresh the cached selections of the path nodes and the leaf: staged records + this backward's updates
-    {
-      const int rounds = in_batch ? (L + kPR) / kPR : 0;  // ceil((L + 1) / kPR)
-      const int rmax = max(rounds, __shfl_xor_sync(0xffffffffu, rounds, kW));
-#pragma unroll 1
-      for (int r = 0; r < rmax; ++r) {
-        const int lev = r * kPR + glev;
-        const bool act_on = in_batch && lev <= L;
-        int node = 0, act_l = 0;
-        float cval_l = 0.0f, cvar_l = 0.0f;
-        if (act_on && lev < L) {
-          const uint32_t pa = s_back[lev];
-          node = (int)(pa & 0xffffu);
-          act_l = (int)(pa >> 16);
-          cval_l = __uint_as_float(s_back[32 + lev]);
-          cvar_l = __uint_as_float(s_back[64 + lev]);
-        } else if (act_on) {
-          node = leaf;
-        }
-        Edge<kG, 1> e;
-        e.ci[0] = -1; e.vis[0] = 0;
-        e.pl[0] = 0.0f; e.rew[0] = 0.0f; e.dis[0] = 0.0f; e.val[0] = 0.0f; e.vvar[0] = 0.0f;
-        float raw = 0.0f, raw_var = 0.0f, prior_p = 0.0f;
-        if (act_on) {
-          const uint32_t* sg0 = s_edge + r * kLaneWords * kW + (hl & ~(kG - 1));  // the group's action-0 lane always holds raw / raw variance
-          raw = __uint_as_float(sg0[7 * kW]);
-          raw_var = __uint_as_float(sg0[8 * kW]);
-          if (lev == L) { raw = value; raw_var = var; }  // the leaf: fresh raw values
-          if (gl < t.A) {
-            const uint32_t* se = s_edge + r * kLaneWords * kW + hl;
-            e.ci[0] = (int)se[0] - 1;
-            e.vis[0] = (int)se[1 * kW];
-            e.pl[0] = __uint_as_float(se[2 * kW]);
-            e.rew[0] = __uint_as_float(se[3 * kW]);
-            e.val[0] = __uint_as_float(se[4 * kW]);
-            e.vvar[0] = __uint_as_float(se[5 * kW]);
-            e.dis[0] = __uint_as_float(se[6 * kW]);
-            prior_p = __uint_as_float(se[9 * kW]);  // (unused for the fresh leaf: none of its children has visits)
-            if (lev == L) {
-              e.pl[0] = __uint_as_float(s_misc[8 + gl]);  // fresh priors
-            } else if (gl == act_l) {  // the edge this simulation went through
-              e.vis[0] += 1;
-              e.val[0] = cval_l;
-              e.vvar[0] = cvar_l;
-              if (lev == L - 1) { e.ci[0] = leaf; e.rew[0] = reward; e.dis[0] = disc; }
-            }
-          }
-        }
-        const bool is_root = act_on && node == 0;
-        float g2 = 0.0f;
-        bool inval = false;
-        int considered_visit = 0;
-        if (r == 0 && is_root && gl < t.A) {
-          g2 = __uint_as_float(s_root[gl]);
-          inval = s_root[2 + gl] != 0u;
-          considered_visit = (int)s_misc[0];
-        }
-        int child;
-        const int act = select_action_staged<kG>(sp, e, valid1[0], raw, raw_var, prior_p, beta, is_root, g2, inval, considered_visit, lane, gl, &child);
-        if (act_on && gl == 0) {
-          const int packed = pack_next(act, child);
-          t.nodes[(unsigned)node * uB + ub].pad0 = packed;
-          s_next[node] = (uint16_t)pack_next16(packed);
-        }
-      }
-    }
-    __syncwarp();
+    staged2_refresh<kG>(t, sp, w, f, beta, s_root, s_root + 2, s_misc, s_next);
     if (lane == 0) trc.stamp(it, tw, 2);
 
     // ---- 4. simulate: follow the cached selections (all 16 lanes of a tree run the same chase), then the DeepSea transition
@@ -699,7 +541,7 @@ __global__ void __launch_bounds__(kThreads, 1) ds_search_kernel(const __grid_con
       __syncwarp();
     }
     if (trc.buf) {
-      const int Lmax = max(L, __shfl_xor_sync(0xffffffffu, L, kW));
+      const int Lmax = max(L, __shfl_xor_sync(0xffffffffu, L, kStaged2Lanes));
       if (lane == 0) {
         trc.stamp(it, tw, 3);
         trc.path(it, tw, Lmax, 0);

@@ -30,6 +30,9 @@ namespace eaz {
 
 // cached selection in NodeRec.pad0: bits 0..7 action, bits 8.. child index + 1 (0 = unvisited)
 __device__ __forceinline__ int pack_next(int action, int child) { return action | ((child + 1) << 8); }
+__device__ __forceinline__ uint32_t pack_next16(int packed) {  // NodeRec.pad0 (action | child + 1 << 8) -> 16 bits (action | child + 1 << 2), A <= 4
+  return (uint32_t)(packed & 3) | ((uint32_t)(packed >> 8) << 2);
+}
 
 // gumbel_muzero_root_action_selection / gumbel_muzero_interior_action_selection for the lane group's node
 // (mctx action_selection.py; SURVEY A.3, A.6, A.7).  Returns the selected action; *child = children_index[node, act].
@@ -780,18 +783,229 @@ __global__ void __launch_bounds__(128, (G == 16 && J == 1) ? 8 : 1) tree_step_ke
 // arithmetic as tree_step_kernel; per tree the staging area holds 32 nodes (path + leaf) in rounds of 16 / G.  If either
 // tree of a pair cannot be staged (first launch, path longer than 31, re-expanded leaf, PUCT) both take the DIRECT path,
 // one after the other, with the whole warp.
+//
+// The staged step of one tree of a pair -- expand, backward, refresh (staged2_* below) -- is also the step of the persistent
+// DeepSea search (psearch.cuh: ds_search_kernel).  The two staging areas share the layout these functions read and write:
+//   edges  [round][word][lane of the tree]: in round r, node group glev = hl / G of the tree holds entry r * 16 / G + glev of
+//          (path nodes..., leaf) and lane gl = hl % G its action gl, in the ten words of staged2_store_lane;
+//   back   [node | action << 16, visits -> child value, value -> child variance, variance][level], levels 0..31;
+//   misc   [8 + a]: the fresh leaf's prior logits.
+// They differ in the number of rounds, in where the root's score terms are kept and in the width of the cached selections.
+constexpr int kStaged2Lanes = 16;          // lanes per tree
+constexpr int kStaged2LaneWords = 10;      // ci1, vis, pl, rew, val, vvar, dis, raw, rawvar, prior probability
+constexpr int kStaged2BackWords = 4 * 32;  // [node | action << 16, visits -> child value, value -> child variance, variance][level]
+
 template <int G>
 struct Stage2 {
-  static constexpr int kW = 16;                      // lanes per tree
-  static constexpr int kPerRound = kW / G;           // nodes refreshed per round
-  static constexpr int kRounds = 32 / kPerRound;     // 32 nodes (path + leaf) fit
-  static constexpr int kLaneWords = 10;              // ci1, vis, pl, rew, val, vvar, dis, raw, rawvar, prior probability
-  static constexpr int kEdgeWords = kRounds * kLaneWords * kW;  // [round][word][lane of the tree]
-  static constexpr int kBackWords = 4 * 32;          // [node | action << 16, visits -> child value, value -> child variance, variance][level]
-  static constexpr int kRootWords = 2 * kW;          // lanes 0..G-1: gumbel + (logit - max logit), invalid flag
-  static constexpr int kMiscWords = 16;              // [2] leaf terminal, [4] reward, [5] considered visit, [8..8+G) leaf priors
-  static __host__ __device__ constexpr int words(int chase_cap) { return kEdgeWords + kBackWords + kRootWords + kMiscWords + 2 * chase_cap; }
+  static constexpr int kPerRound = kStaged2Lanes / G;  // nodes refreshed per round
+  static constexpr int kRounds = 32 / kPerRound;       // 32 nodes (path + leaf) fit
+  static constexpr int kEdgeWords = kRounds * kStaged2LaneWords * kStaged2Lanes;
+  static constexpr int kRootWords = 2 * kStaged2Lanes;  // lanes 0..G-1: gumbel + (logit - max logit), invalid flag
+  static constexpr int kMiscWords = 16;                 // [2] leaf terminal, [4] reward, [5] considered visit, [8..8+G) leaf priors
+  static __host__ __device__ constexpr int words(int chase_cap) { return kEdgeWords + kStaged2BackWords + kRootWords + kMiscWords + 2 * chase_cap; }
 };
+
+// A lane of one tree of the pair: its coordinates, the tree's workspace column and its staging area
+struct Staged2Lane {
+  int lane, hl, hbase, gl, glev;  // lane of the warp, lane of the tree, the tree's first lane, action and node group of the lane
+  bool valid, in_batch;           // action gl exists (gl < A); the tree is in the batch
+  unsigned uB, uA, ub;            // batch, actions, the tree's column (0 outside the batch)
+  uint32_t *s_edge, *s_back, *s_misc;
+};
+// The expansion of one simulation: path length, leaf, the reward into the leaf, and what staged2_expand derives from the leaf's
+// network outputs: value, variance and the discount of the edge into the leaf
+struct Staged2Leaf {
+  int L, leaf;
+  float reward, value, var, disc;
+};
+
+// the ten-word record of one staged (node, action) lane in round r: the edge record's ci1, vis, pl, rew (h0) and val, vvar, dis (h1),
+// the node's raw value and variance (n1.x, n1.y) and p = max(tiny, softmax of the node's prior logits)
+__device__ __forceinline__ void staged2_store_lane(uint32_t* s_edge, int r, int hl, uint4 h0, uint4 h1, uint4 n1, float p) {
+  constexpr int kW = kStaged2Lanes;
+  uint32_t* se = s_edge + r * kStaged2LaneWords * kW + hl;
+  se[0 * kW] = h0.x; se[1 * kW] = h0.y; se[2 * kW] = h0.z; se[3 * kW] = h0.w;
+  se[4 * kW] = h1.x; se[5 * kW] = h1.y; se[6 * kW] = h1.z;
+  se[7 * kW] = n1.x; se[8 * kW] = n1.y;
+  se[9 * kW] = __float_as_uint(eaz_max(EAZ_F32_TINY, p));
+}
+
+// ---- 1. expand the fresh leaf at the end of a path of L levels: lane a of the tree holds action a's logit lg (A <= G, -inf on the
+// other lanes), nv / nu the leaf's value and UBE.  Writes the leaf's prior logits (edge records and s_misc[8 + a]), its node record and
+// the edge into it.
+template <int G>
+__device__ __forceinline__ Staged2Leaf staged2_expand(const Tree& t, const SearchParams& sp, const Staged2Lane& w, int L, int leaf, float reward,
+                                                      float lg, float nv, float nu, bool term) {
+  const unsigned lslot = (unsigned)leaf * w.uB + w.ub;
+  // context.py:135: the max over the logit lanes (all in the node group of the tree's first lane; fmaxf with -inf is exact)
+  const float m = __shfl_sync(0xffffffffu, group_max<G>(lg), w.hbase);
+  const float pl_leaf = __fsub_rn(lg, m);  // legal_action_mask is all True (:137)
+  if (w.in_batch && w.hl < t.A) {
+    t.edges[(size_t)(lslot * w.uA + w.hl)].pl = pl_leaf;
+    w.s_misc[8 + w.hl] = __float_as_uint(pl_leaf);
+  }
+  Staged2Leaf f{L, leaf, reward};
+  f.value = term ? 0.0f : nv;  // :140
+  f.var = term ? 0.0f : nu;    // :141
+  f.disc = sp.discount;
+  if (sp.two_players) f.disc = __fmul_rn(f.disc, -1.0f);  // :142-143
+  if (term) f.disc = 0.0f;                                // :144
+  if (w.in_batch && w.hl == 0) {
+    const uint32_t last = w.s_back[L - 1];
+    const int last_node = (int)(last & 0xffffu), last_act = (int)(last >> 16);
+    uint4* ln = reinterpret_cast<uint4*>(t.nodes + lslot);  // update_tree_node: a fresh leaf (staging condition)
+    ln[0] = make_uint4(1u, __float_as_uint(f.value), __float_as_uint(f.var), 0u);
+    ln[1] = make_uint4(__float_as_uint(f.value), __float_as_uint(f.var), (unsigned)(last_node + 1), (unsigned)(last_act + 1));
+    EdgeRec* pe0 = t.edges + (size_t)(((unsigned)last_node * w.uB + w.ub) * w.uA + (unsigned)last_act);
+    pe0->ci1 = leaf + 1;
+    pe0->rew = reward;  // :139
+    pe0->dis = f.disc;
+  }
+  return f;
+}
+
+// ---- 2. backward: rounds of 16 levels, deepest first; lane = level within the round.  std_backup: EAZ_FLAG_BACKUP_STD.  Leaves each
+// traversed edge's new child value / variance in s_back[32 / 64 + level] for the refresh.
+template <int G>
+__device__ __forceinline__ void staged2_backward(const Tree& t, const Staged2Lane& w, const Staged2Leaf& f, bool std_backup) {
+  constexpr int kW = kStaged2Lanes, kPR = kW / G;
+  const int L = f.L, hl = w.hl, hbase = w.hbase;
+  uint32_t* const s_back = w.s_back;
+  float lv = f.value, lvar = std_backup ? __fsqrt_rn(f.var) : f.var;
+  float below_val = f.value, below_var = f.var;
+  const int Lw = max(L, __shfl_xor_sync(0xffffffffu, L, kW));
+#pragma unroll 1
+  for (int k = Lw > kW ? 1 : 0; k >= 0; --k) {
+    const int lo = kW * k, cnt = min(max(L - lo, 0), kW);
+    const int lev = lo + hl;
+    const bool have = w.in_batch && hl < cnt;
+    int my_node = 0, my_act = 0, nvis = 0, cvis = 0;
+    float nval = 0.0f, nvar = 0.0f, rr = 0.0f, dd = 0.0f;
+    if (have) {
+      const uint32_t pa = s_back[lev];
+      my_node = (int)(pa & 0xffffu);
+      my_act = (int)(pa >> 16);
+      nvis = (int)s_back[32 + lev];
+      nval = __uint_as_float(s_back[64 + lev]);
+      nvar = __uint_as_float(s_back[96 + lev]);
+      const uint32_t* se = w.s_edge + (lev / kPR) * kStaged2LaneWords * kW + (lev % kPR) * G + my_act;  // the traversed edge in the refresh staging
+      cvis = (int)se[1 * kW];
+      rr = __uint_as_float(se[3 * kW]);
+      dd = __uint_as_float(se[6 * kW]);
+      if (lev == L - 1) { rr = f.reward; dd = f.disc; }  // written by the expand step
+    }
+    const int cmax = max(cnt, __shfl_xor_sync(0xffffffffu, cnt, kW));
+    float my_lv = 0.0f, my_lvar = 0.0f;
+    for (int i = cmax - 1; i >= 0; --i) {  // the recurrences, in the reference's op order
+      const float r = __shfl_sync(0xffffffffu, rr, hbase + i), d = __shfl_sync(0xffffffffu, dd, hbase + i);
+      if (i < cnt) {
+        lv = __fadd_rn(r, __fmul_rn(d, lv));
+        lvar = std_backup ? __fadd_rn(0.0f, __fmul_rn(fabsf(d), lvar)) : __fadd_rn(0.0f, __fmul_rn(__fmul_rn(d, d), lvar));
+        if (hl == i) { my_lv = lv; my_lvar = lvar; }
+      }
+    }
+    const float count = (float)nvis;
+    const float pv = __fdiv_rn(__fadd_rn(__fmul_rn(nval, count), my_lv), __fadd_rn(count, 1.0f));
+    float pvar;
+    if (std_backup) {
+      const float psd = __fdiv_rn(__fadd_rn(__fmul_rn(__fsqrt_rn(nvar), count), my_lvar), __fadd_rn(count, 1.0f));
+      pvar = __fmul_rn(psd, psd);
+    } else {
+      pvar = __fdiv_rn(__fadd_rn(__fmul_rn(nvar, count), my_lvar), __fadd_rn(count, 1.0f));
+    }
+    // children_values[parent, a] = the child's CURRENT (already updated) mean: one level deeper
+    float cval = __shfl_down_sync(0xffffffffu, pv, 1, kW), cvarr = __shfl_down_sync(0xffffffffu, pvar, 1, kW);
+    if (hl == cnt - 1) { cval = below_val; cvarr = below_var; }
+    if (have) {
+      const unsigned pslot = (unsigned)my_node * w.uB + w.ub;
+      EdgeRec* pe = t.edges + (size_t)(pslot * w.uA + (unsigned)my_act);
+      reinterpret_cast<uint4*>(t.nodes + pslot)[0] = make_uint4((unsigned)(nvis + 1), __float_as_uint(pv), __float_as_uint(pvar), 0u);
+      pe->vis = cvis + 1;
+      *reinterpret_cast<float2*>(&pe->val) = make_float2(cval, cvarr);
+      s_back[32 + lev] = __float_as_uint(cval);  // for the refresh: the traversed edge's new child value / variance
+      s_back[64 + lev] = __float_as_uint(cvarr);
+    }
+    const float b0v = __shfl_sync(0xffffffffu, pv, hbase), b0r = __shfl_sync(0xffffffffu, pvar, hbase);
+    if (cnt > 0) { below_val = b0v; below_var = b0r; }
+  }
+  __syncwarp();
+}
+
+// ---- 3. refresh the cached selections of the path nodes and the leaf: staged records + this backward's updates.  The root's score
+// terms: root_g2[a] = gumbel + (logit - max logit), root_inval[a] its invalid flag, *considered the seq-halving visit target.  The
+// selection is cached in the node record and in s_next[node]: 32 bits as NodeRec.pad0, or 16 bits (pack_next16).
+template <int G, typename NextT>
+__device__ __forceinline__ void staged2_refresh(const Tree& t, const SearchParams& sp, const Staged2Lane& w, const Staged2Leaf& f, float beta,
+                                                const uint32_t* root_g2, const uint32_t* root_inval, const uint32_t* considered, NextT* s_next) {
+  constexpr int kW = kStaged2Lanes, kPR = kW / G;
+  const int L = f.L, hl = w.hl, gl = w.gl;
+  const uint32_t* const s_back = w.s_back;
+  const int rounds = w.in_batch ? (L + kPR) / kPR : 0;  // ceil((L + 1) / kPR)
+  const int rmax = max(rounds, __shfl_xor_sync(0xffffffffu, rounds, kW));
+#pragma unroll 1
+  for (int r = 0; r < rmax; ++r) {
+    const int lev = r * kPR + w.glev;
+    const bool act_on = w.in_batch && lev <= L;
+    int node = 0, act_l = 0;
+    float cval_l = 0.0f, cvar_l = 0.0f;
+    if (act_on && lev < L) {
+      const uint32_t pa = s_back[lev];
+      node = (int)(pa & 0xffffu);
+      act_l = (int)(pa >> 16);
+      cval_l = __uint_as_float(s_back[32 + lev]);
+      cvar_l = __uint_as_float(s_back[64 + lev]);
+    } else if (act_on) {
+      node = f.leaf;
+    }
+    Edge<G, 1> e;
+    e.ci[0] = -1; e.vis[0] = 0;
+    e.pl[0] = 0.0f; e.rew[0] = 0.0f; e.dis[0] = 0.0f; e.val[0] = 0.0f; e.vvar[0] = 0.0f;
+    float raw = 0.0f, raw_var = 0.0f, prior_p = 0.0f;
+    if (act_on) {
+      const uint32_t* sg0 = w.s_edge + r * kStaged2LaneWords * kW + (hl & ~(G - 1));  // the group's action-0 lane always holds raw / raw variance
+      raw = __uint_as_float(sg0[7 * kW]);
+      raw_var = __uint_as_float(sg0[8 * kW]);
+      if (lev == L) { raw = f.value; raw_var = f.var; }  // the leaf: fresh raw values
+      if (gl < t.A) {
+        const uint32_t* se = w.s_edge + r * kStaged2LaneWords * kW + hl;
+        e.ci[0] = (int)se[0] - 1;
+        e.vis[0] = (int)se[1 * kW];
+        e.pl[0] = __uint_as_float(se[2 * kW]);
+        e.rew[0] = __uint_as_float(se[3 * kW]);
+        e.val[0] = __uint_as_float(se[4 * kW]);
+        e.vvar[0] = __uint_as_float(se[5 * kW]);
+        e.dis[0] = __uint_as_float(se[6 * kW]);
+        prior_p = __uint_as_float(se[9 * kW]);  // (unused for the fresh leaf: none of its children has visits)
+        if (lev == L) {
+          e.pl[0] = __uint_as_float(w.s_misc[8 + gl]);  // fresh priors
+        } else if (gl == act_l) {  // the edge this simulation went through
+          e.vis[0] += 1;
+          e.val[0] = cval_l;
+          e.vvar[0] = cvar_l;
+          if (lev == L - 1) { e.ci[0] = f.leaf; e.rew[0] = f.reward; e.dis[0] = f.disc; }
+        }
+      }
+    }
+    const bool is_root = act_on && node == 0;  // (only at level 0: lane gl of the tree's first node group)
+    float g2 = 0.0f;
+    bool inval = false;
+    int considered_visit = 0;
+    if (r == 0 && is_root && gl < t.A) {
+      g2 = __uint_as_float(root_g2[gl]);
+      inval = root_inval[gl] != 0u;
+      considered_visit = (int)*considered;
+    }
+    int child;
+    const int act = select_action_staged<G>(sp, e, w.valid, raw, raw_var, prior_p, beta, is_root, g2, inval, considered_visit, w.lane, gl, &child);
+    if (act_on && gl == 0) {
+      const int packed = pack_next(act, child);
+      t.nodes[(unsigned)node * w.uB + w.ub].pad0 = packed;
+      if constexpr (sizeof(NextT) == 2) s_next[node] = (NextT)pack_next16(packed);
+      else s_next[node] = (NextT)packed;
+    }
+  }
+  __syncwarp();
+}
 
 template <int G>
 __global__ void __launch_bounds__(128) tree_step2_kernel(Tree t, SearchParams sp, EnvDesc env, int sim, int do_backward, int do_select,
@@ -801,7 +1015,7 @@ __global__ void __launch_bounds__(128) tree_step2_kernel(Tree t, SearchParams sp
   unsigned long long t_entry = 0;
   if (tl && blockIdx.x == 0 && threadIdx.x == 0) t_entry = globaltimer_ns();
   using SG = Stage2<G>;
-  constexpr int kW = SG::kW, kPR = SG::kPerRound;
+  constexpr int kW = kStaged2Lanes, kPR = SG::kPerRound;
   const int lane = threadIdx.x & 31, hl = lane & (kW - 1), hbase = lane & kW, sub = lane >> 4;
   const int warp_global = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int b = 2 * warp_global + sub;  // 16 lanes per tree
@@ -812,7 +1026,7 @@ __global__ void __launch_bounds__(128) tree_step2_kernel(Tree t, SearchParams sp
   uint32_t* const sw = stage_smem + ((threadIdx.x >> 5) * 2 + sub) * SG::words(chase_cap);
   uint32_t* const s_edge = sw;
   uint32_t* const s_back = sw + SG::kEdgeWords;
-  uint32_t* const s_root = s_back + SG::kBackWords;
+  uint32_t* const s_root = s_back + kStaged2BackWords;
   uint32_t* const s_misc = s_root + SG::kRootWords;
   uint32_t* const s_next = s_misc + SG::kMiscWords;
   uint32_t* const s_state = s_next + chase_cap;
@@ -863,13 +1077,7 @@ __global__ void __launch_bounds__(128) tree_step2_kernel(Tree t, SearchParams sp
           const float xl[1] = {__uint_as_float(h0.z)};
           float pr[1];
           group_softmax<G, 1>(xl, valid1, pr);  // p = max(tiny, softmax(prior logits)) of _compute_mixed_value
-          if (on) {
-            uint32_t* se = s_edge + r * SG::kLaneWords * kW + hl;
-            se[0 * kW] = h0.x; se[1 * kW] = h0.y; se[2 * kW] = h0.z; se[3 * kW] = h0.w;
-            se[4 * kW] = h1.x; se[5 * kW] = h1.y; se[6 * kW] = h1.z;
-            se[7 * kW] = n1.x; se[8 * kW] = n1.y;
-            se[9 * kW] = __float_as_uint(eaz_max(EAZ_F32_TINY, pr[0]));
-          }
+          if (on) staged2_store_lane(s_edge, r, hl, h0, h1, n1, pr[0]);
           if (r == 0) {  // the root is level 0 of every path: its seq-halving score terms
             const bool rt = in_batch && glev == 0 && gl < t.A;
             const float gum = rt ? t.gumbel[ub * uA + gl] : 0.0f;
@@ -929,168 +1137,16 @@ __global__ void __launch_bounds__(128) tree_step2_kernel(Tree t, SearchParams sp
   long long* trc = (trace && hl == 0 && in_batch) ? trace + ((size_t)sim * t.B + b) * 8 : nullptr;
   if (trc) { trc[0] = clock64(); trc[7] = 2; }
   const float beta = (in_batch && beta_in) ? beta_in[b] : 0.0f;
-  const unsigned lslot = (unsigned)leaf * uB + ub;
-  // ---- 1. expand (lane a of the tree holds action a's logit)
+  const Staged2Lane w{lane, hl, hbase, gl, glev, valid1[0], in_batch, uB, uA, ub, s_edge, s_back, s_misc};
+  // ---- 1. expand (lane a of the tree holds action a's logit), 2. backward, 3. refresh
   const float lg = (in_batch && hl < t.A) ? t.net_logits[ub * uA + hl] : -INFINITY;
-  const float nv = in_batch ? t.net_value[b] : 0.0f, nu = in_batch ? t.net_ube[b] : 0.0f;
-  float m = lg;
-#pragma unroll
-  for (int s = kW / 2; s > 0; s >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, s));  // context.py:135 (within the tree's 16 lanes)
-  const float pl_leaf = __fsub_rn(lg, m);                                                  // legal_action_mask is all True (:137)
-  if (in_batch && hl < t.A) {
-    t.edges[(size_t)(lslot * uA + hl)].pl = pl_leaf;
-    s_misc[8 + hl] = __float_as_uint(pl_leaf);
-  }
-  const int term = in_batch ? (int)s_misc[2] : 0;
-  const float value = term ? 0.0f : nv;  // :140
-  const float var = term ? 0.0f : nu;    // :141
-  float disc = sp.discount;
-  if (sp.two_players) disc = __fmul_rn(disc, -1.0f);  // :142-143
-  if (term) disc = 0.0f;                              // :144
-  const float reward = in_batch ? __uint_as_float(s_misc[4]) : 0.0f;
-  if (in_batch && hl == 0) {
-    const uint32_t last = s_back[L - 1];
-    const int last_node = (int)(last & 0xffffu), last_act = (int)(last >> 16);
-    uint4* ln = reinterpret_cast<uint4*>(t.nodes + lslot);  // update_tree_node: a fresh leaf (staging condition)
-    ln[0] = make_uint4(1u, __float_as_uint(value), __float_as_uint(var), 0u);
-    ln[1] = make_uint4(__float_as_uint(value), __float_as_uint(var), (unsigned)(last_node + 1), (unsigned)(last_act + 1));
-    EdgeRec* pe0 = t.edges + (size_t)(((unsigned)last_node * uB + ub) * uA + (unsigned)last_act);
-    pe0->ci1 = leaf + 1;
-    pe0->rew = reward;  // :139
-    pe0->dis = disc;
-  }
+  const Staged2Leaf f = staged2_expand<G>(t, sp, w, L, leaf, in_batch ? __uint_as_float(s_misc[4]) : 0.0f, lg, in_batch ? t.net_value[b] : 0.0f,
+                                          in_batch ? t.net_ube[b] : 0.0f, in_batch && s_misc[2] != 0u);
   if (trc) trc[1] = clock64();
-
-  // ---- 2. backward: rounds of 16 levels, deepest first; lane = level within the round
-  const bool std_backup = (sp.flags & EAZ_FLAG_BACKUP_STD) != 0;
-  float lv = value, lvar = std_backup ? __fsqrt_rn(var) : var;
-  float below_val = value, below_var = var;
-  const int Lw = max(L, __shfl_xor_sync(0xffffffffu, L, kW));
-#pragma unroll 1
-  for (int k = Lw > kW ? 1 : 0; k >= 0; --k) {
-    const int lo = kW * k, cnt = min(max(L - lo, 0), kW);
-    const int lev = lo + hl;
-    const bool have = in_batch && hl < cnt;
-    int my_node = 0, my_act = 0, nvis = 0, cvis = 0;
-    float nval = 0.0f, nvar = 0.0f, rr = 0.0f, dd = 0.0f;
-    if (have) {
-      const uint32_t pa = s_back[lev];
-      my_node = (int)(pa & 0xffffu);
-      my_act = (int)(pa >> 16);
-      nvis = (int)s_back[32 + lev];
-      nval = __uint_as_float(s_back[64 + lev]);
-      nvar = __uint_as_float(s_back[96 + lev]);
-      const uint32_t* se = s_edge + (lev / kPR) * SG::kLaneWords * kW + (lev % kPR) * G + my_act;  // the traversed edge in the refresh staging
-      cvis = (int)se[1 * kW];
-      rr = __uint_as_float(se[3 * kW]);
-      dd = __uint_as_float(se[6 * kW]);
-      if (lev == L - 1) { rr = reward; dd = disc; }  // written by the expand step above
-    }
-    const int cmax = max(cnt, __shfl_xor_sync(0xffffffffu, cnt, kW));
-    float my_lv = 0.0f, my_lvar = 0.0f;
-    for (int i = cmax - 1; i >= 0; --i) {  // the recurrences, in the reference's op order
-      const float r = __shfl_sync(0xffffffffu, rr, hbase + i), d = __shfl_sync(0xffffffffu, dd, hbase + i);
-      if (i < cnt) {
-        lv = __fadd_rn(r, __fmul_rn(d, lv));
-        lvar = std_backup ? __fadd_rn(0.0f, __fmul_rn(fabsf(d), lvar)) : __fadd_rn(0.0f, __fmul_rn(__fmul_rn(d, d), lvar));
-        if (hl == i) { my_lv = lv; my_lvar = lvar; }
-      }
-    }
-    const float count = (float)nvis;
-    const float pv = __fdiv_rn(__fadd_rn(__fmul_rn(nval, count), my_lv), __fadd_rn(count, 1.0f));
-    float pvar;
-    if (std_backup) {
-      const float ps = __fdiv_rn(__fadd_rn(__fmul_rn(__fsqrt_rn(nvar), count), my_lvar), __fadd_rn(count, 1.0f));
-      pvar = __fmul_rn(ps, ps);
-    } else {
-      pvar = __fdiv_rn(__fadd_rn(__fmul_rn(nvar, count), my_lvar), __fadd_rn(count, 1.0f));
-    }
-    // children_values[parent, a] = the child's CURRENT (already updated) mean: one level deeper
-    float cval = __shfl_down_sync(0xffffffffu, pv, 1, kW), cvarr = __shfl_down_sync(0xffffffffu, pvar, 1, kW);
-    if (hl == cnt - 1) { cval = below_val; cvarr = below_var; }
-    if (have) {
-      const unsigned pslot = (unsigned)my_node * uB + ub;
-      EdgeRec* pe = t.edges + (size_t)(pslot * uA + (unsigned)my_act);
-      reinterpret_cast<uint4*>(t.nodes + pslot)[0] = make_uint4((unsigned)(nvis + 1), __float_as_uint(pv), __float_as_uint(pvar), 0u);
-      pe->vis = cvis + 1;
-      *reinterpret_cast<float2*>(&pe->val) = make_float2(cval, cvarr);
-      s_back[32 + lev] = __float_as_uint(cval);  // for the refresh below: the traversed edge's new child value / variance
-      s_back[64 + lev] = __float_as_uint(cvarr);
-    }
-    const float b0v = __shfl_sync(0xffffffffu, pv, hbase), b0r = __shfl_sync(0xffffffffu, pvar, hbase);
-    if (cnt > 0) { below_val = b0v; below_var = b0r; }
-  }
-  __syncwarp();
+  staged2_backward<G>(t, w, f, (sp.flags & EAZ_FLAG_BACKUP_STD) != 0);
   if (trc) { trc[2] = clock64(); trc[6] = L; }
   if (!do_select) return;
-
-  // ---- 3. refresh the cached selections of the path nodes and the leaf: staged records + this backward's updates
-  {
-    const int rounds = in_batch ? (L + kPR) / kPR : 0;  // ceil((L + 1) / kPR)
-    const int rmax = max(rounds, __shfl_xor_sync(0xffffffffu, rounds, kW));
-#pragma unroll 1
-    for (int r = 0; r < rmax; ++r) {
-      const int lev = r * kPR + glev;
-      const bool act_on = in_batch && lev <= L;
-      int node = 0, act_l = 0;
-      float cval_l = 0.0f, cvar_l = 0.0f;
-      if (act_on && lev < L) {
-        const uint32_t pa = s_back[lev];
-        node = (int)(pa & 0xffffu);
-        act_l = (int)(pa >> 16);
-        cval_l = __uint_as_float(s_back[32 + lev]);
-        cvar_l = __uint_as_float(s_back[64 + lev]);
-      } else if (act_on) {
-        node = leaf;
-      }
-      Edge<G, 1> e;
-      e.ci[0] = -1; e.vis[0] = 0;
-      e.pl[0] = 0.0f; e.rew[0] = 0.0f; e.dis[0] = 0.0f; e.val[0] = 0.0f; e.vvar[0] = 0.0f;
-      float raw = 0.0f, raw_var = 0.0f, prior_p = 0.0f;
-      if (act_on) {
-        const uint32_t* sg0 = s_edge + r * SG::kLaneWords * kW + (hl & ~(G - 1));  // the group's action-0 lane always holds raw / raw variance
-        raw = __uint_as_float(sg0[7 * kW]);
-        raw_var = __uint_as_float(sg0[8 * kW]);
-        if (lev == L) { raw = value; raw_var = var; }  // the leaf: fresh raw values
-        if (gl < t.A) {
-          const uint32_t* se = s_edge + r * SG::kLaneWords * kW + hl;
-          e.ci[0] = (int)se[0] - 1;
-          e.vis[0] = (int)se[1 * kW];
-          e.pl[0] = __uint_as_float(se[2 * kW]);
-          e.rew[0] = __uint_as_float(se[3 * kW]);
-          e.val[0] = __uint_as_float(se[4 * kW]);
-          e.vvar[0] = __uint_as_float(se[5 * kW]);
-          e.dis[0] = __uint_as_float(se[6 * kW]);
-          prior_p = __uint_as_float(se[9 * kW]);  // (unused for the fresh leaf: none of its children has visits)
-          if (lev == L) {
-            e.pl[0] = __uint_as_float(s_misc[8 + gl]);  // fresh priors
-          } else if (gl == act_l) {  // the edge this simulation went through
-            e.vis[0] += 1;
-            e.val[0] = cval_l;
-            e.vvar[0] = cvar_l;
-            if (lev == L - 1) { e.ci[0] = leaf; e.rew[0] = reward; e.dis[0] = disc; }
-          }
-        }
-      }
-      const bool is_root = act_on && node == 0;
-      float g2 = 0.0f;
-      bool inval = false;
-      int considered_visit = 0;
-      if (r == 0 && is_root && gl < t.A) {
-        g2 = __uint_as_float(s_root[hl]);
-        inval = s_root[kW + hl] != 0u;
-        considered_visit = (int)s_misc[5];
-      }
-      int child;
-      const int act = select_action_staged<G>(sp, e, valid1[0], raw, raw_var, prior_p, beta, is_root, g2, inval, considered_visit, lane, gl, &child);
-      if (act_on && gl == 0) {
-        const int packed = pack_next(act, child);
-        t.nodes[(unsigned)node * uB + ub].pad0 = packed;
-        s_next[node] = (uint32_t)packed;
-      }
-    }
-  }
-  __syncwarp();
+  staged2_refresh<G>(t, sp, w, f, beta, s_root, s_root + kStaged2Lanes, s_misc + 5, s_next);
   if (trc) trc[3] = clock64();
 
   // ---- 4. simulate: follow the cached selections through the staged copy (each tree until its own descent ends)
