@@ -8,7 +8,7 @@ from __future__ import annotations
 
 import ctypes as C
 
-ABI_VERSION = 5
+ABI_VERSION = 6
 
 EAZ_OK = 0
 EAZ_ERR_INVALID_ARG = -1
@@ -306,6 +306,10 @@ ROOT_FIELDS = [f for f in SEARCH_OUTPUT_FIELDS[24:]]  # fused-root mode
 
 class EazSearchOutputs(C.Structure):
     _fields_ = [(name, _p) for name, _, _ in SEARCH_OUTPUT_FIELDS]
+
+
+class EazEvaluateCounters(C.Structure):  # the evaluation loop's device words at the start of the eaz_evaluate workspace
+    _fields_ = [("moves", C.c_int32), ("live", C.c_int32), ("ticket", C.c_uint32), ("cont", C.c_int32)]
 
 
 def default_search_config(**kw) -> EazSearchConfig:

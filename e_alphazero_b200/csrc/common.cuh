@@ -88,6 +88,10 @@ static inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 b
   return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
 }
 
+// Internal eaz_search_config.flags bit (set by eaz_evaluate, never by a caller): enqueue only the search's preparation -- the tree
+// memset, the root states and, unless EAZ_FLAG_REUSE_PREPARED, the parameter-derived tables -- and no simulation.
+constexpr int kFlagPrepareOnly = 1 << 28;
+
 // ---------------------------------------------------------------- env description (by value into kernels)
 struct EnvDesc {
   int kind;
@@ -668,5 +672,94 @@ __device__ __forceinline__ void sq_run_tests_block(SqShared& sh, uint8_t* dyn, i
     }
   }
   __syncthreads();
+}
+
+// ---------------------------------------------------------------- pgx.Env.step on struct-of-arrays states (env.cu, evaluate.cu)
+// DeepSea, one env per thread; auto_reset applies selfplay.py:66-71 to an env that is already terminal.
+__device__ __forceinline__ void deepsea_state_step(const EnvDesc& env, const StateSoA& s, const int32_t* __restrict__ action, int auto_reset, int b) {
+  const int term = s.terminated[b] != 0, trunc = s.truncated ? (s.truncated[b] != 0) : 0;
+  if (auto_reset && (term | trunc)) {  // selfplay.py:66-71
+    s.step_count[b] = 0;
+    s.col[b] = 0;
+    s.rewards[b] = 0.0f;
+    s.terminated[b] = 0;
+    if (s.truncated) s.truncated[b] = 0;
+    return;
+  }
+  float reward;
+  const uint32_t n = deepsea_step(ds_pack(s.step_count[b], s.col[b], term, trunc), action[b], env.size, env.action_map, &reward);
+  s.step_count[b] = EAZ_DS_STEP(n);
+  s.col[b] = EAZ_DS_COL(n);
+  s.terminated[b] = (uint8_t)EAZ_DS_TERM(n);
+  s.rewards[b] = reward;
+}
+
+// Subleq, EAZ_SQ_EPB envs per block of 3*EAZ_SQ_EPB threads (all of them call this; `dyn` = sq_dyn_smem_bytes of dynamic shared
+// memory).  mode: 0 = init (task from task_ids), 1 = step, 2 = step with auto_reset.  On return thread (e, 0) has written env e's leaves.
+__device__ __forceinline__ void subleq_block_step(const EnvDesc& env, const StateSoA& s, const int32_t* __restrict__ action,
+                                                  const int32_t* __restrict__ task_ids, int mode, int B, SqShared& sh, uint8_t* dyn,
+                                                  int* kind /* [EAZ_SQ_EPB] shared: 0 absorbing, 1 terminate now, 2 execute, 3 init/reset */) {
+  const int ws = env.ws;
+  const int e = threadIdx.x / 3, k = threadIdx.x % 3;
+  const int b = blockIdx.x * EAZ_SQ_EPB + e;
+  if (k == 0) {
+    int kd = -1, run = 0;
+    if (b < B) {
+      const int term = s.terminated[b] != 0, trunc = s.truncated ? (s.truncated[b] != 0) : 0;
+      if (mode == 0 || (mode == 2 && (term | trunc))) {
+        const int task = task_ids ? task_ids[b] : (mode == 0 ? 1 : s.task[b]);
+        s.task[b] = task;
+        sh.trow[e] = sq_task_row(task);
+        for (int i = 0; i < ws; i += 1) sh.base[e][i] = 0;  // empty program, subleq.py:630
+        kd = 3;
+        run = 1;
+      } else if (term | trunc) {
+        kd = 0;
+      } else {
+        const int step = s.step_count[b] + 1;
+        s.step_count[b] = step;
+        if (step >= ws - 3 || s.solved[b]) {  // subleq.py:671-673
+          kd = 1;
+        } else {
+          sh.trow[e] = sq_task_row(s.task[b]);
+          const int32_t* m = s.memory + (size_t)b * ws;
+          for (int i = 0; i < ws; ++i) sh.base[e][i] = (uint8_t)m[i];
+          sh.base[e][step - 1] = (uint8_t)action[b];  // :654
+          kd = 2;
+          run = 1;
+        }
+      }
+    }
+    kind[e] = kd;
+    sh.run[e] = run;
+  }
+  __syncthreads();
+  sq_run_tests_block(sh, dyn, ws);
+  if (k != 0 || b >= B) return;
+  const int kd = kind[e];
+  if (kd == 0) {
+    s.rewards[b] = 0.0f;
+  } else if (kd == 1) {
+    s.terminated[b] = 1;
+    s.rewards[b] = 0.0f;
+  } else if (kd >= 2) {
+    const int solved = sh.correct[e][0] & sh.correct[e][1] & sh.correct[e][2];
+    const int bytes = max(sh.bytes[e][0], max(sh.bytes[e][1], sh.bytes[e][2]));
+    s.rewards[b] = subleq_reward(env.reward_fn, solved, bytes);
+    s.solved[b] = (uint8_t)solved;
+    int32_t* m = s.memory + (size_t)b * ws;
+    if (kd == 3) {
+      for (int i = 0; i < ws; ++i) m[i] = 0;
+      s.step_count[b] = 0;
+      s.terminated[b] = 0;
+      if (s.truncated) s.truncated[b] = 0;
+    } else {
+      m[s.step_count[b] - 1] = action[b];
+    }
+    for (int i = 0; i < 8; ++i) {
+      s.input_after[(size_t)b * 8 + i] = sh.in_after[e][i];
+      s.output_after[(size_t)b * 8 + i] = sh.out_after[e][i];
+    }
+  }
 }
 }  // namespace eaz

@@ -66,21 +66,7 @@ __global__ void deepsea_init_kernel(StateSoA s, int B) {
 __global__ void deepsea_step_kernel(EnvDesc env, StateSoA s, const int32_t* __restrict__ action, int auto_reset, int B) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
-  const int term = s.terminated[b] != 0, trunc = s.truncated ? (s.truncated[b] != 0) : 0;
-  if (auto_reset && (term | trunc)) {  // selfplay.py:66-71
-    s.step_count[b] = 0;
-    s.col[b] = 0;
-    s.rewards[b] = 0.0f;
-    s.terminated[b] = 0;
-    if (s.truncated) s.truncated[b] = 0;
-    return;
-  }
-  float reward;
-  const uint32_t n = deepsea_step(ds_pack(s.step_count[b], s.col[b], term, trunc), action[b], env.size, env.action_map, &reward);
-  s.step_count[b] = EAZ_DS_STEP(n);
-  s.col[b] = EAZ_DS_COL(n);
-  s.terminated[b] = (uint8_t)EAZ_DS_TERM(n);
-  s.rewards[b] = reward;
+  deepsea_state_step(env, s, action, auto_reset, b);
 }
 
 // one-hot [N,N] observation, 16 bytes per thread
@@ -103,69 +89,8 @@ __global__ void __launch_bounds__(3 * EAZ_SQ_EPB) subleq_kernel(EnvDesc env, Sta
                                                                  const int32_t* __restrict__ task_ids, int mode, int B) {
   __shared__ SqShared sh;
   extern __shared__ __align__(16) uint8_t sq_dyn[];  // per-(env, test) memory images + cycle-detector snapshots
-  __shared__ int kind[EAZ_SQ_EPB];  // 0 absorbing, 1 terminate now, 2 execute, 3 init/reset
-  const int ws = env.ws;
-  const int e = threadIdx.x / 3, k = threadIdx.x % 3;
-  const int b = blockIdx.x * EAZ_SQ_EPB + e;
-  if (k == 0) {
-    int kd = -1, run = 0;
-    if (b < B) {
-      const int term = s.terminated[b] != 0, trunc = s.truncated ? (s.truncated[b] != 0) : 0;
-      if (mode == 0 || (mode == 2 && (term | trunc))) {
-        const int task = task_ids ? task_ids[b] : (mode == 0 ? 1 : s.task[b]);
-        s.task[b] = task;
-        sh.trow[e] = sq_task_row(task);
-        for (int i = 0; i < ws; i += 1) sh.base[e][i] = 0;  // empty program, subleq.py:630
-        kd = 3;
-        run = 1;
-      } else if (term | trunc) {
-        kd = 0;
-      } else {
-        const int step = s.step_count[b] + 1;
-        s.step_count[b] = step;
-        if (step >= ws - 3 || s.solved[b]) {  // subleq.py:671-673
-          kd = 1;
-        } else {
-          sh.trow[e] = sq_task_row(s.task[b]);
-          const int32_t* m = s.memory + (size_t)b * ws;
-          for (int i = 0; i < ws; ++i) sh.base[e][i] = (uint8_t)m[i];
-          sh.base[e][step - 1] = (uint8_t)action[b];  // :654
-          kd = 2;
-          run = 1;
-        }
-      }
-    }
-    kind[e] = kd;
-    sh.run[e] = run;
-  }
-  __syncthreads();
-  sq_run_tests_block(sh, sq_dyn, ws);
-  if (k != 0 || b >= B) return;
-  const int kd = kind[e];
-  if (kd == 0) {
-    s.rewards[b] = 0.0f;
-  } else if (kd == 1) {
-    s.terminated[b] = 1;
-    s.rewards[b] = 0.0f;
-  } else if (kd >= 2) {
-    const int solved = sh.correct[e][0] & sh.correct[e][1] & sh.correct[e][2];
-    const int bytes = max(sh.bytes[e][0], max(sh.bytes[e][1], sh.bytes[e][2]));
-    s.rewards[b] = subleq_reward(env.reward_fn, solved, bytes);
-    s.solved[b] = (uint8_t)solved;
-    int32_t* m = s.memory + (size_t)b * ws;
-    if (kd == 3) {
-      for (int i = 0; i < ws; ++i) m[i] = 0;
-      s.step_count[b] = 0;
-      s.terminated[b] = 0;
-      if (s.truncated) s.truncated[b] = 0;
-    } else {
-      m[s.step_count[b] - 1] = action[b];
-    }
-    for (int i = 0; i < 8; ++i) {
-      s.input_after[(size_t)b * 8 + i] = sh.in_after[e][i];
-      s.output_after[(size_t)b * 8 + i] = sh.out_after[e][i];
-    }
-  }
+  __shared__ int kind[EAZ_SQ_EPB];
+  subleq_block_step(env, s, action, task_ids, mode, B, sh, sq_dyn, kind);
 }
 
 // Subleq._observe (subleq.py:679-707): one thread per observation row.

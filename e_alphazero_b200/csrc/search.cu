@@ -1235,6 +1235,7 @@ static int search_one(const eaz_search_config* cfg, const eaz_search_inputs* in,
       if (int rc = launch_output_table(t, env, net, tw, lhead, st)) return rc;
   }
   }
+  if (cfg->flags & kFlagPrepareOnly) return 0;
 
   SummaryOut so{out->action, out->action_weights, out->value, out->value_epistemic_std, out->visit_counts, out->visit_probs,
                 out->qvalues, out->qvalues_epistemic_variance};

@@ -5,6 +5,8 @@
 //
 //   eaz_search          emctx.epistemic_gumbel_muzero_policy + Tree.epistemic_summary   selfplay.py:100-121, reanalyze.py:70-86,
 //                       (DeepSea and Subleq; recurrent_fn of context.py:109-157 fused)    evaluate.py:29-45
+//   eaz_evaluate        the evaluate() episode loop (search + env step + reward sum under  evaluate.py:13-57
+//                       a device-decided while condition)
 //   eaz_env_step        pgx Env.step / selfplay.auto_reset                               selfplay.py:26-75,135, evaluate.py:47
 //   eaz_env_init        pgx Env.init (vmapped)                                           selfplay.py:161,166, main.py:205
 //   eaz_mlp_forward_states   forward.apply(params, state, states.observation)            selfplay.py:89, reanalyze.py:67,90
@@ -278,6 +280,67 @@ ffi::Error SearchImpl(cudaStream_t stream, ffi::Buffer<ffi::F32> beta, ffi::Buff
     out.root_ube = root_ube->typed_data();
   }
   return EazError(eaz_search_gumbel(&cfg, &in, &out, ws, ws_bytes, stream), "eaz_search_gumbel");
+}
+
+// ------------------------------------------------------------------------------------------------ evaluation episodes
+// args : beta F32[B], action_map, binary_set U8[2^(bits-3)], workspace_in U8[ws], then the initial state leaves (env.init), then the 24
+//        parameter buffers
+// rets : the final state leaves, returns F32[B] (sum of rewards per episode), workspace U8[eaz_evaluate_workspace_bytes + 256]
+// The loop's CUDA graph is kept with the workspace address: alias workspace_in -> workspace and the state leaves to keep it across calls.
+ffi::Error EvaluateImpl(cudaStream_t stream, ffi::Buffer<ffi::F32> beta, ffi::AnyBuffer action_map, ffi::Buffer<ffi::U8> binary_set,
+                        ffi::Buffer<ffi::U8> workspace_in, ffi::RemainingArgs rest, ffi::RemainingRets rets, int32_t env_kind, int32_t size,
+                        int32_t word_size, int32_t binary_encoding, int32_t reward_fn, int32_t num_simulations, int32_t max_depth,
+                        int32_t max_num_considered_actions, float discount, float value_scale, float maxvisit_init, int32_t rescale_values,
+                        int32_t flags, int32_t mlp_mode, int32_t hash_bits, int32_t hash_io, float max_u, float novelty_scale,
+                        int32_t max_episode_length) {
+  (void)workspace_in;  // (only its aliasing matters: the result `workspace` is the buffer the library uses)
+  const int64_t B = beta.element_count();
+  const eaz_env env = MakeEnv(env_kind, size, word_size, binary_encoding, reward_fn, action_map.untyped_data());
+  if (eaz_env_num_actions(&env) <= 0) return EazError(EAZ_ERR_INVALID_ARG, "EazEvaluate (env)");
+  const size_t nl = NumLeaves(env);
+  if (rest.size() != nl + 24) return Bad("EazEvaluate: expected the state leaves and 24 parameter buffers");
+  if (rets.size() != nl + 2) return Bad("EazEvaluate: expected the state leaves, returns and workspace as results");
+  size_t i = 0, j = 0;
+  eaz_state src, st;
+  EAZ_FFI_TRY(ReadStateArgs(rest, &i, env, B, &src));
+  eaz_fc_params net;
+  EAZ_FFI_TRY(ReadNet(rest, &i, env, binary_set.untyped_data(), hash_bits, hash_io, max_u, novelty_scale, &net));
+  EAZ_FFI_TRY(ReadStateRets(rets, &j, env, B, &st));
+  float* returns = nullptr;
+  EAZ_FFI_TRY(GetRet(rets, j++, "returns", &returns, B));
+  auto workspace = rets.get<ffi::AnyBuffer>(j);
+  if (!workspace.has_value()) return workspace.error();
+
+  eaz_search_config cfg{};
+  cfg.batch = (int32_t)B;
+  cfg.num_simulations = num_simulations;
+  cfg.max_depth = max_depth;
+  cfg.max_num_considered_actions = max_num_considered_actions;
+  cfg.gumbel_scale = 0.0f;  // evaluate.py:44
+  cfg.discount = discount;
+  cfg.exploration = 0;      // the exploitation head (evaluate.py:29-35)
+  cfg.value_scale = value_scale;
+  cfg.maxvisit_init = maxvisit_init;
+  cfg.rescale_values = rescale_values;
+  cfg.use_mixed_value = 1;
+  cfg.epsilon = 1e-8f;
+  cfg.flags = flags & ~EAZ_FLAG_REUSE_PREPARED;
+  cfg.mlp_mode = mlp_mode;
+  cfg.pb_c_init = 1.25f;
+  cfg.pb_c_base = 19652.0f;
+  cfg.temperature = 1.0f;
+
+  const size_t need = eaz_evaluate_workspace_bytes(&cfg, &env);
+  if (need == 0) return EazError(EAZ_ERR_INVALID_ARG, "eaz_evaluate_workspace_bytes");
+  void* ws = AlignUp((*workspace)->untyped_data(), 256);
+  const size_t pad = (size_t)((uint8_t*)ws - (uint8_t*)(*workspace)->untyped_data());
+  if ((*workspace)->size_bytes() < pad + need) return Bad("workspace result must hold eaz_evaluate_workspace_bytes + 256 bytes");
+  EAZ_FFI_TRY(CopyState(env, src, st, B, stream));
+
+  eaz_search_inputs in{};
+  in.beta = beta.typed_data();
+  in.env = &env;
+  return EazError(eaz_evaluate(&cfg, &in, &net, &st, returns, max_episode_length, ws, (*workspace)->size_bytes() - pad, stream), "eaz_evaluate");
 }
 
 // ------------------------------------------------------------------------------------------------ env step / init
@@ -590,6 +653,31 @@ XLA_FFI_DEFINE_HANDLER_SYMBOL(EazSearch, SearchImpl,
                                   .Attr<int32_t>("hash_io")
                                   .Attr<float>("max_u")
                                   .Attr<float>("novelty_scale"));
+
+XLA_FFI_DEFINE_HANDLER_SYMBOL(EazEvaluate, EvaluateImpl,
+                              ffi::Ffi::Bind()
+                                  .Ctx<ffi::PlatformStream<cudaStream_t>>()
+                                  .Arg<ffi::Buffer<ffi::F32>>()  // beta
+                                  .Arg<ffi::AnyBuffer>()         // action_map
+                                  .Arg<ffi::Buffer<ffi::U8>>()   // binary_set
+                                  .Arg<ffi::Buffer<ffi::U8>>()   // workspace_in
+                                  .RemainingArgs()               // initial state leaves, 24 parameter buffers
+                                  .RemainingRets()               // final state leaves, returns, workspace
+                                  EAZ_ENV_ATTRS()
+                                  .Attr<int32_t>("num_simulations")
+                                  .Attr<int32_t>("max_depth")
+                                  .Attr<int32_t>("max_num_considered_actions")
+                                  .Attr<float>("discount")
+                                  .Attr<float>("value_scale")
+                                  .Attr<float>("maxvisit_init")
+                                  .Attr<int32_t>("rescale_values")
+                                  .Attr<int32_t>("flags")
+                                  .Attr<int32_t>("mlp_mode")
+                                  .Attr<int32_t>("hash_bits")
+                                  .Attr<int32_t>("hash_io")
+                                  .Attr<float>("max_u")
+                                  .Attr<float>("novelty_scale")
+                                  .Attr<int32_t>("max_episode_length"));
 
 XLA_FFI_DEFINE_HANDLER_SYMBOL(EazEnvStep, EnvStepImpl,
                               ffi::Ffi::Bind()

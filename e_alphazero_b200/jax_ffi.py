@@ -8,6 +8,7 @@ tests through tests/xla_ffi_stub/.
 
 Call shapes mirror the reference (file:line under /root/reference/src):
     epistemic_gumbel_muzero_policy(...)  selfplay.py:107-117, reanalyze.py:77-85, evaluate.py:36-45  (+ epistemic_summary())
+    evaluate(...)                        evaluate.py:13-57 (the whole episode loop: one custom call)
     env_step(...) / env_init(...)        selfplay.py:26-75,135,161,166
     forward_states(...)                  selfplay.py:89, reanalyze.py:67,90
     reanalyze_targets(...)               reanalyze.py:86-129
@@ -33,7 +34,7 @@ _eaz = ctypes.CDLL(os.path.join(_HERE, "libeaz_b200.so"), mode=ctypes.RTLD_GLOBA
 _shim = ctypes.CDLL(os.path.join(_HERE, "libeaz_xla_ffi.so"))
 for _name, _sym in (("eaz_search", "EazSearch"), ("eaz_env_step", "EazEnvStep"), ("eaz_env_init", "EazEnvInit"),
                     ("eaz_mlp_forward_states", "EazMlpForwardStates"), ("eaz_reanalyze_targets", "EazReanalyzeTargets"),
-                    ("eaz_hash_update", "EazHashUpdate"),
+                    ("eaz_hash_update", "EazHashUpdate"), ("eaz_evaluate", "EazEvaluate"),
                     ("eaz_replay_init", "EazReplayInit"), ("eaz_replay_add", "EazReplayAdd"), ("eaz_replay_sample", "EazReplaySample"),
                     ("eaz_replay_set_priorities", "EazReplaySetPriorities"), ("eaz_replay_status", "EazReplayStatus")):
     jax.ffi.register_ffi_target(_name, jax.ffi.pycapsule(getattr(_shim, _sym)), platform="CUDA")
@@ -150,6 +151,37 @@ def epistemic_gumbel_muzero_policy(params, rng_key, root, env: EnvSpec, model_st
         fused_root=i32(0), draw_gumbel=i32(0), noise_seed=i32(0), reuse_prepared=i32(bool(reuse_prepared) and workspace is not None),
         hash_bits=i32(hash_bits), hash_io=i32(env.kind == ENV_SUBLEQ if hash_io is None else hash_io), max_u=f32(1.0), novelty_scale=f32(1.0))
     return PolicyOutput(action, weights, SearchTreeView(EpistemicSearchSummary(value, std, counts, probs, q, qvar), ws))
+
+
+def evaluate(params, model_state, env: EnvSpec, states, *, num_simulations, discount, max_episode_length, exploitation_beta=0.0,
+             rescale_values=True, mlp_mode=1, hash_io=None, hash_bits=24):
+    """evaluate.py:13-57 from `states` = env.init(...) (evaluate.py:52-54; Subleq tasks drawn by the caller): greedy episodes
+    (gumbel_scale = 0) until every env has terminated or max_episode_length moves have passed.  The loop runs on the device as one CUDA
+    graph whose while condition the device decides.  Returns (mean sum of rewards, sums of rewards [B], final states)."""
+    B = states.terminated.shape[0]
+    leaves = state_leaves(env, states)
+    from . import _abi  # ctypes mirrors of the POD structs (no torch)
+
+    cfg = _abi.default_search_config(batch=B, num_simulations=num_simulations, gumbel_scale=0.0, mlp_mode=mlp_mode)
+    e = _abi.EazEnv(env.kind, env.size, None, env.word_size, env.binary_encoding, env.reward_fn)
+    _eaz.eaz_evaluate_workspace_bytes.restype = ctypes.c_size_t
+    ws_bytes = int(_eaz.eaz_evaluate_workspace_bytes(ctypes.byref(cfg), ctypes.byref(e)))
+    if ws_bytes == 0:
+        raise ValueError(_eaz_error())
+    ws_bytes += 256
+    out_types = [jax.ShapeDtypeStruct(x.shape, x.dtype) for x in leaves] + [jax.ShapeDtypeStruct((B,), jnp.float32),
+                                                                           jax.ShapeDtypeStruct((ws_bytes,), jnp.uint8)]
+    beta = jnp.full((B,), exploitation_beta, jnp.float32)  # evaluate.py:34
+    n = len(leaves)
+    aliases = {3: n + 1} | {4 + k: k for k in range(n)}  # workspace_in -> workspace, leaves stepped in place
+    out = jax.ffi.ffi_call("eaz_evaluate", out_types, input_output_aliases=aliases)(
+        beta, env.amap(), model_state["fc_az_net/xxhash32"]["binary_set"], jnp.zeros((ws_bytes,), jnp.uint8), *leaves, *param_leaves(params),
+        **env.attrs(), num_simulations=i32(num_simulations), max_depth=i32(0), max_num_considered_actions=i32(16), discount=f32(discount),
+        value_scale=f32(0.1), maxvisit_init=f32(50.0), rescale_values=i32(rescale_values), flags=i32(DEFAULT_FLAGS), mlp_mode=i32(mlp_mode),
+        hash_bits=i32(hash_bits), hash_io=i32(env.kind == ENV_SUBLEQ if hash_io is None else hash_io), max_u=f32(1.0), novelty_scale=f32(1.0),
+        max_episode_length=i32(max_episode_length))
+    returns = out[n]
+    return returns.mean(), returns, with_leaves(env, states, out[:n])
 
 
 def env_step(env: EnvSpec, states, action, *, auto_reset=False, task_ids=None):

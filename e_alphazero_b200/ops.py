@@ -170,8 +170,13 @@ def _tasks(task_ids, B, device):
 
 def env_init(env: EnvSpec, B: int, task_ids=None, with_obs=False, device="cuda") -> dict:
     """vmap(env.init): deep_sea.py:54-57 / subleq.py:623-646 (task ids pre-drawn)."""
-    st = alloc_state(env, B, with_obs, device)
-    t = _tasks(task_ids, B, device)
+    return env_init_(env, alloc_state(env, B, with_obs, device), task_ids)
+
+
+def env_init_(env: EnvSpec, st: dict, task_ids=None) -> dict:
+    """env_init into the existing state buffers `st`."""
+    B = _batch(st)
+    t = _tasks(task_ids, B, st["step_count"].device)
     e, s = env.struct(), state_struct(env, st)
     check(load().eaz_env_init(C.byref(e), _ptr(t), C.byref(s), B, _stream()), "eaz_env_init")
     return st
@@ -620,6 +625,36 @@ class SearchPlan:
             return self.out, {k: (float(ms[i]), int(cnt[i])) for i, k in enumerate(self.PROFILE_CLASSES)}
         check(load().eaz_search_gumbel(C.byref(cfg), C.byref(inp), C.byref(o), self._ws_ptr, self._ws_bytes, _stream()), "eaz_search_gumbel")
         return self.out
+
+
+class EvaluatePlan:
+    """Workspace of eaz_evaluate for one (cfg, env) shape.  The library keeps the loop's CUDA graph with the workspace, so repeated
+    run() calls on the same buffers launch the graph built by the first one."""
+
+    def __init__(self, cfg: _abi.EazSearchConfig, env: EnvSpec, net: FcParams, device="cuda"):
+        torch = require_cuda()
+        self.cfg, self.env, self.net = cfg, env, net
+        nbytes = load().eaz_evaluate_workspace_bytes(C.byref(cfg), C.byref(env.struct()))
+        if nbytes == 0:
+            raise EazError("eaz_evaluate_workspace_bytes rejected the configuration: " + load().eaz_last_error().decode())
+        self.workspace = torch.empty(nbytes + 256, dtype=torch.uint8, device=device)
+        off = (-self.workspace.data_ptr()) % 256
+        self._ws_ptr = C.c_void_p(self.workspace.data_ptr() + off)
+        self._ws_bytes = C.c_size_t(nbytes)
+        self.counters = self.workspace[off : off + C.sizeof(_abi.EazEvaluateCounters)].view(torch.int32)  # moves, live, ticket, cont
+
+    def run(self, beta, states: dict, returns, max_episode_length: int, invalid_actions=None):
+        """eaz_evaluate: the episodes from `states` (stepped in place) with the sums of rewards in `returns` [B]."""
+        import torch
+
+        e, n, s = self.env.struct(), self.net.struct(), state_struct(self.env, states)
+        inp = _abi.EazSearchInputs(None, None, None, _ptr(beta, torch.float32), None, _ptr(invalid_actions, torch.uint8), None, C.pointer(e), None, None)
+        check(load().eaz_evaluate(C.byref(self.cfg), C.byref(inp), C.byref(n), C.byref(s), _ptr(returns, torch.float32), int(max_episode_length),
+                                  self._ws_ptr, self._ws_bytes, _stream()), "eaz_evaluate")
+
+    def moves(self) -> int:
+        """Moves the last run() made (reads the device counter: synchronises)."""
+        return int(self.counters[0].item())
 
 
 def reanalyze_targets(discount, exploration_beta, exploration_ube_target, temperature, action, qvalues, qvalues_epistemic_variance, visit_counts,

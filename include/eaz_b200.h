@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define EAZ_ABI_VERSION 5
+#define EAZ_ABI_VERSION 6
 
 enum {
   EAZ_OK = 0,
@@ -347,6 +347,38 @@ int eaz_search_numeric_status(const eaz_search_config* cfg, const eaz_env* env, 
 /* Number of kernel launches one eaz_search_gumbel call enqueues (for bench.py's
  * gpu_launches accounting). */
 int32_t eaz_search_num_launches(const eaz_search_config* cfg, const eaz_env* env);
+
+/* ------------------------------------------------------------------------ */
+/* ABI 6 (appended): the evaluation loop of evaluate.py:13-57 as one device    */
+/* program -- a CUDA graph whose WHILE conditional node repeats {fused-root    */
+/* search, env step, returns += rewards[:,0]} and whose condition the device   */
+/* computes: continue while any env is not terminated and moves <=             */
+/* max_episode_length (cond_fn, evaluate.py:18-20).                            */
+
+/* The loop's device words, at the start of the evaluate workspace.  After an eaz_evaluate call has finished: moves = the number of
+ * moves it ran, cont = 0, live = ticket = 0. */
+typedef struct eaz_evaluate_counters {
+  int32_t moves;   /* moves run so far in this call */
+  int32_t live;    /* envs not terminated after the current move (summed over the CTAs of the step kernel) */
+  uint32_t ticket; /* CTAs of the step kernel done with the current move */
+  int32_t cont;    /* the loop condition after the last move */
+} eaz_evaluate_counters;
+
+/* Workspace of eaz_evaluate (256-byte aligned): the counters, zero Gumbel noise [B,A], the played actions [B] and the search workspace of
+ * `cfg`.  0 if cfg / env are rejected. */
+size_t eaz_evaluate_workspace_bytes(const eaz_search_config* cfg, const eaz_env* env);
+
+/* Greedy evaluation episodes (evaluate.py:13-57) from `states` (the output of eaz_env_init: no env terminated, so the first move always
+ * runs, as in the reference): while any env is not terminated and moves <= max_episode_length, the fused-root search of `cfg` with
+ * zero Gumbel noise picks an action per env (cfg->gumbel_scale must be 0 and cfg->action_sampling EAZ_ACTION_SEARCH), pgx.Env.step
+ * advances `states` in place (no auto-reset: terminated envs are absorbing) and returns[b] += rewards[b,0], starting from 0.
+ * From `in` it reads env, beta [B] and invalid_actions (may be NULL); prior_logits / value / value_epistemic_variance must be NULL
+ * (fused root); the other fields are not read.  A negative max_episode_length runs no move (returns = 0).
+ * The parameter-derived tables are rebuilt once per call, before the loop.  The loop is a CUDA graph built on the first call for a
+ * workspace and kept with it; a call with another cfg / env / net / buffer address rebuilds it.  Asynchronous on `stream`: no
+ * allocation of device memory, no host synchronisation after the graph of the workspace is built. */
+int eaz_evaluate(const eaz_search_config* cfg, const eaz_search_inputs* in, const eaz_fc_params* net, eaz_state* states, float* returns,
+                 int32_t max_episode_length, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------ */
 /* Convolutional evaluators (SURVEY 8f-4): EpistemicResidualAZNet               */
