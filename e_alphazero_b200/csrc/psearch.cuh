@@ -18,13 +18,15 @@
 // search, the cached selection and the compact env state of EVERY node in shared memory (the pointer-chase descent never leaves the
 // SM), plus a staging area with the node / edge records of the current path.  Per simulation a tree warp runs: expand (with the leaf's
 // table entry) + backward + action refresh (tree_step.cuh: staged2_*, the staged step of tree_step2_kernel) -> descent over the cached
-// selections -> DeepSea transition -> load of the new leaf's table entry -> stage the new path's records.  Trees that cannot be staged
-// (path longer than kNodes - 1, re-expanded leaf under a max_depth cut-off) take tree_step_direct for that simulation and
-// re-synchronise their shared-memory caches.
+// selections -> cp.async copies of the new path's records into the staging area -> DeepSea transition -> load of the new leaf's table
+// entry -> wait for the copies and finish the staging.  Trees that cannot be staged (path longer than kNodes - 1, re-expanded leaf
+// under a max_depth cut-off) take tree_step_direct for that simulation and re-synchronise their shared-memory caches.
 //
 // The tree itself (node / edge records, states) still lives in the caller's workspace in HBM/L2 -- it is the search's OUTPUT
-// (finalize / export read it) and the source of the staging loads -- but the per-simulation critical path touches it only with
-// fire-and-forget stores and the staging loads.
+// (finalize / export read it) and the source of the staging copies -- but the per-simulation critical path touches it only with
+// fire-and-forget stores and one round trip of staging copies.  Measured at C2 (B200, 1000 W): 6.0 us mean period per simulation and
+// warp -- refresh 2.44, descent incl. the copy issue and transition 1.67, backward 1.03, staging 0.63, expand 0.25 us
+// (profiles/r5_trace_psearch_c2.txt).
 #pragma once
 #include "umma.cuh"
 
@@ -301,6 +303,12 @@ __device__ __forceinline__ uint32_t lds_u16(uint32_t addr) {
   return v;
 }
 __device__ __forceinline__ void sts_u32(uint32_t addr, uint32_t v) { asm volatile("st.shared.u32 [%0], %1;" ::"r"(addr), "r"(v) : "memory"); }
+// 4-byte global -> shared copy that holds no register until it lands (LDGSTS).  4-byte copies take only the .ca cache operator: the
+// read goes through the SM's L1 and L2.
+__device__ __forceinline__ void cp_async4(uint32_t dst, const void* src) {
+  asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(dst), "l"(src) : "memory");
+}
+__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
 
 // Optional timeline of CTA 0 (eaz_debug_set_ps_trace): per simulation `it` and tree warp w, at [(it * kTWarps + w) * 8 + k], globaltimer
 // stamps of k = 0 expand done (the leaf's table entry has been used), 1 backward done, 2 refresh done, 3 descent done (the next leaf's
@@ -398,46 +406,79 @@ __global__ void __launch_bounds__(kThreads, 1) ds_search_kernel(const __grid_con
     }
     __syncwarp();
   };
-  // ---- stage the records the step for simulation `sim_next` will need (tree_step2_kernel's pre-wait staging)
-  auto stage = [&](int sim_next) {
-    bool ok = true;
-    if (in_batch) ok = L + 1 <= kNodes && reinterpret_cast<const uint4*>(t.nodes + ((unsigned)leaf * uB + ub))[0].x == 0u;  // fits, fresh leaf
-    staged = __all_sync(0xffffffffu, ok) && !(sp.flags & EAZ_FLAG_PUCT);
-    if (!staged) return;
-    if (in_batch) {  // backward operands: this lane owns levels hl and hl + 16
+  // ---- the staging loads of the step for simulation `sim_next`, as cp.async copies straight into the staging slots (no register
+  // holds them while they are in flight).  A tree issues all of them at once as soon as its new path is known -- after the descent,
+  // ahead of the DeepSea transition and the table load -- and stage() waits for them: one L2 round trip.  (Issued level by level
+  // inside the descent instead, their issue cost lengthened the chase by more than it took off the wait; measured at C2 on a B200:
+  // descent 1.20 -> 2.21 us, staging 1.31 -> 0.60 us per simulation.)
+  // Ordering: the records they read were last written in this simulation's expand, backward and refresh (or its DIRECT step) by
+  // lanes of this warp, each phase ending in __syncwarp, which orders those stores before any memory operation the warp's lanes issue
+  // after it.  A non-bulk cp.async is a weak read of the generic proxy by the issuing thread, so it sees those stores exactly as the
+  // plain loads it replaces did.  The slots it fills were last read by this simulation's backward / refresh, before the same
+  // __syncwarp.
+  //
+  // A tree can be staged when its path fits and its leaf is fresh.  The leaf is fresh exactly when the descent ended on an
+  // unexpanded child, which gets the next unused index sim_next (search.py); a descent cut off by max_depth ends on an expanded node
+  // (index < sim_next), which takes the DIRECT step.
+  auto stageable = [&](int sim_next) { return L + 1 <= kNodes && leaf == sim_next && !(sp.flags & EAZ_FLAG_PUCT); };
+  auto issue_staging = [&](int sim_next) {
+    if (!in_batch || !stageable(sim_next)) return;
+    if (hl == 0) cp_async4(smem_u32(s_misc), t.table + (s_misc[1] * sp.n + min(sim_next, sp.n - 1)));  // seq-halving target -> s_misc[0]
+    // backward operands of levels hl and hl + 16: visits, value, variance -> s_back[32 / 64 / 96 + lev]
 #pragma unroll
-      for (int k = 0; k < 2; ++k) {
-        const int lev = hl + kStaged2Lanes * k;
-        if (lev < L) {
-          const uint4 nrec = reinterpret_cast<const uint4*>(t.nodes + ((s_back[lev] & 0xffffu) * uB + ub))[0];
-          s_back[1 * 32 + lev] = nrec.x;
-          s_back[2 * 32 + lev] = nrec.y;
-          s_back[3 * 32 + lev] = nrec.z;
-        }
+    for (int k = 0; k < 2; ++k) {
+      const int lev = hl + kStaged2Lanes * k;
+      if (lev >= L) break;
+      const uint32_t* nrec = reinterpret_cast<const uint32_t*>(t.nodes + ((s_back[lev] & 0xffffu) * uB + ub));
+      const uint32_t d = smem_u32(s_back + 32 + lev);
+      cp_async4(d, nrec + 0);
+      cp_async4(d + 4u * 32, nrec + 1);
+      cp_async4(d + 4u * 64, nrec + 2);
+    }
+    // words 0..8 of staged2_store_lane's record of (path level r * kPR + glev, action gl) in round r
+    if (gl < t.A) {
+#pragma unroll
+      for (int r = 0; r < kRounds; ++r) {
+        const int lev = r * kPR + glev;
+        if (lev >= L) break;
+        const unsigned slot_g = (s_back[lev] & 0xffffu) * uB + ub;
+        const uint32_t* erec = reinterpret_cast<const uint32_t*>(t.edges + (size_t)(slot_g * uA + (unsigned)gl));
+        const uint32_t* nrec = reinterpret_cast<const uint32_t*>(t.nodes + slot_g);
+        const uint32_t d = smem_u32(s_edge + r * kStaged2LaneWords * kStaged2Lanes + hl);
+#pragma unroll
+        for (int k = 0; k < 7; ++k) cp_async4(d + 4u * kStaged2Lanes * k, erec + k);  // ci1, vis, pl, rew, val, vvar, dis
+        cp_async4(d + 4u * kStaged2Lanes * 7, nrec + 4);                            // raw value, raw variance (node half 1)
+        cp_async4(d + 4u * kStaged2Lanes * 8, nrec + 5);
       }
     }
+  };
+  // ---- stage the records the step for simulation `sim_next` will need (tree_step2_kernel's pre-wait staging).  issued: the copies
+  // are in flight (after a descent); otherwise the path comes from a DIRECT step and resync, and they are issued here.
+  auto stage = [&](int sim_next, bool issued) {
+    if (!issued) issue_staging(sim_next);
+    staged = __all_sync(0xffffffffu, !in_batch || stageable(sim_next));
+    cp_async_wait_all();
+    __syncwarp();
+    if (!staged) return;
     const int Lw = max(L, __shfl_xor_sync(0xffffffffu, L, kStaged2Lanes));
 #pragma unroll
     for (int r = 0; r < kRounds; ++r) {
       if (r * kPR <= Lw) {  // warp-uniform
         const int lev = r * kPR + glev;
         const bool on = in_batch && lev <= L && gl < t.A;
-        uint4 h0 = make_uint4(0u, 0u, 0u, 0u), h1 = h0, n1 = h0;
-        if (on && lev < L) {  // (the fresh leaf's records are all zero: nothing to load)
-          const unsigned slot_g = (s_back[lev] & 0xffffu) * uB + ub;
-          const uint4* p = reinterpret_cast<const uint4*>(t.edges + (size_t)(slot_g * uA + (unsigned)gl));
-          h0 = p[0];
-          h1 = p[1];
-          n1 = reinterpret_cast<const uint4*>(t.nodes + slot_g)[1];
-        }
-        const float xl[1] = {__uint_as_float(h0.z)};
+        uint32_t* const se = s_edge + r * kStaged2LaneWords * kStaged2Lanes + hl;
+        const float xl[1] = {on && lev < L ? __uint_as_float(se[2 * kStaged2Lanes]) : 0.0f};
         float pr[1];
         group_softmax<kG, 1>(xl, valid1, pr);  // p = max(tiny, softmax(prior logits)) of _compute_mixed_value
-        if (on) staged2_store_lane(s_edge, r, hl, h0, h1, n1, pr[0]);
+        if (on) {
+          if (lev == L) {  // the fresh leaf's records are all zero
+#pragma unroll
+            for (int k = 0; k < 9; ++k) se[kStaged2Lanes * k] = 0u;
+          }
+          se[kStaged2Lanes * 9] = __float_as_uint(eaz_max(EAZ_F32_TINY, pr[0]));
+        }
       }
     }
-    // the root's seq-halving visit target for the refresh of step `sim_next` (s_root[0..1] hold gumbel + logit, [2..3] the invalid flags)
-    if (in_batch && hl == 0) s_misc[0] = (uint32_t)t.table[s_misc[1] * sp.n + min(sim_next, sp.n - 1)];
     __syncwarp();
   };
 
@@ -457,7 +498,7 @@ __global__ void __launch_bounds__(kThreads, 1) ds_search_kernel(const __grid_con
     }
   }
   __syncwarp();
-  stage(1);
+  stage(1, false);
 
 #pragma unroll 1
   for (int it = 0; it < n; ++it) {
@@ -478,7 +519,7 @@ __global__ void __launch_bounds__(kThreads, 1) ds_search_kernel(const __grid_con
       direct_pair(a, sim, 1, do_select ? 1 : 0, b0, lane);
       if (do_select) {
         resync(sim);
-        stage(sim + 1);
+        stage(sim + 1, false);
       }
       continue;
     }
@@ -519,23 +560,26 @@ __global__ void __launch_bounds__(kThreads, 1) ds_search_kernel(const __grid_con
           else node = child;
         }
       }
+      __syncwarp();  // (lane 0's s_back words of the path -> the lanes that issue the staging copies)
       if (in_batch) {
-        const int new_leaf = child < 0 ? sim + 1 : child;  // search.py: node first expanded on simulation i gets index i+1
+        L = depth;
+        leaf = child < 0 ? sim + 1 : child;  // search.py: node first expanded on simulation i gets index i+1
+      }
+      issue_staging(sim + 1);
+      if (in_batch) {
         float rw;
         const uint32_t ns = deepsea_step(s_state[node], action, a.env.size, amap_n ? s_amap : a.env.action_map, &rw);  // context.py:127 env.step fused here
-        net = __ldg(a.ds_out + deepsea_obs_index(ns, a.env.size));  // the new leaf's network outputs: in flight under the staging loads
-        L = depth;
-        leaf = new_leaf;
+        net = __ldg(a.ds_out + deepsea_obs_index(ns, a.env.size));  // the new leaf's network outputs: in flight with the staging copies
         reward = rw;
         term = EAZ_DS_TERM(ns) != 0;
         if (hl == 0) {
           t.path_len[b] = depth;
           t.parent[b] = node;
           t.action[b] = action;
-          t.leaf[b] = new_leaf;
+          t.leaf[b] = leaf;
           t.reward[b] = rw;
-          st_global[(unsigned)new_leaf * uB + ub] = ns;
-          if (new_leaf < ncap) s_state[new_leaf] = ns;
+          st_global[(unsigned)leaf * uB + ub] = ns;
+          if (leaf < ncap) s_state[leaf] = ns;
         }
       }
       __syncwarp();
@@ -547,7 +591,7 @@ __global__ void __launch_bounds__(kThreads, 1) ds_search_kernel(const __grid_con
         trc.path(it, tw, Lmax, 0);
       }
     }
-    stage(sim + 1);
+    stage(sim + 1, true);
     if (lane == 0) trc.stamp(it, tw, 4);
   }
 }
