@@ -8,7 +8,7 @@ from __future__ import annotations
 
 import ctypes as C
 
-ABI_VERSION = 6
+ABI_VERSION = 7
 
 EAZ_OK = 0
 EAZ_ERR_INVALID_ARG = -1
@@ -310,6 +310,11 @@ class EazSearchOutputs(C.Structure):
 
 class EazEvaluateCounters(C.Structure):  # the evaluation loop's device words at the start of the eaz_evaluate workspace
     _fields_ = [("moves", C.c_int32), ("live", C.c_int32), ("ticket", C.c_uint32), ("cont", C.c_int32)]
+
+
+class EazSelfplayOutputs(C.Structure):  # the stacked per-step outputs of eaz_selfplay: [T,B], [T,B,A], [T,B,4], [T,B,S]
+    _fields_ = [(name, _p) for name in ("action", "root_value", "root_epistemic_std", "value_prediction", "ube_prediction",
+                                        "q_values_epistemic_variance", "trajectory", "states", "rewards")]
 
 
 def default_search_config(**kw) -> EazSearchConfig:

@@ -30,6 +30,7 @@ EXPORTS = [
     "eaz_priority_tree_bytes", "eaz_priority_init", "eaz_priority_add_step", "eaz_priority_set", "eaz_priority_sample", "eaz_priority_status",
     "eaz_replay_add", "eaz_priority_sample_keyed", "eaz_priority_status_async",
     "eaz_evaluate_workspace_bytes", "eaz_evaluate",
+    "eaz_selfplay_workspace_bytes", "eaz_selfplay",
 ]
 
 
@@ -61,6 +62,7 @@ def load():
     lib.eaz_convnet_workspace_bytes.restype = C.c_size_t
     lib.eaz_priority_tree_bytes.restype = C.c_size_t
     lib.eaz_evaluate_workspace_bytes.restype = C.c_size_t
+    lib.eaz_selfplay_workspace_bytes.restype = C.c_size_t
     if lib.eaz_abi_version() != _abi.ABI_VERSION:
         raise EazError(f"ABI version mismatch: library {lib.eaz_abi_version()} vs bindings {_abi.ABI_VERSION}")
     _lib = lib

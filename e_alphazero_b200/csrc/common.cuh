@@ -88,7 +88,7 @@ static inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 b
   return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
 }
 
-// Internal eaz_search_config.flags bit (set by eaz_evaluate, never by a caller): enqueue only the search's preparation -- the tree
+// Internal eaz_search_config.flags bit (set by eaz_evaluate / eaz_selfplay, never by a caller): enqueue only the search's preparation -- the tree
 // memset, the root states and, unless EAZ_FLAG_REUSE_PREPARED, the parameter-derived tables -- and no simulation.
 constexpr int kFlagPrepareOnly = 1 << 28;
 
@@ -172,6 +172,22 @@ __device__ __forceinline__ void pack_state(const EnvDesc& env, const StateSoA& s
   o[35] = (uint8_t)((term ? EAZ_SQ_FLAG_TERM : 0) | (trunc ? EAZ_SQ_FLAG_TRUNC : 0) | (s.solved[b] ? EAZ_SQ_FLAG_SOLVED : 0));
   o[36] = o[37] = o[38] = o[39] = 0;
   for (int i = 0; i < S - EAZ_SQ_HDR; ++i) o[EAZ_SQ_HDR + i] = i < ws ? (uint8_t)s.memory[(size_t)b * ws + i] : 0;
+}
+
+// One 16-byte trajectory record of env b for the replay buffer's wire format (SURVEY 8f-3, main.py:383-385; eaz_trajectory_pack and
+// the stacked outputs of eaz_selfplay): the played action, the reward bits, terminated | truncated << 8 | solved << 16, and the first
+// word of the compact state (DeepSea: the whole state; Subleq: step count | task << 16 -- the memory image travels separately when the
+// caller stores full states).
+__device__ __forceinline__ int4 pack_trajectory(const EnvDesc& env, const StateSoA& s, const int32_t* __restrict__ action, int b) {
+  const int term = s.terminated[b] != 0, trunc = s.truncated ? (s.truncated[b] != 0) : 0;
+  int flags = term | (trunc << 8), word;
+  if (env.kind == EAZ_ENV_DEEPSEA) {
+    word = (int)ds_pack(s.step_count[b], s.col[b], term, trunc);
+  } else {
+    flags |= (s.solved[b] != 0) << 16;
+    word = (s.step_count[b] & 0xffff) | (s.task[b] << 16);
+  }
+  return make_int4(action[b], __float_as_int(s.rewards[b]), flags, word);
 }
 
 // pgx.Env.step around DeepSea._step (deep_sea.py:59-81).  Returns the new

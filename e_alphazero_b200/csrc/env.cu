@@ -128,21 +128,11 @@ __global__ void subleq_observe_kernel(EnvDesc env, StateSoA s, uint8_t* __restri
 using namespace eaz;
 
 namespace eaz {
-// One 16-byte trajectory record per env for the replay buffer's wire format (SURVEY 8f-3, main.py:383-385): the chosen action, the
-// reward bits, terminated | truncated << 8 | solved << 16, and the first word of the compact state (DeepSea: the whole state;
-// Subleq: step count | task << 16 -- the memory image travels separately when the caller stores full states).
+// one pack_trajectory record per env
 __global__ void trajectory_pack_kernel(EnvDesc env, StateSoA s, const int32_t* __restrict__ action, int4* __restrict__ out, int B) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
-  const int term = s.terminated[b] != 0, trunc = s.truncated ? (s.truncated[b] != 0) : 0;
-  int flags = term | (trunc << 8), word;
-  if (env.kind == EAZ_ENV_DEEPSEA) {
-    word = (int)ds_pack(s.step_count[b], s.col[b], term, trunc);
-  } else {
-    flags |= (s.solved[b] != 0) << 16;
-    word = (s.step_count[b] & 0xffff) | (s.task[b] << 16);
-  }
-  out[b] = make_int4(action[b], __float_as_int(s.rewards[b]), flags, word);
+  out[b] = pack_trajectory(env, s, action, b);
 }
 }  // namespace eaz
 

@@ -7,10 +7,8 @@
 // condition with cudaGraphSetConditional.  The host launches the graph once per evaluation and never waits inside it.
 //
 // Workspace: [eaz_evaluate_counters | 256 B][zero Gumbel noise B*A f32][played actions B i32][search workspace], each 256-byte aligned.
+#include "loop_graph.cuh"
 #include "mlp.cuh"
-
-#include <cstring>
-#include <mutex>
 
 namespace eaz {
 
@@ -90,12 +88,8 @@ static int launch_eval_step(const EnvDesc& env, const eaz_state* states, const i
   return 0;
 }
 
-// ---- the loop's graph, one per workspace (like the auxiliary streams of EAZ_FLAG_STREAMS), rebuilt when anything it bakes in changes
-struct EvalGraph {
-  bool used = false;
-  int device = -1;
-  const void* workspace = nullptr;
-  // what the captured launches hold by value
+// what the loop's graph bakes in (the captured launches hold these by value)
+struct EvalRec {
   eaz_search_config cfg;
   eaz_env env;
   eaz_fc_params net;
@@ -105,80 +99,12 @@ struct EvalGraph {
   float* returns;
   int32_t max_episode_length;
   size_t bytes;
-  cudaStream_t capture = nullptr;
-  cudaGraph_t graph = nullptr;
-  cudaGraphExec_t exec = nullptr;
+  bool same(const EvalRec& o) const {
+    return !memcmp(&cfg, &o.cfg, sizeof(cfg)) && same_env(env, o.env) && same_net(net, o.net) && !memcmp(&states, &o.states, sizeof(eaz_state)) &&
+           beta == o.beta && invalid == o.invalid && returns == o.returns && max_episode_length == o.max_episode_length && bytes == o.bytes;
+  }
 };
-
-static bool same_env(const eaz_env& a, const eaz_env& b) {
-  return a.kind == b.kind && a.size == b.size && a.action_map == b.action_map && a.word_size == b.word_size &&
-         a.binary_encoding == b.binary_encoding && a.reward_fn == b.reward_fn;
-}
-static bool same_net(const eaz_fc_params& a, const eaz_fc_params& b) {
-  return a.in_dim == b.in_dim && a.hidden == b.hidden && a.num_actions == b.num_actions && !memcmp(a.w, b.w, sizeof(a.w)) &&
-         !memcmp(a.b, b.b, sizeof(a.b)) && a.binary_set == b.binary_set && a.hash_bits == b.hash_bits && a.hash_io == b.hash_io &&
-         a.word_size == b.word_size && !memcmp(&a.max_u, &b.max_u, sizeof(float)) && !memcmp(&a.novelty_scale, &b.novelty_scale, sizeof(float));
-}
-
-// Captures the loop body into a WHILE node (default value 1: the reference's loop always runs its first move) and instantiates it.
-static int build_graph(EvalGraph* g, const eaz_search_config* body_cfg, const eaz_search_inputs* in, eaz_search_outputs* out, void* search_ws,
-                       size_t search_bytes, const EnvDesc& env, eaz_state* states, float* returns, eaz_evaluate_counters* ctr, int max_len) {
-  if (!g->capture)
-    if (cudaError_t e = cudaStreamCreateWithFlags(&g->capture, cudaStreamNonBlocking); e != cudaSuccess) return cuda_fail(e, "evaluate capture stream");
-  cudaGraph_t graph = nullptr;
-  if (cudaError_t e = cudaGraphCreate(&graph, 0); e != cudaSuccess) return cuda_fail(e, "evaluate graph");
-  auto fail = [&](cudaError_t e, const char* what) {
-    cudaGraphDestroy(graph);
-    return cuda_fail(e, what);
-  };
-  cudaGraphConditionalHandle handle;
-  if (cudaError_t e = cudaGraphConditionalHandleCreate(&handle, graph, 1, cudaGraphCondAssignDefault); e != cudaSuccess)
-    return fail(e, "evaluate conditional handle");
-  cudaGraphNodeParams p{};
-  p.type = cudaGraphNodeTypeConditional;
-  p.conditional.handle = handle;
-  p.conditional.type = cudaGraphCondTypeWhile;
-  p.conditional.size = 1;
-  cudaGraphNode_t node;
-  if (cudaError_t e = cudaGraphAddNode(&node, graph, nullptr, 0, &p); e != cudaSuccess) return fail(e, "evaluate WHILE node");
-  cudaGraph_t body = p.conditional.phGraph_out[0];
-  if (cudaError_t e = cudaStreamBeginCaptureToGraph(g->capture, body, nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed); e != cudaSuccess)
-    return fail(e, "evaluate body capture");
-  int rc = eaz_search_gumbel(body_cfg, in, out, search_ws, search_bytes, g->capture);
-  if (rc == 0) rc = launch_eval_step(env, states, out->action, returns, ctr, max_len, body_cfg->batch, handle, 1, g->capture);
-  cudaGraph_t captured = nullptr;
-  const cudaError_t ce = cudaStreamEndCapture(g->capture, &captured);  // (always: the stream must leave capture mode)
-  if (rc) {
-    cudaGraphDestroy(graph);
-    return rc;
-  }
-  if (ce != cudaSuccess) return fail(ce, "evaluate body capture");
-  cudaGraphExec_t exec = nullptr;
-  if (cudaError_t e = cudaGraphInstantiate(&exec, graph, 0); e != cudaSuccess) return fail(e, "evaluate graph instantiate");
-  if (g->exec) cudaGraphExecDestroy(g->exec);  // (an in-flight launch of the old one completes first)
-  if (g->graph) cudaGraphDestroy(g->graph);
-  g->graph = graph;
-  g->exec = exec;
-  return 0;
-}
-
-constexpr int kEvalGraphs = 64;
-static EvalGraph g_eval_graphs[kEvalGraphs];
-static std::mutex g_eval_mu;  // held for the whole enqueue of one eaz_evaluate call
-
-static EvalGraph* graph_slot(const void* workspace, int dev) {
-  for (auto& g : g_eval_graphs)
-    if (g.used && g.workspace == workspace && g.device == dev) return &g;
-  for (auto& g : g_eval_graphs)
-    if (!g.used) return &g;
-  // table full: reuse a slot of this device (its graph is rebuilt for this workspace)
-  const size_t h = ((uintptr_t)workspace >> 8) * 0x9E3779B97F4A7C15ull >> 32;
-  for (int k = 0; k < kEvalGraphs; ++k) {
-    EvalGraph* g = &g_eval_graphs[(h + k) % kEvalGraphs];
-    if (g->device == dev) return g;
-  }
-  return nullptr;
-}
+static LoopGraphs<EvalRec> g_eval_graphs;
 
 }  // namespace eaz
 
@@ -235,7 +161,7 @@ int eaz_evaluate(const eaz_search_config* cfg, const eaz_search_inputs* in, cons
   lo.action = reinterpret_cast<int32_t*>(ws + L.action);
   void* search_ws = ws + L.search;
 
-  std::lock_guard<std::mutex> lock(g_eval_mu);
+  std::lock_guard<std::mutex> lock(g_eval_graphs.mu);
   // the first move's table preparation, once, outside the loop (the reference's model is constant over the episodes)
   eaz_search_config prep = *cfg;
   prep.flags = (prep.flags & ~EAZ_FLAG_REUSE_PREPARED) | kFlagPrepareOnly;
@@ -243,38 +169,12 @@ int eaz_evaluate(const eaz_search_config* cfg, const eaz_search_inputs* in, cons
 
   eaz_search_config body = *cfg;
   body.flags |= EAZ_FLAG_REUSE_PREPARED;
-  int dev = 0;
-  if (cudaError_t e = cudaGetDevice(&dev); e != cudaSuccess) return cuda_fail(e, "evaluate device");
-  EvalGraph* g = graph_slot(workspace, dev);
-  if (!g) {
-    set_error("eaz_evaluate: no graph slot for this device");
-    return EAZ_ERR_CUDA;
-  }
-  const bool same = g->used && g->workspace == workspace && g->device == dev && g->exec && !memcmp(&g->cfg, &body, sizeof(body)) &&
-                    same_env(g->env, *in->env) && same_net(g->net, *net) && !memcmp(&g->states, states, sizeof(eaz_state)) &&
-                    g->beta == in->beta && g->invalid == in->invalid_actions && g->returns == returns &&
-                    g->max_episode_length == max_episode_length && g->bytes == workspace_bytes;
-  if (!same) {
-    g->used = true;  // (the slot is this workspace's from now on; a failed build leaves exec NULL and is retried next call)
-    g->workspace = workspace;
-    g->device = dev;
-    if (g->exec) {
-      cudaGraphExecDestroy(g->exec);
-      g->exec = nullptr;
-    }
-    if (int rc = build_graph(g, &body, &li, &lo, search_ws, L.search_bytes, env, states, returns, ctr, max_episode_length)) return rc;
-    g->cfg = body;
-    g->env = *in->env;
-    g->net = *net;
-    g->states = *states;
-    g->beta = in->beta;
-    g->invalid = in->invalid_actions;
-    g->returns = returns;
-    g->max_episode_length = max_episode_length;
-    g->bytes = workspace_bytes;
-  }
-  if (cudaError_t e = cudaGraphLaunch(g->exec, st); e != cudaSuccess) return cuda_fail(e, "evaluate graph launch");
-  return 0;
+  const EvalRec rec{body, *in->env, *net, *states, in->beta, in->invalid_actions, returns, max_episode_length, workspace_bytes};
+  return g_eval_graphs.launch("evaluate", workspace, rec, st, [&](cudaStream_t cap, cudaGraphConditionalHandle handle) {
+    int rc = eaz_search_gumbel(&body, &li, &lo, search_ws, L.search_bytes, cap);
+    if (rc == 0) rc = launch_eval_step(env, states, lo.action, returns, ctr, max_episode_length, B, handle, 1, cap);
+    return rc;
+  });
 }
 
 // Test hook (not in the public header): one eval_step_kernel launch outside a graph -- env step on `action`, returns += rewards[:,0],

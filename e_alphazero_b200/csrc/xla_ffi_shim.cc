@@ -7,6 +7,8 @@
 //                       (DeepSea and Subleq; recurrent_fn of context.py:109-157 fused)    evaluate.py:29-45
 //   eaz_evaluate        the evaluate() episode loop (search + env step + reward sum under  evaluate.py:13-57
 //                       a device-decided while condition)
+//   eaz_selfplay        the selfplay() scan (T steps of search + auto-reset env step, every  selfplay.py:78-149
+//                       output stacked over the steps)
 //   eaz_env_step        pgx Env.step / selfplay.auto_reset                               selfplay.py:26-75,135, evaluate.py:47
 //   eaz_env_init        pgx Env.init (vmapped)                                           selfplay.py:161,166, main.py:205
 //   eaz_mlp_forward_states   forward.apply(params, state, states.observation)            selfplay.py:89, reanalyze.py:67,90
@@ -341,6 +343,99 @@ ffi::Error EvaluateImpl(cudaStream_t stream, ffi::Buffer<ffi::F32> beta, ffi::An
   in.beta = beta.typed_data();
   in.env = &env;
   return EazError(eaz_evaluate(&cfg, &in, &net, &st, returns, max_episode_length, ws, (*workspace)->size_bytes() - pad, stream), "eaz_evaluate");
+}
+
+// ------------------------------------------------------------------------------------------------ self-play scan
+// args : beta F32[B], action_map, binary_set U8[2^(bits-3)], gumbel F32[T,B,A], sample_gumbel F32[T,B,A], task_ids S32[T,B] (each of
+//        the three: any 1-element dummy = not given -- the noise is then drawn in the search, the task ids are required for Subleq),
+//        workspace_in U8[ws] (alias it to `workspace` to keep the graph, and with reuse_prepared the tables, across calls), then the
+//        initial state leaves, then the 24 parameter buffers
+// rets : the final state leaves, action S32[T,B], root_value F32[T,B], root_epistemic_std F32[T,B], value_prediction F32[T,B],
+//        ube_prediction F32[T,B], q_values_epistemic_variance F32[T,B,A], trajectory S32[T,B,4], states U8[T,B,S] (the states after
+//        each step, eaz_env_compact records), rewards F32[T,B], workspace U8[eaz_selfplay_workspace_bytes + 256]
+ffi::Error SelfplayImpl(cudaStream_t stream, ffi::Buffer<ffi::F32> beta, ffi::AnyBuffer action_map, ffi::Buffer<ffi::U8> binary_set,
+                        ffi::Buffer<ffi::F32> gumbel, ffi::Buffer<ffi::F32> sample_gumbel, ffi::Buffer<ffi::S32> task_ids,
+                        ffi::Buffer<ffi::U8> workspace_in, ffi::RemainingArgs rest, ffi::RemainingRets rets, int32_t env_kind, int32_t size,
+                        int32_t word_size, int32_t binary_encoding, int32_t reward_fn, int32_t num_simulations, int32_t max_depth,
+                        int32_t max_num_considered_actions, float gumbel_scale, float discount, int32_t two_players_game, int32_t exploration,
+                        float value_scale, float maxvisit_init, int32_t rescale_values, int32_t flags, int32_t mlp_mode, int32_t hash_bits,
+                        int32_t hash_io, float max_u, float novelty_scale, int32_t steps, int32_t root_prior, int32_t action_sampling,
+                        float temperature, int32_t noise_seed, int32_t reuse_prepared) {
+  const int64_t B = beta.element_count(), T = steps;
+  const eaz_env env = MakeEnv(env_kind, size, word_size, binary_encoding, reward_fn, action_map.untyped_data());
+  const int32_t A = eaz_env_num_actions(&env), S = eaz_env_compact_bytes(&env);
+  if (A <= 0 || S <= 0) return EazError(EAZ_ERR_INVALID_ARG, "EazSelfplay (env)");
+  if (T < 0) return Bad("EazSelfplay: steps must be >= 0");
+  const size_t nl = NumLeaves(env);
+  if (rest.size() != nl + 24) return Bad("EazSelfplay: expected the state leaves and 24 parameter buffers");
+  if (rets.size() != nl + 10) return Bad("EazSelfplay: expected the state leaves, the 9 stacked outputs and workspace as results");
+  const bool noise = (int64_t)gumbel.element_count() == T * B * A, sample = (int64_t)sample_gumbel.element_count() == T * B * A,
+             tasks = (int64_t)task_ids.element_count() == T * B;
+  if (!noise && gumbel.element_count() != 1) return Bad("EazSelfplay: gumbel must be [steps, B, num_actions] or a 1-element dummy");
+  if (!sample && sample_gumbel.element_count() != 1) return Bad("EazSelfplay: sample_gumbel must be [steps, B, num_actions] or a 1-element dummy");
+  if (!tasks && task_ids.element_count() != 1) return Bad("EazSelfplay: task_ids must be [steps, B] or a 1-element dummy");
+  size_t i = 0, j = 0;
+  eaz_state src, st;
+  EAZ_FFI_TRY(ReadStateArgs(rest, &i, env, B, &src));
+  eaz_fc_params net;
+  EAZ_FFI_TRY(ReadNet(rest, &i, env, binary_set.untyped_data(), hash_bits, hash_io, max_u, novelty_scale, &net));
+  EAZ_FFI_TRY(ReadStateRets(rets, &j, env, B, &st));
+  eaz_selfplay_outputs out{};
+  EAZ_FFI_TRY(GetRet(rets, j++, "action", &out.action, T * B));
+  EAZ_FFI_TRY(GetRet(rets, j++, "root_value", &out.root_value, T * B));
+  EAZ_FFI_TRY(GetRet(rets, j++, "root_epistemic_std", &out.root_epistemic_std, T * B));
+  EAZ_FFI_TRY(GetRet(rets, j++, "value_prediction", &out.value_prediction, T * B));
+  EAZ_FFI_TRY(GetRet(rets, j++, "ube_prediction", &out.ube_prediction, T * B));
+  EAZ_FFI_TRY(GetRet(rets, j++, "q_values_epistemic_variance", &out.q_values_epistemic_variance, T * B * A));
+  EAZ_FFI_TRY(GetRet(rets, j++, "trajectory", &out.trajectory, T * B * 4));
+  EAZ_FFI_TRY(GetRet(rets, j++, "states", &out.states, T * B * S));
+  EAZ_FFI_TRY(GetRet(rets, j++, "rewards", &out.rewards, T * B));
+  auto workspace = rets.get<ffi::AnyBuffer>(j);
+  if (!workspace.has_value()) return workspace.error();
+
+  eaz_search_config cfg{};
+  cfg.batch = (int32_t)B;
+  cfg.num_simulations = num_simulations;
+  cfg.max_depth = max_depth;
+  cfg.max_num_considered_actions = max_num_considered_actions;
+  cfg.gumbel_scale = gumbel_scale;
+  cfg.discount = discount;
+  cfg.two_players_game = two_players_game;
+  cfg.exploration = exploration;
+  cfg.value_scale = value_scale;
+  cfg.maxvisit_init = maxvisit_init;
+  cfg.rescale_values = rescale_values;
+  cfg.use_mixed_value = 1;
+  cfg.epsilon = 1e-8f;
+  cfg.flags = flags & ~EAZ_FLAG_REUSE_PREPARED;
+  cfg.mlp_mode = mlp_mode;
+  cfg.pb_c_init = 1.25f;
+  cfg.pb_c_base = 19652.0f;
+  cfg.temperature = temperature;
+  cfg.noise_seed = (uint32_t)noise_seed;
+  cfg.root_prior = root_prior;
+  cfg.action_sampling = action_sampling;
+
+  const size_t need = eaz_selfplay_workspace_bytes(&cfg, &env);
+  if (need == 0) return EazError(EAZ_ERR_INVALID_ARG, "eaz_selfplay_workspace_bytes");
+  void* ws = AlignUp((*workspace)->untyped_data(), 256);
+  const size_t pad = (size_t)((uint8_t*)ws - (uint8_t*)(*workspace)->untyped_data());
+  if ((*workspace)->size_bytes() < pad + need) return Bad("workspace result must hold eaz_selfplay_workspace_bytes + 256 bytes");
+  if (reuse_prepared) {  // only meaningful when XLA aliased workspace_in to the result (the tables of the previous call are in it)
+    if (workspace_in.untyped_data() != (*workspace)->untyped_data())
+      return Bad("reuse_prepared needs input_output_aliases={workspace_in: workspace}: the tables live in the workspace");
+    cfg.flags |= EAZ_FLAG_REUSE_PREPARED;
+  }
+  EAZ_FFI_TRY(CopyState(env, src, st, B, stream));
+
+  eaz_search_inputs in{};
+  in.beta = beta.typed_data();
+  in.gumbel = noise ? gumbel.typed_data() : nullptr;
+  in.sample_gumbel = sample ? sample_gumbel.typed_data() : nullptr;
+  in.env = &env;
+  return EazError(eaz_selfplay(&cfg, &in, &net, &st, (int32_t)T, tasks ? task_ids.typed_data() : nullptr, &out, ws,
+                               (*workspace)->size_bytes() - pad, stream),
+                  "eaz_selfplay");
 }
 
 // ------------------------------------------------------------------------------------------------ env step / init
@@ -678,6 +773,42 @@ XLA_FFI_DEFINE_HANDLER_SYMBOL(EazEvaluate, EvaluateImpl,
                                   .Attr<float>("max_u")
                                   .Attr<float>("novelty_scale")
                                   .Attr<int32_t>("max_episode_length"));
+
+XLA_FFI_DEFINE_HANDLER_SYMBOL(EazSelfplay, SelfplayImpl,
+                              ffi::Ffi::Bind()
+                                  .Ctx<ffi::PlatformStream<cudaStream_t>>()
+                                  .Arg<ffi::Buffer<ffi::F32>>()  // beta
+                                  .Arg<ffi::AnyBuffer>()         // action_map
+                                  .Arg<ffi::Buffer<ffi::U8>>()   // binary_set
+                                  .Arg<ffi::Buffer<ffi::F32>>()  // gumbel
+                                  .Arg<ffi::Buffer<ffi::F32>>()  // sample_gumbel
+                                  .Arg<ffi::Buffer<ffi::S32>>()  // task_ids
+                                  .Arg<ffi::Buffer<ffi::U8>>()   // workspace_in
+                                  .RemainingArgs()               // initial state leaves, 24 parameter buffers
+                                  .RemainingRets()               // final state leaves, 9 stacked outputs, workspace
+                                  EAZ_ENV_ATTRS()
+                                  .Attr<int32_t>("num_simulations")
+                                  .Attr<int32_t>("max_depth")
+                                  .Attr<int32_t>("max_num_considered_actions")
+                                  .Attr<float>("gumbel_scale")
+                                  .Attr<float>("discount")
+                                  .Attr<int32_t>("two_players_game")
+                                  .Attr<int32_t>("exploration")
+                                  .Attr<float>("value_scale")
+                                  .Attr<float>("maxvisit_init")
+                                  .Attr<int32_t>("rescale_values")
+                                  .Attr<int32_t>("flags")
+                                  .Attr<int32_t>("mlp_mode")
+                                  .Attr<int32_t>("hash_bits")
+                                  .Attr<int32_t>("hash_io")
+                                  .Attr<float>("max_u")
+                                  .Attr<float>("novelty_scale")
+                                  .Attr<int32_t>("steps")
+                                  .Attr<int32_t>("root_prior")
+                                  .Attr<int32_t>("action_sampling")
+                                  .Attr<float>("temperature")
+                                  .Attr<int32_t>("noise_seed")
+                                  .Attr<int32_t>("reuse_prepared"));
 
 XLA_FFI_DEFINE_HANDLER_SYMBOL(EazEnvStep, EnvStepImpl,
                               ffi::Ffi::Bind()

@@ -9,6 +9,7 @@ tests through tests/xla_ffi_stub/.
 Call shapes mirror the reference (file:line under /root/reference/src):
     epistemic_gumbel_muzero_policy(...)  selfplay.py:107-117, reanalyze.py:77-85, evaluate.py:36-45  (+ epistemic_summary())
     evaluate(...)                        evaluate.py:13-57 (the whole episode loop: one custom call)
+    selfplay(...)                        selfplay.py:78-149 (the whole scan of self-play steps: one custom call)
     env_step(...) / env_init(...)        selfplay.py:26-75,135,161,166
     forward_states(...)                  selfplay.py:89, reanalyze.py:67,90
     reanalyze_targets(...)               reanalyze.py:86-129
@@ -34,7 +35,7 @@ _eaz = ctypes.CDLL(os.path.join(_HERE, "libeaz_b200.so"), mode=ctypes.RTLD_GLOBA
 _shim = ctypes.CDLL(os.path.join(_HERE, "libeaz_xla_ffi.so"))
 for _name, _sym in (("eaz_search", "EazSearch"), ("eaz_env_step", "EazEnvStep"), ("eaz_env_init", "EazEnvInit"),
                     ("eaz_mlp_forward_states", "EazMlpForwardStates"), ("eaz_reanalyze_targets", "EazReanalyzeTargets"),
-                    ("eaz_hash_update", "EazHashUpdate"), ("eaz_evaluate", "EazEvaluate"),
+                    ("eaz_hash_update", "EazHashUpdate"), ("eaz_evaluate", "EazEvaluate"), ("eaz_selfplay", "EazSelfplay"),
                     ("eaz_replay_init", "EazReplayInit"), ("eaz_replay_add", "EazReplayAdd"), ("eaz_replay_sample", "EazReplaySample"),
                     ("eaz_replay_set_priorities", "EazReplaySetPriorities"), ("eaz_replay_status", "EazReplayStatus")):
     jax.ffi.register_ffi_target(_name, jax.ffi.pycapsule(getattr(_shim, _sym)), platform="CUDA")
@@ -182,6 +183,60 @@ def evaluate(params, model_state, env: EnvSpec, states, *, num_simulations, disc
         max_episode_length=i32(max_episode_length))
     returns = out[n]
     return returns.mean(), returns, with_leaves(env, states, out[:n])
+
+
+class SelfplayOutput(NamedTuple):  # selfplay.py:17-23, every field stacked over the steps
+    state: tuple                          # the states after each step as (eaz_env_compact records U8[T,B,S], rewards F32[T,B]): the
+    root_value: jax.Array                 # replay ring's format (one row per time slot)
+    root_epistemic_std: jax.Array
+    value_prediction: jax.Array
+    ube_prediction: jax.Array
+    q_values_epistemic_variance: jax.Array
+    action: jax.Array
+    trajectory: jax.Array                 # eaz_trajectory_pack records [T,B,4] (what the replay gather of main.py:383-385 sends)
+
+
+def selfplay(params, model_state, env: EnvSpec, states, rng_key, *, selfplay_steps, num_simulations, discount, exploration_beta=0.0,
+             directed_exploration=False, rescale_values=True, tasks=(1,), mlp_mode=1, uniform_prior=False, action_sampling=0, temperature=1.0,
+             hash_io=None, hash_bits=24):
+    """selfplay.py:78-149 from `states` (the last carry): selfplay_steps steps of the fused-root Gumbel search (the recurrent_fn's policy
+    head: exploration = directed_exploration, beta = exploration_beta * linspace(0, 1, B) when directed, selfplay.py:92,105) and the
+    auto-reset env step, as one custom call whose loop runs on the device.  The root noise [T,B,A] and the Subleq reset tasks [T,B]
+    (jax.random.choice over `tasks`, subleq.py:624) are drawn from rng_key; action_sampling (EAZ_ACTION_*) draws its noise in the
+    search.  Returns (final states, SelfplayOutput): lax.scan's (carry, ys) order."""
+    B, A, T = states.terminated.shape[0], env.num_actions, int(selfplay_steps)
+    leaves = state_leaves(env, states)
+    from . import _abi  # ctypes mirrors of the POD structs (no torch)
+
+    flags = DEFAULT_FLAGS
+    cfg = _abi.default_search_config(batch=B, num_simulations=num_simulations, mlp_mode=mlp_mode, action_sampling=int(action_sampling))
+    e = _abi.EazEnv(env.kind, env.size, None, env.word_size, env.binary_encoding, env.reward_fn)
+    _eaz.eaz_selfplay_workspace_bytes.restype = ctypes.c_size_t
+    ws_bytes = int(_eaz.eaz_selfplay_workspace_bytes(ctypes.byref(cfg), ctypes.byref(e)))
+    S = int(_eaz.eaz_env_compact_bytes(ctypes.byref(e)))
+    if ws_bytes == 0 or S <= 0:
+        raise ValueError(_eaz_error())
+    ws_bytes += 256
+    noise_key, task_key = jax.random.split(rng_key)
+    gumbel = jax.random.gumbel(noise_key, (T, B, A), jnp.float32)
+    task_ids = (jax.random.choice(task_key, jnp.asarray(tasks, jnp.int32), (T, B)) if env.kind == ENV_SUBLEQ else jnp.zeros((1,), jnp.int32))
+    beta = (exploration_beta if directed_exploration else 0.0) * jnp.linspace(0.0, 1.0, B, dtype=jnp.float32)
+    TB = lambda *s, dt=jnp.float32: jax.ShapeDtypeStruct((T, B) + s, dt)
+    out_types = ([jax.ShapeDtypeStruct(x.shape, x.dtype) for x in leaves] +
+                 [TB(dt=jnp.int32), TB(), TB(), TB(), TB(), TB(A), TB(4, dt=jnp.int32), TB(S, dt=jnp.uint8), TB(),
+                  jax.ShapeDtypeStruct((ws_bytes,), jnp.uint8)])
+    n = len(leaves)
+    aliases = {6: n + 9} | {7 + k: k for k in range(n)}  # workspace_in -> workspace, leaves stepped in place
+    out = jax.ffi.ffi_call("eaz_selfplay", out_types, input_output_aliases=aliases)(
+        beta, env.amap(), model_state["fc_az_net/xxhash32"]["binary_set"], gumbel, jnp.zeros((1,), jnp.float32), task_ids,
+        jnp.zeros((ws_bytes,), jnp.uint8), *leaves, *param_leaves(params), **env.attrs(), num_simulations=i32(num_simulations), max_depth=i32(0),
+        max_num_considered_actions=i32(16), gumbel_scale=f32(1.0), discount=f32(discount), two_players_game=i32(0),
+        exploration=i32(directed_exploration), value_scale=f32(0.1), maxvisit_init=f32(50.0), rescale_values=i32(rescale_values),
+        flags=i32(flags), mlp_mode=i32(mlp_mode), hash_bits=i32(hash_bits), hash_io=i32(env.kind == ENV_SUBLEQ if hash_io is None else hash_io),
+        max_u=f32(1.0), novelty_scale=f32(1.0), steps=i32(T), root_prior=i32(bool(uniform_prior)), action_sampling=i32(action_sampling),
+        temperature=f32(temperature), noise_seed=i32(0), reuse_prepared=i32(0))
+    action, rv, rstd, vp, up, qvar, traj, compact, rewards = out[n:n + 9]
+    return with_leaves(env, states, out[:n]), SelfplayOutput((compact, rewards), rv, rstd, vp, up, qvar, action, traj)
 
 
 def env_step(env: EnvSpec, states, action, *, auto_reset=False, task_ids=None):

@@ -657,6 +657,62 @@ class EvaluatePlan:
         return int(self.counters[0].item())
 
 
+SELFPLAY_OUTPUTS = ("action", "root_value", "root_epistemic_std", "value_prediction", "ube_prediction", "q_values_epistemic_variance",
+                    "trajectory", "states", "rewards")
+
+
+def alloc_selfplay_outputs(env: EnvSpec, T: int, B: int, device="cuda") -> dict:
+    """The stacked outputs of eaz_selfplay: [T,B] rows, q_values_epistemic_variance [T,B,A], trajectory [T,B,4], states [T,B,S]."""
+    torch = require_cuda()
+    f = lambda *s: torch.empty((T, B) + s, dtype=torch.float32, device=device)
+    return dict(action=torch.empty((T, B), dtype=torch.int32, device=device), root_value=f(), root_epistemic_std=f(), value_prediction=f(),
+                ube_prediction=f(), q_values_epistemic_variance=f(env.num_actions), trajectory=torch.empty((T, B, 4), dtype=torch.int32, device=device),
+                states=torch.empty((T, B, env.compact_bytes), dtype=torch.uint8, device=device), rewards=f())
+
+
+class SelfplayPlan:
+    """Workspace of eaz_selfplay for one (cfg, env) shape.  The library keeps the scan's CUDA graph with the workspace, so repeated
+    run() calls on the same buffers launch the graph built by the first one.  The workspace starts zeroed: the draw counter of the
+    in-search noise starts at 0."""
+
+    def __init__(self, cfg: _abi.EazSearchConfig, env: EnvSpec, net: FcParams, device="cuda"):
+        torch = require_cuda()
+        self.cfg, self.env, self.net = cfg, env, net
+        nbytes = load().eaz_selfplay_workspace_bytes(C.byref(cfg), C.byref(env.struct()))
+        if nbytes == 0:
+            raise EazError("eaz_selfplay_workspace_bytes rejected the configuration: " + load().eaz_last_error().decode())
+        self.workspace = torch.zeros(nbytes + 256, dtype=torch.uint8, device=device)
+        off = (-self.workspace.data_ptr()) % 256
+        self._ws_ptr = C.c_void_p(self.workspace.data_ptr() + off)
+        self._ws_bytes = C.c_size_t(nbytes)
+
+    def run(self, beta, states: dict, T: int, out: dict, gumbel=None, sample_gumbel=None, task_ids=None, invalid_actions=None,
+            reuse_prepared: bool = False):
+        """eaz_selfplay: T steps from `states` (stepped in place) into the stacked outputs `out` (alloc_selfplay_outputs; a missing or
+        None entry is not written).  gumbel / sample_gumbel [T,B,A] (None: drawn in the search), task_ids [T,B] (Subleq).
+        reuse_prepared: the tables an earlier run() built for the same net are still in the workspace (no preparation)."""
+        import torch
+
+        B, A = self.cfg.batch, self.env.num_actions
+        shapes = dict(q_values_epistemic_variance=(T, B, A), trajectory=(T, B, 4), states=(T, B, self.env.compact_bytes))
+        for name in SELFPLAY_OUTPUTS:
+            t = out.get(name)
+            if t is not None and tuple(t.shape) != shapes.get(name, (T, B)):
+                raise EazError(f"selfplay output {name} must have shape {shapes.get(name, (T, B))}, got {tuple(t.shape)}")
+        for name, t, shape in (("gumbel", gumbel, (T, B, A)), ("sample_gumbel", sample_gumbel, (T, B, A)), ("task_ids", task_ids, (T, B))):
+            if t is not None and tuple(t.shape) != shape:
+                raise EazError(f"selfplay {name} must have shape {shape}, got {tuple(t.shape)}")
+        cfg = _abi.EazSearchConfig.from_buffer_copy(self.cfg)
+        if reuse_prepared:
+            cfg.flags |= _abi.FLAG_REUSE_PREPARED
+        e, n, s = self.env.struct(), self.net.struct(), state_struct(self.env, states)
+        inp = _abi.EazSearchInputs(None, None, None, _ptr(beta, torch.float32), None, _ptr(invalid_actions, torch.uint8), _ptr(gumbel, torch.float32),
+                                   C.pointer(e), None, _ptr(sample_gumbel, torch.float32))
+        o = _abi.EazSelfplayOutputs(*[_ptr(out.get(name)) for name in SELFPLAY_OUTPUTS])
+        check(load().eaz_selfplay(C.byref(cfg), C.byref(inp), C.byref(n), C.byref(s), int(T), _ptr(task_ids, torch.int32), C.byref(o), self._ws_ptr,
+                                  self._ws_bytes, _stream()), "eaz_selfplay")
+
+
 def reanalyze_targets(discount, exploration_beta, exploration_ube_target, temperature, action, qvalues, qvalues_epistemic_variance, visit_counts,
                       value, value_epistemic_std, next_state_value, next_rewards, next_terminated, terminated, invalid_actions=None, out=None) -> dict:
     """eaz_reanalyze_targets (reanalyze.py:86-129) on device tensors; `out` may hold pre-allocated result tensors."""

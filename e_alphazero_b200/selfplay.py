@@ -1,6 +1,8 @@
 """Host-side mirror of the reference's selfplay step (selfplay.py:86-143) and reanalyze search
 (reanalyze.py:52-131) on top of the fused CUDA path.  One `SelfplayRunner.step()` is the unit the
-benchmark times: root forward -> E-MCTS search -> auto-reset env step."""
+benchmark times: root forward -> E-MCTS search -> auto-reset env step.  `SelfplayRunner.scan()` and the
+drop-in `selfplay()` run the reference's whole scan of such steps (selfplay.py:78-149) as one device
+program (csrc/selfplay.cu: eaz_selfplay)."""
 from __future__ import annotations
 
 from dataclasses import dataclass
@@ -19,6 +21,7 @@ class SelfplayOutput:  # selfplay.py:17-23
     ube_prediction: Any
     q_values_epistemic_variance: Any
     action: Any = None
+    trajectory: Any = None  # scan(): the eaz_trajectory_pack records [T,B,4] of the states after every step
 
 
 class SelfplayRunner:
@@ -79,10 +82,14 @@ class SelfplayRunner:
         self._graphs = {}
         self._static = None
         self._stale = True
+        self._scan_plan = None   # eaz_selfplay's workspace (its own parameter-derived tables: staleness tracked apart from step()'s)
+        self._scan_stale = True
+        self._scan_out = None    # (T, stacked output buffers)
 
     def params_updated(self):
         """Call after the network parameters / hash set changed (learner update, broadcast)."""
         self._stale = True
+        self._scan_stale = True
 
     def draw_gumbel(self):
         torch = require_cuda()
@@ -102,6 +109,44 @@ class SelfplayRunner:
         reuse = not self._stale
         self._stale = False
         return self._step_eager(states, gumbel, task_ids, reuse_prepared=reuse, sample_gumbel=sample_gumbel)
+
+    def scan(self, states: dict, T: int, gumbel=None, sample_gumbel=None, task_ids=None):
+        """The reference's selfplay() scan (selfplay.py:78-149): T steps of step() as one device program (a CUDA graph whose loop the
+        device stops after T steps; the host launches it once).  states: device state dict, stepped in place to the final carry.
+        gumbel / sample_gumbel [T,B,A] and task_ids [T,B] hold row t for step t; without them the noise follows the runner's rules
+        (drawn from its generator, [T,B,A] in one call, or inside the search with device_noise=True) and the Subleq reset tasks are
+        drawn from the generator in one [T,B] call.
+        Returns (states, SelfplayOutput) whose fields are [T,B] stacks in buffers this runner owns (the next scan of the same T
+        overwrites them): row t equals step t's output of T step() calls.  `state` is the states after every step in the replay ring's
+        wire format, dict(compact=[T,B,S] uint8, rewards=[T,B]) (ops.env_uncompact decodes a row); `trajectory` holds the
+        trajectory() records [T,B,4]."""
+        torch = require_cuda()
+        T = int(T)
+        if T < 0:
+            raise ValueError(f"scan: T must be >= 0, got {T}")
+        if self._scan_plan is None:
+            self._scan_plan = ops.SelfplayPlan(self.cfg, self.env, self.net, device=self.device)
+        if self._scan_out is None or self._scan_out[0] != T:
+            self._scan_out = (T, ops.alloc_selfplay_outputs(self.env, T, self.B, device=self.device))
+        out = self._scan_out[1]
+        noise = lambda: (-(-torch.rand((T, self.B, self.A), device=self.device, generator=self.gen).clamp_(1e-20, 1.0 - 1e-7).log()).log())
+        if gumbel is None and not self.device_noise:
+            gumbel = noise()
+        if sample_gumbel is None and self.sampling and not self.device_noise:
+            sample_gumbel = noise()
+        if task_ids is None and self.env.kind == _abi.ENV_SUBLEQ:
+            task_ids = self.tasks[torch.randint(0, self.tasks.numel(), (T, self.B), device=self.device, generator=self.gen)]
+        as_f32 = lambda t: None if t is None else t.to(dtype=torch.float32).contiguous()
+        task_ids = None if task_ids is None else task_ids.to(dtype=torch.int32).contiguous()
+        self._scan_plan.run(self.beta, states, T, out, gumbel=as_f32(gumbel), sample_gumbel=as_f32(sample_gumbel) if self.sampling else None,
+                            task_ids=task_ids, reuse_prepared=not self._scan_stale)
+        if T > 0:
+            self._scan_stale = False
+        res = SelfplayOutput(state=dict(compact=out["states"], rewards=out["rewards"]), root_value=out["root_value"],
+                             root_epistemic_std=out["root_epistemic_std"], value_prediction=out["value_prediction"],
+                             ube_prediction=out["ube_prediction"], q_values_epistemic_variance=out["q_values_epistemic_variance"],
+                             action=out["action"], trajectory=out["trajectory"])
+        return states, res
 
     def _step_graph(self, states, gumbel, task_ids, sample_gumbel=None):
         torch = require_cuda()
@@ -200,3 +245,63 @@ class SelfplayRunner:
         """Pack this step's replay record (ops.trajectory_pack: action, reward bits, flags, compact-state word) into `dst`
         (int32 [B,4], e.g. one row of a [T,B,4] scan buffer): one small kernel, nothing aliased."""
         return ops.trajectory_pack(self.env, states, out.action, dst)
+
+
+_runners: dict = {}
+
+
+def _leaves(state):
+    return state.leaves if hasattr(state, "leaves") else state
+
+
+def selfplay(model, config, context, last_states, rng_key=None):
+    """Drop-in for selfplay.selfplay (selfplay.py:78-149): config.selfplay_steps steps of the self-play step from `last_states` (a
+    pgx State of e_alphazero_b200.pgx, not modified) as one device program.  `config` needs the attributes the reference reads:
+    selfplay_steps, selfplay_simulations_per_step, discount, exploration_beta, directed_exploration, rescale_q_values_in_search
+    (+ optional mlp_mode); `context.env` is an e_alphazero_b200.pgx env.  rng_key: an emctx.PreDrawnGumbel carrying the root noise
+    [T,B,A], an int seed of the runner's generator, or None (the generator continues).
+
+    The reference's return statement is not in the sources this mirrors; the order here follows lax.scan's (carry, ys):
+    (final states, SelfplayOutput) with every field stacked over the T steps and `state` decoded to pgx State leaves [T,B,...] (the
+    states after each step), plus `trajectory` [T,B,4]."""
+    from .context import as_fc_params
+    from .emctx import PreDrawnGumbel
+    from .pgx import State, Subleq
+
+    require_cuda()
+    env = context.env
+    net = as_fc_params(model, env=env)
+    states = {k: v.clone() for k, v in _leaves(last_states).items() if k != "observation"}
+    B, T = states["terminated"].shape[0], int(config.selfplay_steps)
+    key = (id(env), id(net), B, int(config.selfplay_simulations_per_step), float(config.discount), float(config.exploration_beta),
+           bool(config.directed_exploration), bool(config.rescale_q_values_in_search), int(getattr(config, "mlp_mode", _abi.MLP_EXACT)))
+    hit = _runners.get(key)  # (env, net, runner): the strong references keep the id()s in the key unique
+    if hit is None or hit[0] is not env or hit[1] is not net:
+        while len(_runners) >= 8:
+            _runners.pop(next(iter(_runners)))
+        hit = _runners[key] = (env, net, SelfplayRunner(env.spec, net, B, int(config.selfplay_simulations_per_step), float(config.discount),
+                                                        exploration_beta=float(config.exploration_beta),
+                                                        directed_exploration=bool(config.directed_exploration),
+                                                        rescale_values=bool(config.rescale_q_values_in_search),  # selfplay.py:114-116
+                                                        mlp_mode=int(getattr(config, "mlp_mode", _abi.MLP_EXACT)),
+                                                        tasks=env.tasks if isinstance(env, Subleq) else (1,), device=str(states["terminated"].device),
+                                                        fused_root=True))
+    r = hit[2]
+    tok = net.content_token()
+    if getattr(r, "_net_token", None) != tok:  # rebuild the parameter-derived tables only when the parameters moved
+        r.params_updated()
+        r._net_token = tok
+    gumbel = None
+    if isinstance(rng_key, PreDrawnGumbel):
+        gumbel = rng_key.gumbel
+    elif isinstance(rng_key, int):
+        r.gen.manual_seed(rng_key)
+    states, out = r.scan(states, T, gumbel=gumbel)
+    S = env.spec.compact_bytes
+    dec = ops.env_uncompact(env.spec, out.state["compact"].reshape(T * B, S), out.state["rewards"].reshape(T * B))
+    stacked = State(env, {k: v.reshape((T, B) + tuple(v.shape[1:])) for k, v in dec.items()})
+    keep = lambda t: t.clone()
+    return State(env, states), SelfplayOutput(state=stacked, root_value=keep(out.root_value), root_epistemic_std=keep(out.root_epistemic_std),
+                                              value_prediction=keep(out.value_prediction), ube_prediction=keep(out.ube_prediction),
+                                              q_values_epistemic_variance=keep(out.q_values_epistemic_variance), action=keep(out.action),
+                                              trajectory=keep(out.trajectory))

@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define EAZ_ABI_VERSION 6
+#define EAZ_ABI_VERSION 7
 
 enum {
   EAZ_OK = 0,
@@ -379,6 +379,49 @@ size_t eaz_evaluate_workspace_bytes(const eaz_search_config* cfg, const eaz_env*
  * allocation of device memory, no host synchronisation after the graph of the workspace is built. */
 int eaz_evaluate(const eaz_search_config* cfg, const eaz_search_inputs* in, const eaz_fc_params* net, eaz_state* states, float* returns,
                  int32_t max_episode_length, void* workspace, size_t workspace_bytes, void* stream);
+
+/* ------------------------------------------------------------------------ */
+/* ABI 7 (appended): the self-play scan of selfplay.py:78-149 as one device    */
+/* program -- lax.scan(step_fn, starting_states, key_seq) over T steps of      */
+/* {fused-root search, auto-reset env step, row t of every stacked output},    */
+/* a CUDA graph whose WHILE conditional node the device stops after T steps.   */
+
+/* The stacked per-step outputs of the scan (SelfplayOutput, selfplay.py:17-23, stacked over the steps as lax.scan stacks them).  Row t
+ * holds what step t returns; every pointer may be NULL (not written).  A = eaz_env_num_actions, S = eaz_env_compact_bytes. */
+typedef struct eaz_selfplay_outputs {
+  int32_t* action;                    /* [T,B] the played action (the sampled one with cfg.action_sampling != EAZ_ACTION_SEARCH) */
+  float* root_value;                  /* [T,B] search summary value (selfplay.py:137) */
+  float* root_epistemic_std;          /* [T,B] search summary value_epistemic_std (:138) */
+  float* value_prediction;            /* [T,B] the fused root's network value (:139) */
+  float* ube_prediction;              /* [T,B] the fused root's network UBE (:140) */
+  float* q_values_epistemic_variance; /* [T,B,A] search summary qvalues_epistemic_variance (:141) */
+  int32_t* trajectory;                /* [T,B,4] the eaz_trajectory_pack record of the states AFTER step t and its played action */
+  uint8_t* states;                    /* [T,B,S] SelfplayOutput.state: the states AFTER step t (auto-reset applied), eaz_env_compact
+                                         encoding -- the replay ring's format, decodable with eaz_env_uncompact */
+  float* rewards;                     /* [T,B] rewards[:,0] of the states after step t (the leaf the compact encoding does not carry) */
+} eaz_selfplay_outputs;
+
+/* Workspace of eaz_selfplay (256-byte aligned): the loop's device words, the staged noise of one step (gumbel and sample_gumbel, [B,A]
+ * each), one step's search outputs and the search workspace of `cfg`.  0 if cfg / env are rejected. */
+size_t eaz_selfplay_workspace_bytes(const eaz_search_config* cfg, const eaz_env* env);
+
+/* selfplay() (selfplay.py:78-149): T steps of step_fn (selfplay.py:86-143) from `states`, stepped in place -- on return `states` holds
+ * the final carry.  Step t: the fused-root search of `cfg` (forward.apply on the states, selfplay.py:89, with the recurrent_fn's policy
+ * head; root_prior / action_sampling / temperature as in eaz_search_gumbel), the auto-reset env step on the played actions
+ * (selfplay.py:26-75,135; Subleq resets take their task from row t of task_ids [T,B], required for Subleq, ignored for DeepSea) and
+ * row t of every non-NULL output of `out`.
+ * From `in` it reads env, beta [B] (non-NULL), invalid_actions [B,A] (may be NULL; the same for every step) and the noise:
+ * gumbel / sample_gumbel are [T,B,A] (row t for step t) or NULL = drawn inside the search from (cfg.noise_seed, the workspace's draw
+ * counter, which advances once per step whose search draws noise itself, tree, action).  prior_logits / value /
+ * value_epistemic_variance must be NULL (fused root); the other fields are not read.  EAZ_FLAG_PUCT is refused (the reference's
+ * self-play uses the Gumbel policy).  states->observation must be NULL (the loop does not materialise observations).  T == 0 writes
+ * and enqueues nothing.  Every argument is checked before anything is enqueued.
+ * The parameter-derived tables are rebuilt once per call, before the loop, unless cfg->flags has EAZ_FLAG_REUSE_PREPARED (an earlier
+ * call on this workspace built them for the same net); this does not advance the draw counter.  The loop is a CUDA graph built on the
+ * first call for a workspace and kept with it; a call with another cfg / env / net / T / buffer address rebuilds it.  Asynchronous on
+ * `stream`: no allocation of device memory, no host synchronisation after the graph of the workspace is built. */
+int eaz_selfplay(const eaz_search_config* cfg, const eaz_search_inputs* in, const eaz_fc_params* net, eaz_state* states, int32_t T,
+                 const int32_t* task_ids, eaz_selfplay_outputs* out, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------ */
 /* Convolutional evaluators (SURVEY 8f-4): EpistemicResidualAZNet               */
