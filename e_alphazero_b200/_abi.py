@@ -8,7 +8,7 @@ from __future__ import annotations
 
 import ctypes as C
 
-ABI_VERSION = 7
+ABI_VERSION = 8
 
 EAZ_OK = 0
 EAZ_ERR_INVALID_ARG = -1

@@ -31,6 +31,7 @@ EXPORTS = [
     "eaz_replay_add", "eaz_priority_sample_keyed", "eaz_priority_status_async",
     "eaz_evaluate_workspace_bytes", "eaz_evaluate",
     "eaz_selfplay_workspace_bytes", "eaz_selfplay",
+    "eaz_replay_add_sequence",
 ]
 
 

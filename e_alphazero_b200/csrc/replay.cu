@@ -34,11 +34,23 @@
 // A keyed sample (eaz_priority_sample_keyed) is sample(K) with (seed, draw_ctr) := (key[0], key[1]) that writes nothing into
 // the buffer: no counter advance, no status bit.  eaz_replay_add's add_step is add_step(c) with c = the header's cursor.
 //
+// add_sequence(n) (eaz_replay_add_sequence) IS n calls of add_step(cursor), in every byte of the buffer; it is not a second rule.
+//   Derivation, with c, len, m = the header's cursor, length, max_priority before the call and w = w(m): call k (0 <= k < n) is
+//   add_step(c + k), which sets length min(len + k + 1, T), so it writes row c + k - 1 := w if len + k >= 1 (else 0), then row
+//   c + k := 0.  Call k only writes logical rows c + k - 1 and c + k, so a physical row ends with the value of the LAST logical
+//   row j == it (mod T) in c - 1 .. c + n - 1: logical row c + n - 1 ends at 0, logical row c + k - 1 (k < n) at w if
+//   len + k >= 1, else 0.  The touched physical rows are the last min(n + 1, T) of those logical rows.  The header ends with
+//   cursor (c + n) % T and length min(len + n, T); max_priority, alpha, status and the tags are not written by add_step(cursor).
+//   The levels being a pure function of the leaves, setting the touched leaves to their final values and recomputing their
+//   ancestors gives the bytes of the n sequential calls, for any n (n > T included) and any starting ring.
+//
 // Kernels: add_step is one CTA (two rows of B leaves, then their ancestors level by level); set is a tag pass (atomicMax
 // of k per leaf: last occurrence wins), a leaf pass, and one launch per level above the leaves; sample is one warp per
 // sample (descent + gather of both slots' compact records and rewards) and, unless keyed, a one-thread counter bump.
 // eaz_replay_add is a compaction kernel that writes ring row `cursor` (read from the header) followed by add_step with the
-// slot taken from the header, so the cursor never leaves the device.  All latency-bound.
+// slot taken from the header, so the cursor never leaves the device.  eaz_replay_add_sequence is a row-copy kernel (the last
+// min(n, T) rows into their slots), a leaf pass over the touched rows and one launch per level above the leaves, the root's
+// launch also writing the header: L + 1 launches whatever n.  All latency-bound.
 #include "common.cuh"
 
 #include <float.h>
@@ -287,6 +299,79 @@ __global__ void replay_compact_kernel(EnvDesc env, StateSoA s, const PrioHeader*
   ring_rewards[slot * B + b] = s.rewards[b];
 }
 
+// ---- eaz_replay_add_sequence (add_sequence(n) of the contract).  `keep` = min(n, T) rows are written, `rows` = min(n + 1, T) leaf
+// rows are touched.  Every kernel reads the cursor c from the header; only the root's level pass, the last launch, writes it.
+
+// physical slot of the first of the last `count` logical slots c .. c + n - 1 (ring rows: (c, n); leaf rows: (c - 1, n + 1))
+__device__ __forceinline__ int seq_first_slot(int c, int n, int count, int T) { return (int)(((int64_t)c + n - count + T) % T); }
+
+// ring rows j = n - keep .. n - 1 of the sequence into slots (c + j) % T; V: the widest word dividing a row of B records
+template <typename V>
+__global__ void __launch_bounds__(256) replay_seq_copy_kernel(const PrioHeader* __restrict__ hdr, const V* __restrict__ src, V* __restrict__ dst,
+                                                              int64_t row_words, const float* __restrict__ rewards, float* __restrict__ ring_rewards,
+                                                              int B, int T, int n, int keep) {
+  const int s0 = seq_first_slot(hdr->cursor, n, keep, T);
+  const int64_t j0 = n - keep, stride = (int64_t)gridDim.x * blockDim.x, first = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  for (int64_t e = first; e < keep * row_words; e += stride) {
+    const int64_t q = e / row_words, o = e - q * row_words;
+    const int64_t slot = s0 + q < T ? s0 + q : s0 + q - T;
+    dst[slot * row_words + o] = src[(j0 + q) * row_words + o];
+  }
+  for (int64_t e = first; e < (int64_t)keep * B; e += stride) {
+    const int64_t q = e / B, b = e - q * B;
+    const int64_t slot = s0 + q < T ? s0 + q : s0 + q - T;
+    ring_rewards[slot * B + b] = rewards[(j0 + q) * B + b];
+  }
+}
+
+// the leaves of the touched rows: logical row c - 1 + k (k = n + 1 - rows + q) gets w if len + k >= 1, the last (k = n) gets 0
+__global__ void __launch_bounds__(256) prio_seq_leaf_kernel(PrioTree tr, int n, int rows) {
+  const PrioHeader h = *tr.hdr;
+  const int T = tr.T, B = tr.B, p0 = seq_first_slot(h.cursor - 1, n + 1, rows, T);
+  const float w = prio_weight(h.max_priority, h.alpha);
+  const int stride = gridDim.x * blockDim.x;
+  for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < rows * B; e += stride) {
+    const int q = e / B, b = e - q * B, k = n + 1 - rows + q;
+    const int p = p0 + q < T ? p0 + q : p0 + q - T;
+    tr.lvl[0][(size_t)p * B + b] = q == rows - 1 ? 0.0f : (h.length > 0 || k > 0) ? w : 0.0f;
+  }
+}
+
+// one warp per ancestor at level l (>= 1) of the touched leaves: every node of the level when rows == T, else the nodes over the
+// touched leaf range, which wraps past slot T - 1 into at most two ranges (merged where they meet, so no node is computed twice).
+// The root's pass (n_nodes == 1, one warp) then writes the header: cursor (c + n) % T, length min(length + n, T).
+__global__ void __launch_bounds__(256) prio_seq_level_kernel(PrioHeader* hdr, const float* child, float* node, int l, int n_nodes, int T, int B,
+                                                             int n, int rows) {
+  const int q = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  const int c = hdr->cursor;
+  int lo0 = 0, n0 = n_nodes, lo1 = 0, n1 = 0;
+  if (rows < T) {
+    const int p0 = seq_first_slot(c - 1, n + 1, rows, T), p1 = p0 + rows;
+    lo0 = p0 * B;
+    int hi0 = min(p1, T) * B - 1, hi1 = -1;
+    if (p1 > T) hi1 = (p1 - T) * B - 1;
+    lo0 >>= 5 * l, hi0 >>= 5 * l;
+    n0 = hi0 - lo0 + 1;
+    if (hi1 >= 0) {
+      hi1 >>= 5 * l;
+      if (lo1 <= hi0 + 1 && lo0 <= hi1 + 1) {
+        const int lo = min(lo0, lo1), hi = max(hi0, hi1);
+        lo0 = lo, n0 = hi - lo + 1;
+      } else {
+        n1 = hi1 - lo1 + 1;
+      }
+    }
+  }
+  if (q < n0 + n1) prio_recompute(child, node, q < n0 ? lo0 + q : lo1 + (q - n0), lane);
+  if (n_nodes == 1 && q == 0) {
+    __syncwarp();  // every lane has read the cursor
+    if (lane == 0) {
+      hdr->cursor = (int)(((int64_t)c + n) % T);
+      hdr->length = (int)min((int64_t)hdr->length + n, (int64_t)T);
+    }
+  }
+}
+
 static int prio_sample_launch(void* tree, size_t tree_bytes, int32_t T, int32_t B, int32_t K, const uint32_t* key, const uint8_t* states,
                               const float* rewards, int32_t S, int32_t* indices, float* probabilities, uint8_t* first, float* first_rewards,
                               uint8_t* second, float* second_rewards, cudaStream_t s, const char* who) {
@@ -392,6 +477,48 @@ int eaz_replay_add(const eaz_env* env, const eaz_state* state, uint8_t* ring_sta
   EAZ_CHECK_LAUNCH("replay_compact_kernel");
   prio_add_step_kernel<<<1, 1024, 0, s>>>(tr, -1);
   EAZ_CHECK_LAUNCH("prio_add_step_kernel");
+  return 0;
+}
+
+int eaz_replay_add_sequence(const eaz_env* env, const uint8_t* compact, const float* rewards, int32_t steps, uint8_t* ring_states,
+                            float* ring_rewards, void* tree, size_t tree_bytes, int32_t T, int32_t B, int32_t S, void* stream) {
+  EnvDesc d;
+  if (int rc = make_env_desc(env, &d)) return rc;
+  PrioTree tr;
+  if (int rc = prio_view(tree, tree_bytes, T, B, &tr, "eaz_replay_add_sequence")) return rc;
+  EAZ_CHECK_ARG(steps >= 0 && steps < INT32_MAX, "eaz_replay_add_sequence: steps = %d outside [0, 2^31 - 1)", steps);
+  EAZ_CHECK_ARG(S == d.compact_bytes, "eaz_replay_add_sequence: S = %d, eaz_env_compact_bytes(env) = %d", S, d.compact_bytes);
+  EAZ_CHECK_ARG(ring_states && ring_rewards, "eaz_replay_add_sequence: NULL ring_states / ring_rewards");
+  EAZ_CHECK_ARG(steps == 0 || (compact && rewards), "eaz_replay_add_sequence: NULL compact / rewards");
+  if (steps == 0) return 0;
+  cudaStream_t s = (cudaStream_t)stream;
+  const int keep = min(steps, T), rows = steps < T ? steps + 1 : T;
+  const size_t row_bytes = (size_t)B * S;
+  const int64_t copy_elems = (int64_t)keep * (int64_t)row_bytes;
+  const int copy_blocks = (int)std::min<int64_t>((copy_elems + 255) / 256, 4096);
+  const bool a16 = row_bytes % 16 == 0 && (uintptr_t)compact % 16 == 0 && (uintptr_t)ring_states % 16 == 0;
+  const bool a4 = row_bytes % 4 == 0 && (uintptr_t)compact % 4 == 0 && (uintptr_t)ring_states % 4 == 0;
+  if (a16)
+    replay_seq_copy_kernel<uint4><<<copy_blocks, 256, 0, s>>>(tr.hdr, (const uint4*)compact, (uint4*)ring_states, (int64_t)(row_bytes / 16), rewards,
+                                                              ring_rewards, B, T, steps, keep);
+  else if (a4)
+    replay_seq_copy_kernel<uint32_t><<<copy_blocks, 256, 0, s>>>(tr.hdr, (const uint32_t*)compact, (uint32_t*)ring_states, (int64_t)(row_bytes / 4),
+                                                                 rewards, ring_rewards, B, T, steps, keep);
+  else
+    replay_seq_copy_kernel<uint8_t><<<copy_blocks, 256, 0, s>>>(tr.hdr, compact, ring_states, (int64_t)row_bytes, rewards, ring_rewards, B, T,
+                                                                steps, keep);
+  EAZ_CHECK_LAUNCH("replay_seq_copy_kernel");
+  prio_seq_leaf_kernel<<<(int)std::min<int64_t>(((int64_t)rows * B + 255) / 256, 4096), 256, 0, s>>>(tr, steps, rows);
+  EAZ_CHECK_LAUNCH("prio_seq_leaf_kernel");
+  for (int l = 1; l < tr.L; ++l) {
+    const int n_nodes = (int)((((int64_t)tr.N - 1) >> (5 * l)) + 1);
+    // the host does not know the cursor: it launches enough warps for the widest placement of the touched leaves (two ranges
+    // of rows * B leaves in all cover at most rows * B / 32^l + 4 nodes)
+    const int warps = rows == T ? n_nodes : (int)std::min<int64_t>(n_nodes, ((int64_t)rows * B >> (5 * l)) + 4);
+    const int wpb = std::min(warps, 8);  // warps per block
+    prio_seq_level_kernel<<<ceil_div(warps, wpb), 32 * wpb, 0, s>>>(tr.hdr, tr.lvl[l - 1], tr.lvl[l], l, n_nodes, T, B, steps, rows);
+    EAZ_CHECK_LAUNCH("prio_seq_level_kernel");
+  }
   return 0;
 }
 

@@ -14,8 +14,9 @@
 //   eaz_mlp_forward_states   forward.apply(params, state, states.observation)            selfplay.py:89, reanalyze.py:67,90
 //   eaz_reanalyze_targets    the target arithmetic after the search                      reanalyze.py:86-129
 //   eaz_hash_update     BaseHash.update on the observations of a training batch           network/hashes.py:45-50, train.py:22
-//   eaz_replay_init / _add / _sample / _set_priorities / _status
+//   eaz_replay_init / _add / _add_sequence / _sample / _set_priorities / _status
 //                       flashbax make_prioritised_flat_buffer on the compact ring         main.py:217-225, 383-385, 413-414, 454
+//                       (_add_sequence: a whole self-play scan's states, add_sequences=True)
 //                       (csrc/replay.cu: the write cursor lives in the tree header, sampling is keyed and reads nothing it writes)
 //
 // XLA owns every buffer (results and the workspace are XLA-allocated), the stream comes from PlatformStream, errors travel as
@@ -635,6 +636,37 @@ ffi::Error ReplayAddImpl(cudaStream_t stream, ffi::AnyBuffer action_map, ffi::Bu
                   "eaz_replay_add");
 }
 
+// args : action_map, ring_states_in U8[T,B,S], ring_rewards_in F32[T,B], tree_in U8, compact U8[T',B,S], rewards F32[T',B] (a scan's
+//        SelfplayOutput.state: T' time steps of the B envs, appended in time order at the device cursor)
+// rets : ring_states, ring_rewards, tree (alias each to its input; otherwise the inputs are copied first)
+ffi::Error ReplayAddSequenceImpl(cudaStream_t stream, ffi::AnyBuffer action_map, ffi::Buffer<ffi::U8> states_in, ffi::Buffer<ffi::F32> rewards_in,
+                                 ffi::Buffer<ffi::U8> tree_in, ffi::Buffer<ffi::U8> compact, ffi::Buffer<ffi::F32> rewards,
+                                 ffi::ResultBuffer<ffi::U8> ring_states, ffi::ResultBuffer<ffi::F32> ring_rewards, ffi::ResultBuffer<ffi::U8> tree,
+                                 int32_t env_kind, int32_t size, int32_t word_size, int32_t binary_encoding, int32_t reward_fn) {
+  const eaz_env env = MakeEnv(env_kind, size, word_size, binary_encoding, reward_fn, action_map.untyped_data());
+  int64_t T, B, S;
+  EAZ_FFI_TRY(RingDims(states_in, rewards_in, &T, &B, &S));
+  size_t in_bytes = 0, tree_bytes = 0;
+  EAZ_FFI_TRY(CheckTree(tree_in, T, B, &in_bytes));
+  EAZ_FFI_TRY(CheckTree(*tree, T, B, &tree_bytes));
+  EAZ_FFI_TRY(CheckRecord(env, S));
+  if (ring_states->size_bytes() != states_in.size_bytes() || ring_rewards->size_bytes() != rewards_in.size_bytes() || tree_bytes != in_bytes)
+    return Bad("EazReplayAddSequence: each result must have the shape of its input");
+  const auto dc = compact.dimensions();
+  const auto dr = rewards.dimensions();
+  if (dc.size() != 3 || dc[1] != B || dc[2] != S)
+    return Bad("EazReplayAddSequence: compact must be [T', B, S] = [T', " + std::to_string(B) + ", " + std::to_string(S) + "] for the ring's B envs");
+  if (dr.size() != 2 || dr[0] != dc[0] || dr[1] != B)
+    return Bad("EazReplayAddSequence: rewards must be [T', B] = [" + std::to_string(dc[0]) + ", " + std::to_string(B) + "]");
+  if (dc[0] >= INT32_MAX) return Bad("EazReplayAddSequence: T' = " + std::to_string(dc[0]) + " time steps, at most 2^31 - 2");
+  EAZ_FFI_TRY(CopyUnlessAliased(ring_states->untyped_data(), states_in.untyped_data(), states_in.size_bytes(), stream));
+  EAZ_FFI_TRY(CopyUnlessAliased(ring_rewards->untyped_data(), rewards_in.untyped_data(), rewards_in.size_bytes(), stream));
+  EAZ_FFI_TRY(CopyUnlessAliased(tree->untyped_data(), tree_in.untyped_data(), in_bytes, stream));
+  return EazError(eaz_replay_add_sequence(&env, compact.typed_data(), rewards.typed_data(), (int32_t)dc[0], ring_states->typed_data(),
+                                          ring_rewards->typed_data(), tree->untyped_data(), tree_bytes, (int32_t)T, (int32_t)B, (int32_t)S, stream),
+                  "eaz_replay_add_sequence");
+}
+
 // args : action_map, ring_states U8[T,B,S], ring_rewards F32[T,B], tree U8, key U32[2] = (seed, draw counter); none is aliased or written
 // rets : indices S32[K], probabilities F32[K], the decoded `first` state leaves (K envs), the `second` state leaves,
 //        scratch U8[2 K (S + 4) + 16] (the gathered compact records and rewards)
@@ -897,6 +929,20 @@ XLA_FFI_DEFINE_HANDLER_SYMBOL(EazReplayAdd, ReplayAddImpl,
                                   .Arg<ffi::Buffer<ffi::F32>>()  // ring_rewards_in
                                   .Arg<ffi::Buffer<ffi::U8>>()   // tree_in
                                   .RemainingArgs()               // state leaves
+                                  .Ret<ffi::Buffer<ffi::U8>>()   // ring_states
+                                  .Ret<ffi::Buffer<ffi::F32>>()  // ring_rewards
+                                  .Ret<ffi::Buffer<ffi::U8>>()   // tree
+                                  EAZ_ENV_ATTRS());
+
+XLA_FFI_DEFINE_HANDLER_SYMBOL(EazReplayAddSequence, ReplayAddSequenceImpl,
+                              ffi::Ffi::Bind()
+                                  .Ctx<ffi::PlatformStream<cudaStream_t>>()
+                                  .Arg<ffi::AnyBuffer>()         // action_map
+                                  .Arg<ffi::Buffer<ffi::U8>>()   // ring_states_in
+                                  .Arg<ffi::Buffer<ffi::F32>>()  // ring_rewards_in
+                                  .Arg<ffi::Buffer<ffi::U8>>()   // tree_in
+                                  .Arg<ffi::Buffer<ffi::U8>>()   // compact [T',B,S]
+                                  .Arg<ffi::Buffer<ffi::F32>>()  // rewards [T',B]
                                   .Ret<ffi::Buffer<ffi::U8>>()   // ring_states
                                   .Ret<ffi::Buffer<ffi::F32>>()  // ring_rewards
                                   .Ret<ffi::Buffer<ffi::U8>>()   // tree

@@ -14,7 +14,9 @@ Call shapes mirror the reference (file:line under /root/reference/src):
     forward_states(...)                  selfplay.py:89, reanalyze.py:67,90
     reanalyze_targets(...)               reanalyze.py:86-129
     hash_update(...)                     train.py:22 (network/hashes.py:45-50)
-    make_prioritised_flat_buffer(...)    main.py:217-225 (init / add / sample / set_priorities: main.py:383-385, 413-414, 454)
+    make_prioritised_flat_buffer(...)    main.py:217-225 (init / add / sample / set_priorities: main.py:383-385, 413-414, 454);
+                                         add also takes selfplay()'s SelfplayOutput.state, the whole scan in one call
+                                         (main.py:383-385 with add_sequences=True)
 """
 from __future__ import annotations
 
@@ -36,8 +38,9 @@ _shim = ctypes.CDLL(os.path.join(_HERE, "libeaz_xla_ffi.so"))
 for _name, _sym in (("eaz_search", "EazSearch"), ("eaz_env_step", "EazEnvStep"), ("eaz_env_init", "EazEnvInit"),
                     ("eaz_mlp_forward_states", "EazMlpForwardStates"), ("eaz_reanalyze_targets", "EazReanalyzeTargets"),
                     ("eaz_hash_update", "EazHashUpdate"), ("eaz_evaluate", "EazEvaluate"), ("eaz_selfplay", "EazSelfplay"),
-                    ("eaz_replay_init", "EazReplayInit"), ("eaz_replay_add", "EazReplayAdd"), ("eaz_replay_sample", "EazReplaySample"),
-                    ("eaz_replay_set_priorities", "EazReplaySetPriorities"), ("eaz_replay_status", "EazReplayStatus")):
+                    ("eaz_replay_init", "EazReplayInit"), ("eaz_replay_add", "EazReplayAdd"), ("eaz_replay_add_sequence", "EazReplayAddSequence"),
+                    ("eaz_replay_sample", "EazReplaySample"), ("eaz_replay_set_priorities", "EazReplaySetPriorities"),
+                    ("eaz_replay_status", "EazReplayStatus")):
     jax.ffi.register_ffi_target(_name, jax.ffi.pycapsule(getattr(_shim, _sym)), platform="CUDA")
 
 i32, f32 = np.int32, np.float32
@@ -187,7 +190,7 @@ def evaluate(params, model_state, env: EnvSpec, states, *, num_simulations, disc
 
 class SelfplayOutput(NamedTuple):  # selfplay.py:17-23, every field stacked over the steps
     state: tuple                          # the states after each step as (eaz_env_compact records U8[T,B,S], rewards F32[T,B]): the
-    root_value: jax.Array                 # replay ring's format (one row per time slot)
+    root_value: jax.Array                 # replay ring's format (one row per time slot; make_prioritised_flat_buffer(...).add takes it)
     root_epistemic_std: jax.Array
     value_prediction: jax.Array
     ube_prediction: jax.Array
@@ -335,6 +338,8 @@ def make_prioritised_flat_buffer(env: EnvSpec, max_length_time_axis, add_batch_s
 
         init(template_state, seed) -> ReplayState          (seed: a Python int, it becomes an attribute)
         add(rs, states) -> ReplayState                     one time step of the add_batch_size envs, at the device cursor
+        add(rs, (compact, rewards)) -> ReplayState         T' time steps at once, in time order: selfplay()'s SelfplayOutput.state
+                                                           (U8[T',B,S], F32[T',B]), so `rs = add(rs, out.state)` is main.py:383-385
         sample(rs, key) -> PrioritisedSample               sample_batch_size pairs drawn from key; rs is only read
         set_priorities(rs, indices, priorities) -> ReplayState
         can_sample(rs) -> bool[]                           at least two time steps stored
@@ -362,6 +367,11 @@ def make_prioritised_flat_buffer(env: EnvSpec, max_length_time_axis, add_batch_s
         return ReplayState(*out)
 
     def add(rs: ReplayState, states):
+        if isinstance(states, tuple):  # (compact records [T',B,S], rewards [T',B]): a scan's time steps
+            compact, rewards = states
+            out = jax.ffi.ffi_call("eaz_replay_add_sequence", ring_types, input_output_aliases={1: 0, 2: 1, 3: 2})(
+                env.amap(), rs.states, rs.rewards, rs.tree, compact.astype(jnp.uint8), rewards.astype(jnp.float32), **env.attrs())
+            return ReplayState(*out)
         out = jax.ffi.ffi_call("eaz_replay_add", ring_types, input_output_aliases={1: 0, 2: 1, 3: 2})(
             env.amap(), rs.states, rs.rewards, rs.tree, *state_leaves(env, states), **env.attrs())
         return ReplayState(*out)

@@ -299,6 +299,26 @@ def replay_add(env: EnvSpec, st: dict, ring_states, ring_rewards, tree) -> None:
                                 C.c_size_t(tree.numel()), int(T), int(B), _stream()), "eaz_replay_add")
 
 
+def replay_add_sequence(env: EnvSpec, compact, rewards, ring_states, ring_rewards, tree) -> None:
+    """eaz_replay_add_sequence: the T' time steps of compact [T',B,S] (eaz_env_compact records, e.g. a scan's SelfplayOutput.state) and
+    rewards [T',B] into ring rows cursor .. cursor + T' - 1 (mod T) of ring_states [T,B,S] / ring_rewards [T,B], the tree ending as after
+    T' calls of replay_add.  The cursor is read and advanced on the device; nothing is allocated or synchronised, so the call can be
+    captured in a CUDA graph."""
+    import torch
+
+    T, B, S = ring_states.shape[0], ring_states.shape[1], env.compact_bytes
+    if ring_states.dim() != 3 or ring_states.shape[2] != S or tuple(ring_rewards.shape) != (T, B):
+        raise EazError("replay_add_sequence: ring_states must be [T, B, compact_bytes] and ring_rewards [T, B]")
+    if compact.dim() != 3 or tuple(compact.shape[1:]) != (B, S) or tuple(rewards.shape) != tuple(compact.shape[:2]):
+        raise EazError(f"replay_add_sequence: compact must be [T', {B}, {S}] and rewards [T', {B}] (got {tuple(compact.shape)} and "
+                       f"{tuple(rewards.shape)})")
+    empty = compact.shape[0] == 0
+    check(load().eaz_replay_add_sequence(C.byref(env.struct()), None if empty else _ptr(compact, torch.uint8),
+                                         None if empty else _ptr(rewards, torch.float32), int(compact.shape[0]),
+                                         _ptr(ring_states, torch.uint8), _ptr(ring_rewards, torch.float32), _ptr(tree),
+                                         C.c_size_t(tree.numel()), int(T), int(B), int(S), _stream()), "eaz_replay_add_sequence")
+
+
 def priority_sample_keyed(tree, T: int, B: int, key, indices, probabilities, states=None, rewards=None, first=None, first_rewards=None,
                           second=None, second_rewards=None) -> None:
     """eaz_priority_sample_keyed: as priority_sample with (seed, draw counter) = key, a uint32-valued int32 [2] device tensor; the

@@ -44,6 +44,43 @@ class CompactReplayRing:
         self.cursor = (self.cursor + 1) % self.T
         self.length = min(self.length + 1, self.T)
 
+    def add_sequence(self, x) -> None:
+        """Append T' time steps at once, in time order: the cursor and length advance by T' (only the last T rows survive when
+        T' > T), exactly as T' add() calls would.  `x` is a scan's SelfplayOutput.state, dict(compact=[T',B,S] uint8, rewards=[T',B])
+        (SelfplayRunner.scan), or state leaves with a leading time axis [T',B,...], as a dict or the pgx State of selfplay(); those
+        are compacted in one eaz_env_compact call over the T' * B rows."""
+        compact, rewards = self._sequence(x)
+        n = compact.shape[0]
+        keep = min(n, self.T)
+        s0 = (self.cursor + n - keep) % self.T
+        k1 = min(keep, self.T - s0)  # rows before the ring wraps
+        self.states[s0:s0 + k1].copy_(compact[n - keep:n - keep + k1])
+        self.rewards[s0:s0 + k1].copy_(rewards[n - keep:n - keep + k1])
+        self.states[:keep - k1].copy_(compact[n - keep + k1:])
+        self.rewards[:keep - k1].copy_(rewards[n - keep + k1:])
+        self._advance(n)
+
+    def _advance(self, n: int) -> None:
+        self.cursor = (self.cursor + n) % self.T
+        self.length = min(self.length + n, self.T)
+
+    def _sequence(self, x):
+        """-> (compact [T',B,S] uint8, rewards [T',B] float32), contiguous device tensors"""
+        torch = require_cuda()
+        if isinstance(x, dict) and "compact" in x:
+            compact, rewards = x["compact"], x["rewards"]
+        else:
+            leaves = x.leaves if hasattr(x, "leaves") else x  # pgx State of e_alphazero_b200.pgx, or a dict of its leaves
+            n, B = leaves["step_count"].shape[:2]
+            flat = {k: leaves[k].reshape((n * B,) + tuple(leaves[k].shape[2:])).contiguous() for k in ops.state_fields(self.env)}
+            compact = ops.env_compact(self.env, flat).reshape(n, B, self.S) if n > 0 else torch.empty((0, B, self.S), dtype=torch.uint8,
+                                                                                                       device=self.device)
+            rewards = leaves["rewards"].reshape(n, B)
+        if compact.dim() != 3 or tuple(compact.shape[1:]) != (self.B, self.S) or tuple(rewards.shape[:2]) != tuple(compact.shape[:2]):
+            raise EazError(f"add_sequence: expected [T', {self.B}, ...] time steps of the ring's {self.B} envs (compact records "
+                           f"[T', {self.B}, {self.S}], rewards [T', {self.B}])")
+        return compact.contiguous(), rewards.reshape(compact.shape[:2]).to(torch.float32).contiguous()
+
     def can_sample(self, min_length: int = 2) -> bool:
         return self.length >= max(2, min_length)
 
@@ -95,6 +132,13 @@ class PrioritisedReplayRing(CompactReplayRing):
         slot = self.cursor
         super().add(state)
         ops.priority_add_step(self.tree, self.T, self.B, slot)
+
+    def add_sequence(self, x) -> None:
+        """CompactReplayRing.add_sequence with the tree: one eaz_replay_add_sequence call (the rows, the leaves they touch and the
+        header), bit for bit what T' add() calls leave."""
+        compact, rewards = self._sequence(x)
+        ops.replay_add_sequence(self.env, compact, rewards, self.states, self.rewards, self.tree)
+        self._advance(compact.shape[0])
 
     def alloc_sample(self, batch_size: int, with_obs: bool = False) -> PrioritisedSample:
         """Output buffers for sample(batch_size, with_obs, out=...)."""

@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define EAZ_ABI_VERSION 7
+#define EAZ_ABI_VERSION 8
 
 enum {
   EAZ_OK = 0,
@@ -569,6 +569,18 @@ int eaz_priority_sample_keyed(const void* tree, size_t tree_bytes, int32_t T, in
                               uint8_t* second, float* second_rewards, void* stream);
 /* Copies the sticky EAZ_PRIORITY_* word into the device int32 *flags_dev on `stream`; does not synchronise. */
 int eaz_priority_status_async(const void* tree, size_t tree_bytes, int32_t* flags_dev, void* stream);
+
+/* ABI 8 (appended): a whole self-play scan into the ring in one call -- flashbax's add with add_sequences=True after the scan
+ * (main.py:383-385). */
+
+/* Appends `steps` time steps to the ring at the DEVICE cursor: row j of compact [steps,B,S] (eaz_env_compact records, e.g.
+ * eaz_selfplay_outputs.states) and of rewards [steps,B] goes to slot (c + j) % T, c = the header's cursor, so only the last T rows
+ * survive when steps > T.  The tree buffer, header included, ends exactly as after `steps` calls of eaz_replay_add (add_step at the
+ * header's cursor each time), from any ring state.  S must equal eaz_env_compact_bytes(env); compact / rewards may be NULL only
+ * when steps == 0, which enqueues nothing.  Every argument is checked before anything is enqueued.  L + 1 launches for a tree of L
+ * levels, independent of `steps`; no allocation, no synchronisation. */
+int eaz_replay_add_sequence(const eaz_env* env, const uint8_t* compact, const float* rewards, int32_t steps, uint8_t* ring_states,
+                            float* ring_rewards, void* tree, size_t tree_bytes, int32_t T, int32_t B, int32_t S, void* stream);
 
 #ifdef __cplusplus
 }
